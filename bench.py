@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark of the HermNet hot path on B200 (contract: see the task brief / DESIGN.md "Measurement").
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload C4] [--scale S]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload C4] [--scale S] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[3], the configuration the metric "atom-steps/s (energy+forces)" is quoted on and the
 largest that fits one GPU): HVNet, 3 interactions, F=128, K=128, rc=5 A on the synthetic 1 000 000-atom Li/Al/Si/O
@@ -13,6 +13,9 @@ One JSON line on stdout (rank 0).  ``value``: graph and inputs resident in HBM, 
 neighbour-list build, forward, backward, D2H of forces + energy all inside the timed region.
 ``--impl reference`` times the CPU restatement of the reference PyG path (oracle/, the reference itself cannot be
 imported without PyG / torch_scatter / ASE) on a bounded sample of the same workload with all host threads.
+``--dump-outputs DIR`` (C4 / C5): after the timed steps, rank 0 writes what the timed path returned in its last step as
+``DIR/energy.npy`` (float32 [1]) and ``DIR/forces.npy`` (float32 [N, 3], minus dE/dpos).  Inputs and weights are seeded,
+so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -49,7 +52,13 @@ def parse_args():
     ap.add_argument("--skin", type=float, default=0.4, help="C3: Verlet skin in Angstrom")
     ap.add_argument("--graph-skin", type=float, default=1.0, help="C3: Verlet skin of the CUDA-graph variant")
     ap.add_argument("--cuda-graph", type=int, default=1, help="C4: replay the resident step as ONE captured CUDA graph (0: eager launches)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the energy and forces of the last timed step to DIR/*.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.workload in ("C2", "C3")):
+        ap.error("--dump-outputs is supported for the energy + forces workloads (C4, C5) of --impl b200")
+    return args
 
 
 # --------------------------------------------------------------------------------------------------------------
@@ -98,6 +107,22 @@ def hbm_peak():
         except Exception:
             pass
     return HBM_FALLBACK_GBS, "fallback (B200_PROFILING.md)"
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, energy, grad):
+    """``energy [1]`` and ``forces = -grad [N, 3]`` as float32 ``.npy`` files of at most DUMP_LIMIT_BYTES together; a larger
+    force array is cut to a fixed, seeded sample of rows (the same rows in every run with the same N)."""
+    os.makedirs(out_dir, exist_ok=True)
+    e = energy.detach().float().cpu().numpy().reshape(-1)
+    f = (-grad.detach()).float().cpu().numpy()
+    max_rows = (DUMP_LIMIT_BYTES - 4096 - e.nbytes) // (3 * f.itemsize)     # 4096: room for the two .npy headers
+    if f.shape[0] > max_rows:
+        f = f[np.sort(np.random.default_rng(0).choice(f.shape[0], size=max_rows, replace=False))]
+    np.save(os.path.join(out_dir, "energy.npy"), e)
+    np.save(os.path.join(out_dir, "forces.npy"), f)
 
 
 def workload(name: str, scale: float):
@@ -531,7 +556,8 @@ def main():
     barrier()
 
     def timed(step_fn, collect):
-        """K steps bracketed by barrier + synchronize, CUDA events, max over ranks; ``collect``: per-kernel events."""
+        """K steps bracketed by barrier + synchronize, CUDA events, max over ranks; ``collect``: per-kernel events.
+        Also returns what the last step returned, ``(energy, dE/dpos)``."""
         if collect:
             ops.TIMERS = {}
         ops.LAUNCHES["n"] = 0
@@ -539,7 +565,7 @@ def main():
         barrier()
         a.record()
         for _ in range(args.steps):
-            step_fn()
+            out = step_fn()
         b.record()
         barrier()
         n_launch = ops.LAUNCHES["n"]
@@ -549,13 +575,13 @@ def main():
             t = torch.tensor([t_ms], device=dev)
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             t_ms = float(t)
-        return t_ms, n_launch, tm
+        return t_ms, n_launch, tm, out
 
     # eager pass: every launch individually, CUDA events around each kernel (the per-kernel table / roofline come from here)
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
-    ms_eager, launches, timers = timed(step_resident, True)
+    ms_eager, launches, timers, last = timed(step_resident, True)
     # graphed pass: the same step (forward_graph + autograd.grad [+ halo exchange and all-reduces]) captured ONCE and replayed
     graphed, graph_note = None, "eager launches"
     if args.cuda_graph:
@@ -573,11 +599,13 @@ def main():
         if float(ok) == 0:
             graphed = None
     if graphed is not None:
-        ms, _, _ = timed(graphed, False)
+        ms, _, _, last = timed(graphed, False)
         graph_note = "one captured CUDA graph per step (forward + backward [+ halo exchange, all-reduces]) replayed"
     else:
         ms = ms_eager
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *last)
     ms_per_step = ms / args.steps
     value = N * args.steps / (ms * 1e-3)
 
@@ -650,8 +678,9 @@ def main():
 
 
 def _finish(world, real_stdout, line):
-    """Print the line (rank 0) and leave WITHOUT tearing down NCCL / symmetric memory / captured graphs: destroying a
-    process group whose collectives live in a CUDA graph can block, and the process is done anyway."""
+    """Print the line (rank 0) and end the process.  A single process exits normally, so atexit handlers and library
+    teardown run.  Ranks of a multi-GPU run leave WITHOUT tearing down NCCL / symmetric memory / captured graphs:
+    destroying a process group whose collectives live in a CUDA graph can block, and the process is done anyway."""
     sys.stdout.flush()
     sys.stderr.flush()
     if line is not None:
@@ -660,7 +689,9 @@ def _finish(world, real_stdout, line):
         torch.cuda.synchronize()
     except Exception:  # noqa: BLE001
         pass
-    os._exit(0)
+    if world > 1:
+        os._exit(0)
+    sys.exit(0)
 
 
 if __name__ == "__main__":
