@@ -48,7 +48,7 @@ SIGNATURES = {
     "hn_painn_edge_fwd": (c_int32, [POINTER(EdgeParams)] + [P] * 13),
     "hn_painn_edge_bwd_dst": (c_int32, [POINTER(EdgeParams)] + [P] * 13 + [c_int64, P]),
     "hn_painn_edge_bwd_src": (c_int32, [POINTER(EdgeParams)] + [P] * 16),
-    "hn_painn_edge_bwd_w": (c_int32, [POINTER(EdgeParams)] + [P] * 12 + [c_int32, P]),
+    "hn_painn_edge_bwd_w": (c_int32, [POINTER(EdgeParams)] + [P] * 13 + [c_int32, P]),
     "hn_tc_supported": (c_int32, [c_int32, c_int32]),
     "hn_tc_block_rows": (c_int32, [c_int32]),
     "hn_tc_tile_edges": (c_int32, []),
@@ -111,7 +111,7 @@ def load(build_if_missing: bool = True):
         fn = getattr(lib, name)  # AttributeError here = ABI mismatch, fail loudly
         fn.restype = res
         fn.argtypes = args
-    if lib.hn_abi_version() != 1:
+    if lib.hn_abi_version() != 2:
         raise RuntimeError("hermnet_b200: ABI version mismatch between _lib.py and the shared library")
     _LIB = lib
     return lib

@@ -356,13 +356,15 @@ edge_bwd_src_kernel(const hn_edge_params P, const float *__restrict__ xh, const 
 
 // Filter-weight gradient (only needed when rbf_proj parameters require grad on the fused path):
 //   gW[m][k][c] = sum_e env*g_k(d_e) * gphi_e[c],   gb[m][c] = sum_e gphi_e[c]
-// One CTA = one (row chunk, module, 384-column slice); thread t owns column t of the slice, the [K][384]
-// accumulator lives in shared memory and is updated without atomics (each thread only touches its own
-// column).  Partials per chunk are reduced by the caller (fixed order -> deterministic).
+// One CTA = one (row chunk, module, column slice of <= 384 columns); thread t owns column t of the slice, the
+// [K][cols] accumulator lives in shared memory and is updated without atomics (each thread only touches its own
+// column).  Partials per chunk are reduced by the caller (fixed order -> deterministic).  edge_live (NULL: every
+// entry is an edge) drops the dead entries of a Verlet-skin list from both sums.
 __global__ void __launch_bounds__(384)
 edge_bwd_w_kernel(const hn_edge_params P, const float *__restrict__ xh, const float *__restrict__ vec,
                   const float4 *__restrict__ geom, const int *__restrict__ rowptr, const int *__restrict__ col,
-                  const int *__restrict__ row_mod, const long long *__restrict__ row_xoff, const float *__restrict__ offset,
+                  const int *__restrict__ row_mod, const long long *__restrict__ row_xoff,
+                  const unsigned char *__restrict__ edge_live, const float *__restrict__ offset,
                   const float *__restrict__ g_dx, const float *__restrict__ g_dvec, float *__restrict__ gW_part,
                   float *__restrict__ gb_part, int n_chunks, int cols_per_cta) {
     extern __shared__ float acc[];  // [K][cols_per_cta]
@@ -393,6 +395,7 @@ edge_bwd_w_kernel(const hn_edge_params P, const float *__restrict__ xh, const fl
             }
         }
         for (int e = e0; e < e1; ++e) {
+            if (edge_live != nullptr && __ldg(edge_live + e) == 0) continue;   // uniform across the CTA
             const int s = __ldg(col + e);
             const float4 g = __ldg(geom + e);
             float gphi = 0.f;
@@ -426,13 +429,15 @@ edge_bwd_w_kernel(const hn_edge_params P, const float *__restrict__ xh, const fl
 
 int pick_vec(int F) { return F % 128 == 0 ? 4 : (F % 64 == 0 ? 2 : (F % 32 == 0 ? 1 : 0)); }
 
-int validate(const char *where, const hn_edge_params *p) {
+// masked_ok: the entry point takes a live mask and honours flags bit 0 (Verlet-skin superset lists)
+int validate(const char *where, const hn_edge_params *p, bool masked_ok = false) {
     HN_REQUIRE(p != nullptr, where, "null params");
     HN_REQUIRE(pick_vec(p->hidden) != 0, where, "hidden_channels must be a multiple of 32");
     HN_REQUIRE(p->num_rbf >= 2, where, "num_rbf must be >= 2");
     HN_REQUIRE(p->env_p >= 1, where, "envelope exponent must be >= 1");
     HN_REQUIRE(p->n_modules >= 1, where, "n_modules must be >= 1");
-    HN_REQUIRE(!(p->flags & 1), where, "Verlet-skin superset lists (flags bit 0) are only supported by the hn_tc_edge_* kernels");
+    HN_REQUIRE(masked_ok || !(p->flags & 1), where,
+               "Verlet-skin superset lists (flags bit 0) are only supported by the hn_tc_edge_* kernels and hn_painn_edge_bwd_w");
     return 0;
 }
 
@@ -524,19 +529,24 @@ extern "C" int hn_painn_edge_bwd_src(const hn_edge_params *p, const float *xh, c
 
 extern "C" int hn_painn_edge_bwd_w(const hn_edge_params *p, const float *xh, const float *vec, const float *geom,
                                    const int32_t *rowptr, const int32_t *col, const int32_t *row_mod, const int64_t *row_xoff,
-                                   const float *offset, const float *g_dx, const float *g_dvec, float *gW_part,
-                                   float *gb_part, int32_t n_chunks, void *stream) {
+                                   const uint8_t *live, const float *offset, const float *g_dx, const float *g_dvec,
+                                   float *gW_part, float *gb_part, int32_t n_chunks, void *stream) {
     const char *where = "hn_painn_edge_bwd_w";
-    if (int rc = validate(where, p)) return rc;
+    if (int rc = validate(where, p, true)) return rc;
+    HN_REQUIRE(!(p->flags & 1) || live != nullptr, where, "a Verlet-skin list (flags bit 0) needs the live mask");
     HN_REQUIRE(n_chunks >= 1, where, "n_chunks must be >= 1");
+    // column slice: the widest multiple of 32 (F % 32 == 0, so 3F is one) up to 384 whose [K][cols] fp32 accumulator fits in
+    // shared memory; several slices when 3F is wider, the last one partly filled
     const int F3 = 3 * p->hidden;
-    const int cols = F3 < 384 ? F3 : 384;              // multiple of 32 because F % 32 == 0
+    const int fit = (int)((size_t)227 * 1024 / ((size_t)p->num_rbf * sizeof(float))) / 32 * 32;
+    int cols = F3 < 384 ? F3 : 384;
+    cols = cols < fit ? cols : fit;
+    HN_REQUIRE(cols >= 32, where, "num_rbf too large for the shared-memory accumulator (K * 32 columns * 4 bytes > 227 KB)");
     const size_t smem = (size_t)p->num_rbf * cols * sizeof(float);
-    HN_REQUIRE(smem <= 227 * 1024, where, "num_rbf too large for the shared-memory accumulator");
     HN_CUDA(cudaFuncSetAttribute(edge_bwd_w_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem), where);
     dim3 grid(n_chunks, (F3 + cols - 1) / cols, p->n_modules);
     edge_bwd_w_kernel<<<grid, cols, smem, (cudaStream_t)stream>>>(*p, xh, vec, (const float4 *)geom, rowptr, col, row_mod,
-                                                                  (const long long *)row_xoff, offset, g_dx, g_dvec, gW_part,
-                                                                  gb_part, n_chunks, cols);
+                                                                  (const long long *)row_xoff, (p->flags & 1) ? live : nullptr,
+                                                                  offset, g_dx, g_dvec, gW_part, gb_part, n_chunks, cols);
     return hn::check_launch(where);
 }

@@ -310,18 +310,23 @@ def painn_edge_bwd_src(p: EdgeParams, xh, vec, geom, g, Wt, bias, offset, g_dx, 
 
 
 def painn_edge_bwd_w(p: EdgeParams, xh, vec, geom, g, offset, g_dx, g_dvec):
-    """Gradients of the filter projection: ``gWt [M,K,3F]``, ``gb [M,3F]`` (partials reduced in fixed order)."""
+    """Gradients of the filter projection: ``gWt [M,K,3F]``, ``gb [M,3F]`` (partials reduced in fixed order).  A Verlet-skin
+    list (``p.flags`` bit 0) needs ``p.live``, the uint8 [E] mask the model attaches next to the flag: entries marked 0
+    contribute nothing."""
     lib = _lib.load()
-    dev = _chk("painn_edge_bwd_w", xh, vec, geom, offset, g_dx, g_dvec)
+    live = getattr(p, "live", None) if p.flags & 1 else None
+    dev = _chk("painn_edge_bwd_w", xh, vec, geom, offset, g_dx, g_dvec, live)
     _f32("painn_edge_bwd_w", xh, vec, geom, offset, g_dx, g_dvec)
+    if live is not None and (live.dtype != torch.uint8 or live.numel() != geom.size(0)):
+        raise TypeError("hermnet_b200.painn_edge_bwd_w: live must be uint8 [E]")
     M, K, F3 = p.n_modules, p.num_rbf, 3 * p.hidden
     n_chunks = max(1, min(p.n_rows, (2 * max(sm_count(), 1)) // max(M, 1)))
     gW = torch.empty((n_chunks, M, K, F3), dtype=torch.float32, device=dev)
     gb = torch.empty((n_chunks, M, F3), dtype=torch.float32, device=dev)
     with torch.cuda.device(dev), _timed("painn_edge_bwd_w", dev):
         _lib.check(lib.hn_painn_edge_bwd_w(ctypes.byref(p), _ptr(xh), _ptr(vec), _ptr(geom), _ptr(g.rowptr), _ptr(g.col),
-                                           _ptr(g.row_mod), _ptr(g.row_xoff), _ptr(offset), _ptr(g_dx), _ptr(g_dvec), _ptr(gW), _ptr(gb),
-                                           n_chunks, _stream(dev)), "hn_painn_edge_bwd_w")
+                                           _ptr(g.row_mod), _ptr(g.row_xoff), _ptr(live), _ptr(offset), _ptr(g_dx), _ptr(g_dvec), _ptr(gW),
+                                           _ptr(gb), n_chunks, _stream(dev)), "hn_painn_edge_bwd_w")
     return gW.sum(0), gb.sum(0)
 
 

@@ -30,7 +30,7 @@
 extern "C" {
 #endif
 
-#define HN_ABI_VERSION 1
+#define HN_ABI_VERSION 2
 
 int hn_abi_version(void);
 const char *hn_last_error(void);
@@ -137,8 +137,8 @@ typedef struct {
                              else row-per-warp), 1 = row-per-warp only (A/B measurements).  Per call: no library state. */
     int32_t flags;        /* bit 0: the edge list is a Verlet-skin SUPERSET (built with rc + skin): the entries marked dead
                              by hn_tc_tile_windows(live) must contribute nothing -- not even the filter bias (rmnet.py:55:
-                             the reference has no such edge).  Honoured by the hn_tc_edge_* kernels; the other families
-                             reject it. */
+                             the reference has no such edge).  Honoured by the hn_tc_edge_* kernels and by
+                             hn_painn_edge_bwd_w (through its live argument); the other families reject it. */
 } hn_edge_params;
 
 /* Planes of g_geom that hn_painn_edge_bwd_dst writes for this F and kernel family (the caller sums them); 0 = unsupported F. */
@@ -160,10 +160,12 @@ int hn_painn_edge_bwd_src(const hn_edge_params *p, const float *xh, const float 
 /* Filter-weight gradient of the fused path (autograd of nn.Linear rbf_proj, rmnet.py:45,55):
  *   gW_part[chunk][m][k][c] / gb_part[chunk][m][c] hold per-row-chunk partial sums of
  *   gW[m][k][c] = sum_e env*gauss_k(d_e) * dL/dphi_e[c],  gb[m][c] = sum_e dL/dphi_e[c];
- *   the caller adds the n_chunks partials in fixed order (deterministic). */
+ *   the caller adds the n_chunks partials in fixed order (deterministic).
+ *   live: uint8 [E], 0 = entry of a Verlet-skin list that is not an edge now (left out of both sums); required with
+ *   p->flags bit 0, ignored (may be NULL) without it.  num_rbf up to 1816 (a [K][32] fp32 accumulator fits in 227 KB). */
 int hn_painn_edge_bwd_w(const hn_edge_params *p, const float *xh, const float *vec, const float *geom,
                         const int32_t *rowptr, const int32_t *col, const int32_t *row_mod, const int64_t *row_xoff,
-                        const float *offset, const float *g_dx, const float *g_dvec,
+                        const uint8_t *live, const float *offset, const float *g_dx, const float *g_dvec,
                         float *gW_part /*[n_chunks,M,K,3F]*/, float *gb_part /*[n_chunks,M,3F]*/, int32_t n_chunks,
                         void *stream);
 

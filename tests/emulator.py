@@ -216,13 +216,16 @@ def painn_edge_bwd_w(p, xh, vec, geom, g, offset, g_dx, g_dvec):
     F = p.hidden
     row = g.edge_row.long()
     m = g.row_mod.long()[row]
-    live = (m >= 0).to(xh.dtype)[:, None]
+    act = m >= 0
+    if p.flags & 1:                      # Verlet-skin superset list: dead entries feed neither gW nor gb
+        act = act & p.live.bool()
+    lv = act.to(xh.dtype)[:, None]
     mm = m.clamp(min=0)
     s = g.col.long()
     P = xh[(g.row_xoff[row] + s).clamp(min=0)]
     V = vec[s]
     gv, tb, tc, c1, c2 = _t_terms(p, V, geom, g_dvec, row, F)
-    gphi = torch.cat([g_dx[row] * P[:, :F], tb * P[:, F:2 * F], tc * P[:, 2 * F:]], 1) * live
+    gphi = torch.cat([g_dx[row] * P[:, :F], tb * P[:, F:2 * F], tc * P[:, 2 * F:]], 1) * lv
     val = _band(p, geom, offset)
     gW = torch.zeros((p.n_modules, p.num_rbf, 3 * F), dtype=xh.dtype)
     gW.index_add_(0, mm, val[:, :, None] * gphi[:, None, :])

@@ -33,7 +33,7 @@ def test_library_builds_and_exports_every_declared_symbol():
 def test_ctypes_table_matches_header():
     assert sorted(_lib.SIGNATURES) == declared_symbols()
     lib = _lib.load()
-    assert lib.hn_abi_version() == 1
+    assert lib.hn_abi_version() == 2
     assert lib.hn_painn_edge_num_slices(128, 0) == 1 and lib.hn_painn_edge_num_slices(256, 0) == 2
     assert lib.hn_painn_edge_num_slices(96, 0) == 3 and lib.hn_painn_edge_num_slices(100, 1) == 0
     assert lib.hn_painn_edge_num_slices(128, 1) == lib.hn_painn_edge_num_slices(128, 1) >= 1 and lib.hn_segment_sum_workspace_bytes(2, 1) > 0

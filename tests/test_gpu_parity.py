@@ -307,34 +307,46 @@ def test_sort_by_key_is_a_stable_counting_sort(n, n_keys):
     assert torch.equal(order.cpu().long(), ref_order)
 
 
-@pytest.mark.parametrize("kind,pbc_shift", [("HVNet", "reference"), ("HVNet", "physical"), ("HTNet", "reference")])
-def test_verlet_skin_list_reuse_on_gpu(kind, pbc_shift):
+@pytest.mark.parametrize("kind,pbc_shift,trainable",
+                         [pytest.param(k, s, t, id=f"{k}-{s}" + ("-trainable" if t else ""))
+                          for t in (False, True) for k, s in (("HVNet", "reference"), ("HVNet", "physical"), ("HTNet", "reference"))])
+def test_verlet_skin_list_reuse_on_gpu(kind, pbc_shift, trainable):
     """SURVEY 8(f) rank 1: a list searched with rc + skin, re-used after the atoms moved (< skin / 2), gives the energies /
     forces / cell gradient of a fresh list through the tensor-core edge kernels (dead entries stage zeros: they contribute
-    nothing, not even the filter bias); the device MD loop re-uses it and follows the rebuild-every-step trajectory."""
+    nothing, not even the filter bias); the device MD loop re-uses it and follows the rebuild-every-step trajectory.
+    trainable: an eval-mode model whose parameters still require grad runs the filter-weight backward on every force
+    call; its rbf_proj gradients on the skin list equal those of a fresh list."""
     from hermnet_b200.plugin import md
     pos, Z, cell = synthetic.water_box(5, seed=9)
     pos, Z, cell = torch.from_numpy(pos).to(DEV), torch.from_numpy(Z).to(DEV), torch.from_numpy(cell)[None].to(DEV)
     torch.manual_seed(11)
     model = getattr(H, kind)(elems=["H", "O"], rc=4.5, num_layers=2, hidden_channels=128, num_rbf=64, pbc_shift=pbc_shift).to(DEV).eval()
     for p in model.parameters():
-        p.requires_grad_(False)
+        p.requires_grad_(trainable)
     g_skin = model.build_graph(pos, Z, cell, skin=0.8)
     assert g_skin.masked and g_skin.n_edges > model.build_graph(pos, Z, cell).n_edges
     gen = torch.Generator().manual_seed(1)
     pos2 = pos + (0.38 * (2 * torch.rand(pos.shape, generator=gen) - 1) / 3 ** 0.5).to(DEV)
-    out = []
+    out, wgrads = [], []
     for graph in (g_skin, None):
         d = H.Data(pos=pos2.clone().requires_grad_(True), atomic_number=Z, cell=cell.clone().requires_grad_(True))
         if graph is not None:
             d.graph = graph
         e = model(d)
-        gp, gc = torch.autograd.grad(e.sum(), [d.pos, d.cell])
+        gp, gc = torch.autograd.grad(e.sum(), [d.pos, d.cell], retain_graph=trainable)
         out.append((e.detach(), gp, gc))
+        if trainable:
+            model.zero_grad()
+            e.sum().backward()
+            wgrads.append({k: q.grad.clone() for k, q in model.named_parameters() if "rbf_proj" in k})
     assert util.rel_err(out[0][0], out[1][0]) < 3e-6
     fs = max(1.0, float(out[1][1].abs().max()))
     assert float((out[0][1] - out[1][1]).abs().max()) < 3e-5 * fs
     assert float((out[0][2] - out[1][2]).abs().max()) < 3e-4 * max(1.0, float(out[1][2].abs().max()))
+    if trainable:
+        assert len(wgrads[1]) >= 8
+        for k, ref in wgrads[1].items():
+            assert float((wgrads[0][k] - ref).abs().max()) < 3e-4 * float(ref.abs().max()), k
     if kind == "HVNet":
         v0 = 0.003 * torch.randn(pos.shape, generator=torch.Generator().manual_seed(2)).numpy()
         runs = {}

@@ -229,35 +229,47 @@ def test_loader_side_batched_graph_build_equals_per_sample_transform(emu):
     assert util.rel_err(model(d2).detach(), model(d).detach()) < 1e-6
 
 
-@pytest.mark.parametrize("path", ["fused", "composite"])
-def test_verlet_skin_list_gives_the_energy_of_a_fresh_list(emu, path):
+@pytest.mark.parametrize("path,trainable", [pytest.param("fused", False, id="fused"),
+                                            pytest.param("composite", False, id="composite"),
+                                            pytest.param("fused", True, id="fused-trainable"),
+                                            pytest.param("composite", True, id="composite-trainable")])
+def test_verlet_skin_list_gives_the_energy_of_a_fresh_list(emu, path, trainable):
     """SURVEY 8(f) rank 1: a list searched with rc + skin and re-used after the atoms moved (< skin / 2) must give the
-    energies / forces of a fresh list: entries at or beyond rc contribute nothing, not even the filter bias."""
+    energies / forces of a fresh list: entries at or beyond rc contribute nothing, not even the filter bias.  With trainable
+    parameters (an eval-mode model nobody froze) the filter-weight backward runs too and must drop the dead entries."""
     from tests.util import lattice_system
     pos, Z, cell = lattice_system(5, [3, 8], 21)
     torch.manual_seed(5)
     model = H.HVNet(elems=["Li", "O"], rc=4.0, num_layers=2, hidden_channels=128, num_rbf=32).eval()
     for p in model.parameters():
-        p.requires_grad_(False)
+        p.requires_grad_(trainable)
     model.edge_path = path
     g_skin = model.build_graph(pos, Z, cell, skin=0.6)
     g_plain = model.build_graph(pos, Z, cell)
     assert g_skin.masked and g_skin.n_edges > g_plain.n_edges
     gen = torch.Generator().manual_seed(1)
     pos2 = pos + 0.28 * (2 * torch.rand(pos.shape, generator=gen) - 1) / 3 ** 0.5     # every atom moved < 0.28 A < skin / 2
-    out = []
+    out, wgrads = [], []
     for graph in (g_skin, None):
         d = H.Data(pos=pos2.clone().requires_grad_(True), atomic_number=Z, cell=cell.clone().requires_grad_(True))
         if graph is not None:
             d.graph = graph
         e = model(d)
-        gp, gc = torch.autograd.grad(e.sum(), [d.pos, d.cell])
+        gp, gc = torch.autograd.grad(e.sum(), [d.pos, d.cell], retain_graph=trainable)
         out.append((e.detach(), gp, gc))
+        if trainable:
+            model.zero_grad()
+            e.sum().backward()
+            wgrads.append({k: q.grad.clone() for k, q in model.named_parameters() if "rbf_proj" in k})
     fresh = model.build_graph(pos2, Z, cell)
     assert fresh.n_edges != g_plain.n_edges or True
     assert util.rel_err(out[0][0], out[1][0]) < 2e-6
     assert float((out[0][1] - out[1][1]).abs().max()) < 2e-5 * max(1.0, float(out[1][1].abs().max()))
     assert float((out[0][2] - out[1][2]).abs().max()) < 2e-4 * max(1.0, float(out[1][2].abs().max()))
+    if trainable:
+        assert len(wgrads[1]) == 8          # 2 layers x 2 sub-networks x (weight, bias)
+        for k, ref in wgrads[1].items():
+            assert float((wgrads[0][k] - ref).abs().max()) < 2e-4 * float(ref.abs().max()), k
 
 
 def test_device_md_reuses_the_verlet_list(emu):

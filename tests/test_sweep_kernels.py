@@ -39,11 +39,13 @@ def _run(variant, g, p, geom, xh, vec, Wt, bias, off, g_dx, g_dvec):
     return dx, dv, gg, gxh, gvec
 
 
-def _dense_reference(g, p, geom, xh, vec, Wt, bias, off, g_dx, g_dvec):
-    """float64, all K basis functions, autograd for the three gradients."""
+def _dense_reference(g, p, geom, xh, vec, Wt, bias, off, g_dx, g_dvec, filter_grads=False):
+    """float64, all K basis functions, autograd for the three gradients (``filter_grads``: and for ``Wt`` / ``bias``,
+    appended to the result)."""
     F = p.hidden
     dd = lambda t: t.detach().double()
     xh64, vec64, geom64 = dd(xh).requires_grad_(True), dd(vec).requires_grad_(True), dd(geom).requires_grad_(True)
+    Wt64, bias64 = dd(Wt).requires_grad_(filter_grads), dd(bias).requires_grad_(filter_grads)
     row = g.edge_row.long()
     mod = g.row_mod.long()[row]
     live = mod >= 0
@@ -53,7 +55,7 @@ def _dense_reference(g, p, geom, xh, vec, Wt, bias, off, g_dx, g_dvec):
     a, b, c = -(pe + 1) * (pe + 2) / 2, pe * (pe + 2), -pe * (pe + 1) / 2
     env = torch.where(u < 1, 1 + a * u ** pe + b * u ** (pe + 1) + c * u ** (pe + 2), torch.zeros_like(u))
     emb = env[:, None] * torch.exp(float(p.coeff) * (u[:, None] - dd(off)[None, :]) ** 2)
-    phi = torch.einsum("ek,ekc->ec", emb, dd(Wt)[m]) + dd(bias)[m]
+    phi = torch.einsum("ek,ekc->ec", emb, Wt64[m]) + bias64[m]
     P = xh64[g.row_xoff.long()[row] + g.col.long()]
     V = vec64[g.col.long()]
     A, B, C = torch.split(P * phi, F, dim=-1)
@@ -62,6 +64,9 @@ def _dense_reference(g, p, geom, xh, vec, Wt, bias, off, g_dx, g_dvec):
     dx = torch.zeros((g.n_rows, F), dtype=torch.float64, device=xh.device).index_add_(0, row, A * w)
     dv = torch.zeros((g.n_rows, 3, F), dtype=torch.float64, device=xh.device).index_add_(0, row, mv * w[:, :, None])
     loss = (dx * dd(g_dx)).sum() + (dv * dd(g_dvec)).sum()
+    if filter_grads:
+        gxh, gvec, gg, gW, gb = torch.autograd.grad(loss, [xh64, vec64, geom64, Wt64, bias64])
+        return dx.detach(), dv.detach(), gg, gxh, gvec, gW, gb
     gxh, gvec, gg = torch.autograd.grad(loss, [xh64, vec64, geom64])
     return dx.detach(), dv.detach(), gg, gxh, gvec
 
