@@ -4,6 +4,7 @@
 #include <stdint.h>
 #include <stdio.h>
 #include <string>
+#include <type_traits>
 
 #include "../../include/hermnet_b200.h"
 
@@ -34,6 +35,13 @@ inline int check_launch(const char *where) {
     } while (0)
 
 inline int64_t align_up(int64_t x, int64_t a) { return (x + a - 1) / a * a; }
+
+// Runtime flag -> template argument: calls f(std::true_type{}) or f(std::false_type{}).
+template <class Fn>
+inline void dispatch_bool(bool b, Fn &&f) {
+    if (b) f(std::true_type{});
+    else f(std::false_type{});
+}
 
 inline int num_sms() {
     static int cached = 0;

@@ -19,6 +19,8 @@
 // These row kernels are the fallback for F % 32 == 0 outside {64, 128, 256, 512} and the A/B partner of the tile-sweep
 // kernels of hn_edge_quad.cu, which share one band sweep between consecutive edges of a row and are the default
 // (hn_edge_params.variant = 1 selects these).
+// Verlet-skin superset lists (flags bit 0): the MASKED instantiations skip an entry whose geom[e].w < 0 (the caller stores
+// -d for the entries that are not edges now) before its gathers and band; MASKED = false is the unmasked kernel unchanged.
 #include <cstdlib>
 #include <cstring>
 
@@ -67,7 +69,7 @@ __device__ __forceinline__ int band_setup(float u, const hn_edge_params &P, cons
     return k0;
 }
 
-template <int VEC>
+template <int VEC, bool MASKED>
 __global__ void __launch_bounds__(256)
 edge_fwd_kernel(const hn_edge_params P, const float *__restrict__ xh, const float *__restrict__ vec,
                 const float4 *__restrict__ geom, const int *__restrict__ rowptr, const int *__restrict__ col,
@@ -97,6 +99,7 @@ edge_fwd_kernel(const hn_edge_params P, const float *__restrict__ xh, const floa
         for (int e = e0; e < e1; ++e) {
             const int s = __ldg(col + e);
             const float4 g = __ldg(geom + e);
+            if (MASKED && g.w < 0.f) continue;     // dead entry of a Verlet-skin list: no gathers, no band
             const float *xs = xm + (size_t)s * F3;
             const Vec<VEC> Pa = ldv<VEC>(xs), Pb = ldv<VEC>(xs + F), Pc = ldv<VEC>(xs + 2 * F);
             Vec<VEC> V0 = vzero, V1 = vzero, V2 = vzero;
@@ -152,7 +155,7 @@ edge_fwd_kernel(const hn_edge_params P, const float *__restrict__ xh, const floa
 }
 
 // Destination-major backward: per row-edge (dL/du, dL/dd) for this channel slice.
-template <int VEC>
+template <int VEC, bool MASKED>
 __global__ void __launch_bounds__(256)
 edge_bwd_dst_kernel(const hn_edge_params P, const float *__restrict__ xh, const float *__restrict__ vec,
                     const float4 *__restrict__ geom, const int *__restrict__ rowptr, const int *__restrict__ col,
@@ -182,6 +185,10 @@ edge_bwd_dst_kernel(const hn_edge_params P, const float *__restrict__ xh, const 
     for (int e = e0; e < e1; ++e) {
         const int s = __ldg(col + e);
         const float4 g = __ldg(geom + e);
+        if (MASKED && g.w < 0.f) {             // dead entry of a Verlet-skin list: exact zeros, no gathers, no band
+            if (lane == 0) out[e] = make_float4(0.f, 0.f, 0.f, 0.f);
+            continue;
+        }
         const float *xs = xm + (size_t)s * F3;
         const Vec<VEC> Pa = ldv<VEC>(xs), Pb = ldv<VEC>(xs + F), Pc = ldv<VEC>(xs + 2 * F);
         Vec<VEC> V0, V1, V2;
@@ -240,7 +247,7 @@ edge_bwd_dst_kernel(const hn_edge_params P, const float *__restrict__ xh, const 
 
 // Source-major backward over the transposed view: grad_xh[m][s] (+=, buffer zero-filled by the caller;
 // each (m, s) row is only ever touched by the warp that owns s) and grad_vec[s].
-template <int VEC>
+template <int VEC, bool MASKED>
 __global__ void __launch_bounds__(256)
 edge_bwd_src_kernel(const hn_edge_params P, const float *__restrict__ xh, const float *__restrict__ vec,
                     const float4 *__restrict__ geom, const int *__restrict__ t_rowptr, const int *__restrict__ t_eid,
@@ -287,6 +294,7 @@ edge_bwd_src_kernel(const hn_edge_params P, const float *__restrict__ xh, const 
     const int q0 = __ldg(t_rowptr + s), q1 = __ldg(t_rowptr + s + 1);
     for (int q = q0; q < q1; ++q) {
         const int e = __ldg(t_eid + q);
+        if (MASKED && __ldg(&geom[e].w) < 0.f) continue;    // dead entry of a Verlet-skin list
         const int row = __ldg(edge_row + e);
         const int m = __ldg(row_mod + row);
         if (m < 0) continue;
@@ -429,15 +437,14 @@ edge_bwd_w_kernel(const hn_edge_params P, const float *__restrict__ xh, const fl
 
 int pick_vec(int F) { return F % 128 == 0 ? 4 : (F % 64 == 0 ? 2 : (F % 32 == 0 ? 1 : 0)); }
 
-// masked_ok: the entry point takes a live mask and honours flags bit 0 (Verlet-skin superset lists)
-int validate(const char *where, const hn_edge_params *p, bool masked_ok = false) {
+// Every entry point honours flags bit 0 (Verlet-skin superset lists): the row and tile-sweep kernels read the mask from the
+// sign of geom[e].w, hn_painn_edge_bwd_w from its live argument.
+int validate(const char *where, const hn_edge_params *p) {
     HN_REQUIRE(p != nullptr, where, "null params");
     HN_REQUIRE(pick_vec(p->hidden) != 0, where, "hidden_channels must be a multiple of 32");
     HN_REQUIRE(p->num_rbf >= 2, where, "num_rbf must be >= 2");
     HN_REQUIRE(p->env_p >= 1, where, "envelope exponent must be >= 1");
     HN_REQUIRE(p->n_modules >= 1, where, "n_modules must be >= 1");
-    HN_REQUIRE(masked_ok || !(p->flags & 1), where,
-               "Verlet-skin superset lists (flags bit 0) are only supported by the hn_tc_edge_* kernels and hn_painn_edge_bwd_w");
     return 0;
 }
 
@@ -460,12 +467,16 @@ extern "C" int32_t hn_painn_edge_num_slices(int32_t hidden, int32_t variant) {
     return row_slices(hidden);
 }
 
-#define HN_DISPATCH_VEC(F, CALL)            \
-    switch (pick_vec(F)) {                  \
-        case 4: { constexpr int VEC = 4; CALL; break; } \
-        case 2: { constexpr int VEC = 2; CALL; break; } \
-        default: { constexpr int VEC = 1; CALL; break; } \
-    }
+// VEC from F; MASKED from flags bit 0 (Verlet-skin superset list, dead entries stored as -d in geom)
+#define HN_DISPATCH_VEC(F, FLAGS, CALL)                                         \
+    hn::dispatch_bool((FLAGS) & 1, [&](auto masked_) {                          \
+        constexpr bool MASKED = decltype(masked_)::value;                       \
+        switch (pick_vec(F)) {                                                  \
+            case 4: { constexpr int VEC = 4; CALL; break; }                     \
+            case 2: { constexpr int VEC = 2; CALL; break; }                     \
+            default: { constexpr int VEC = 1; CALL; break; }                    \
+        }                                                                       \
+    })
 
 extern "C" int hn_painn_edge_fwd(const hn_edge_params *p, const float *xh, const float *vec, const float *geom,
                                  const int32_t *rowptr, const int32_t *col, const int32_t *row_mod, const int64_t *row_xoff,
@@ -480,7 +491,7 @@ extern "C" int hn_painn_edge_fwd(const hn_edge_params *p, const float *xh, const
     }
     const int wpb = 8;
     dim3 grid((p->n_rows + wpb - 1) / wpb, row_slices(p->hidden));
-    HN_DISPATCH_VEC(p->hidden, (edge_fwd_kernel<VEC><<<grid, 32 * wpb, 0, (cudaStream_t)stream>>>(
+    HN_DISPATCH_VEC(p->hidden, p->flags, (edge_fwd_kernel<VEC, MASKED><<<grid, 32 * wpb, 0, (cudaStream_t)stream>>>(
                                    *p, xh, vec, (const float4 *)geom, rowptr, col, row_mod, (const long long *)row_xoff, Wt, bias, offset, dx,
                                    dvec)));
     return hn::check_launch(where);
@@ -500,7 +511,7 @@ extern "C" int hn_painn_edge_bwd_dst(const hn_edge_params *p, const float *xh, c
     }
     const int wpb = 8;
     dim3 grid((p->n_rows + wpb - 1) / wpb, row_slices(p->hidden));
-    HN_DISPATCH_VEC(p->hidden, (edge_bwd_dst_kernel<VEC><<<grid, 32 * wpb, 0, (cudaStream_t)stream>>>(
+    HN_DISPATCH_VEC(p->hidden, p->flags, (edge_bwd_dst_kernel<VEC, MASKED><<<grid, 32 * wpb, 0, (cudaStream_t)stream>>>(
                                    *p, xh, vec, (const float4 *)geom, rowptr, col, row_mod, (const long long *)row_xoff, Wt, bias, offset,
                                    g_dx, g_dvec, (float4 *)g_geom, n_edges)));
     return hn::check_launch(where);
@@ -521,7 +532,7 @@ extern "C" int hn_painn_edge_bwd_src(const hn_edge_params *p, const float *xh, c
     }
     const int wpb = 8;
     dim3 grid((p->n_atoms + wpb - 1) / wpb, row_slices(p->hidden));
-    HN_DISPATCH_VEC(p->hidden, (edge_bwd_src_kernel<VEC><<<grid, 32 * wpb, 0, (cudaStream_t)stream>>>(
+    HN_DISPATCH_VEC(p->hidden, p->flags, (edge_bwd_src_kernel<VEC, MASKED><<<grid, 32 * wpb, 0, (cudaStream_t)stream>>>(
                                    *p, xh, vec, (const float4 *)geom, t_rowptr, t_eid, edge_row, row_mod, (const long long *)row_xoff, Wt,
                                    bias, offset, g_dx, g_dvec, grad_xh, grad_vec)));
     return hn::check_launch(where);
@@ -532,7 +543,7 @@ extern "C" int hn_painn_edge_bwd_w(const hn_edge_params *p, const float *xh, con
                                    const uint8_t *live, const float *offset, const float *g_dx, const float *g_dvec,
                                    float *gW_part, float *gb_part, int32_t n_chunks, void *stream) {
     const char *where = "hn_painn_edge_bwd_w";
-    if (int rc = validate(where, p, true)) return rc;
+    if (int rc = validate(where, p)) return rc;
     HN_REQUIRE(!(p->flags & 1) || live != nullptr, where, "a Verlet-skin list (flags bit 0) needs the live mask");
     HN_REQUIRE(n_chunks >= 1, where, "n_chunks must be >= 1");
     // column slice: the widest multiple of 32 (F % 32 == 0, so 3F is one) up to 384 whose [K][cols] fp32 accumulator fits in

@@ -18,7 +18,9 @@
 //     tile span more than 64 basis functions (rows that are no longer distance-sorted because the graph is re-used
 //     after the atoms moved) the tile falls back to a single edge: sharing is lost, accuracy never;
 //   * accumulation per row stays private to the warp: no atomics, deterministic order;
-//   * F is a template parameter, so every address inside the sweep is base + immediate.
+//   * F is a template parameter, so every address inside the sweep is base + immediate;
+//   * Verlet-skin superset lists (flags bit 0, geom.w = -d on the dead entries) run the MASKED instantiations: a dead entry
+//     is padding to its tile (no band, no gathers, exact-zero g_geom) and is dropped by the source-major pipeline.
 #include "hn_common.cuh"
 #include "hn_edge_quad.cuh"
 
@@ -102,13 +104,15 @@ __device__ __forceinline__ void envelope(float u, int p, float &env, float &denv
     if (DERIV) denv = a * (float)p * um + b * (float)(p + 1) * u0 + c * (float)(p + 2) * u1;
 }
 
-// Edge eb + (lane % T) of the row: source atom and geometry (zeros past the end of the row).
+// Edge eb + (lane % T) of the row: source atom and geometry (zeros past the end of the row).  MASKED: a dead entry of a
+// Verlet-skin list (geom.w = -d < 0) gets s = -1 like the padding past the row end, so it adds nothing to the tile's band
+// union and takes no gathers; it still counts as one of the tile's edges.
 template <int T>
 struct Head {
     float4 g;
     int s;
 };
-template <int T>
+template <int T, bool MASKED>
 __device__ __forceinline__ Head<T> load_head(const float4 *__restrict__ geom, const int *__restrict__ col, int eb, int e1,
                                              int lane) {
     Head<T> h;
@@ -118,6 +122,7 @@ __device__ __forceinline__ Head<T> load_head(const float4 *__restrict__ geom, co
     if (e < e1) {
         h.g = __ldg(geom + e);
         h.s = __ldg(col + e);
+        if (MASKED && h.g.w < 0.f) h.s = -1;
     }
     return h;
 }
@@ -198,7 +203,7 @@ __device__ __forceinline__ void load_pairs(const float *tab_row, u64 (&gg)[T]) {
 // forward.  One warp = one (row, slice of 64*NP channels); the slices of a row sit in the same CTA.
 // ---------------------------------------------------------------------------------------------------------------
 // HV = false: vec is identically zero (first layer, hermnet.py:124): the b part of the filter and the vec gathers vanish.
-template <int F, int NP, bool HV>
+template <int F, int NP, bool HV, bool MASKED>
 __global__ void __launch_bounds__(32 * kWarps, 2)
 edge_fwd_quad_kernel(const hn_edge_params P, const float *__restrict__ xh, const float *__restrict__ vec,
                      const float4 *__restrict__ geom, const int *__restrict__ rowptr, const int *__restrict__ col,
@@ -225,12 +230,12 @@ edge_fwd_quad_kernel(const hn_edge_params P, const float *__restrict__ xh, const
         const float *bm = bias + (size_t)m * F3 + ch;
         const float c1 = 1.0f / sqrtf(3.0f * (float)F), c2 = 1.0f / sqrtf((float)F);
         int eb = e0;
-        Head<T> h = load_head<T>(geom, col, eb, e1, lane);
+        Head<T> h = load_head<T, MASKED>(geom, col, eb, e1, lane);
         while (eb < e1) {
             int kmin;
             u64 mask;
             const int cnt = tile_setup<T, false>(P, offset, h, e1 - eb, lane, tab, kmin, mask);
-            const Head<T> hn = load_head<T>(geom, col, eb + cnt, e1, lane);    // next tile's head, in flight during the sweep
+            const Head<T> hn = load_head<T, MASKED>(geom, col, eb + cnt, e1, lane);    // next tile's head, in flight during the sweep
             u64 fa[T][NP], fb[T][NP], fc[T][NP];
             {
                 const Pairs<NP> ba = ldp<NP>(bm), bb = ldp<NP>(bm + F), bc = ldp<NP>(bm + 2 * F);
@@ -341,7 +346,7 @@ edge_fwd_quad_kernel(const hn_edge_params P, const float *__restrict__ xh, const
                     }
                 }
             };
-            if constexpr (!HV || HN_FWD_PIPE) {
+            if constexpr ((!HV || HN_FWD_PIPE) && !MASKED) {
             gather(0, G0, U0);
             if (cnt > 1) gather(1, G1, U1);
             fold(0, G0, U0);
@@ -355,9 +360,11 @@ edge_fwd_quad_kernel(const hn_edge_params P, const float *__restrict__ xh, const
                 }
             }
             } else {
+                // MASKED: lane j < T holds edge j of the tile; a dead edge (s < 0) is neither gathered nor folded
+                const unsigned live = MASKED ? __ballot_sync(kFull, h.s >= 0) : ~0u;
 #pragma unroll
                 for (int j = 0; j < T; ++j)
-                    if (j < cnt) {
+                    if (j < cnt && ((live >> j) & 1u)) {
                         gather(j, G0, U0);
                         fold(j, G0, U0);
                     }
@@ -387,7 +394,7 @@ edge_fwd_quad_kernel(const hn_edge_params P, const float *__restrict__ xh, const
 // registers per edge); the gathers are issued before the sweep, so their latency hides behind it.  The 8 per-tile
 // partial sums (2 edges x 4 values) are reduced across the warp with a halving exchange (8 shuffles instead of 40).
 // ---------------------------------------------------------------------------------------------------------------
-template <int F, int NP, bool HV>
+template <int F, int NP, bool HV, bool MASKED>
 __global__ void __launch_bounds__(32 * kWarps, 2)
 edge_bwd_dst_quad_kernel(const hn_edge_params P, const float *__restrict__ xh, const float *__restrict__ vec,
                          const float4 *__restrict__ geom, const int *__restrict__ rowptr, const int *__restrict__ col,
@@ -428,17 +435,24 @@ edge_bwd_dst_quad_kernel(const hn_edge_params P, const float *__restrict__ xh, c
     }
     const float c1 = 1.0f / sqrtf(3.0f * (float)F), c2 = 1.0f / sqrtf((float)F);
     int eb = e0;
-    Head<T> h = load_head<T>(geom, col, eb, e1, lane);
+    Head<T> h = load_head<T, MASKED>(geom, col, eb, e1, lane);
     while (eb < e1) {
         // gathers of the T edges first (independent of the table), then the table, then the sweep
         Pairs<NP> Pa[T], Pb[T], Pc[T], V0[T], V1[T], V2[T];
         float ux[T], uy[T], uz[T];
+        // MASKED: lane j < T holds edge j of the tile; a dead edge (s < 0) is not gathered and its outputs are exact zeros
+        const unsigned live = MASKED ? __ballot_sync(kFull, h.s >= 0) : ~0u;
 #pragma unroll
         for (int j = 0; j < T; ++j) {
             int sj = __shfl_sync(kFull, h.s, j);
             ux[j] = __shfl_sync(kFull, h.g.x, j);
             uy[j] = __shfl_sync(kFull, h.g.y, j);
             uz[j] = __shfl_sync(kFull, h.g.z, j);
+            if (MASKED && sj < 0) {    // dead or past the row end: zeros feed the sweep, nothing is loaded
+#pragma unroll
+                for (int n = 0; n < NP; ++n) Pa[j].p[n] = Pb[j].p[n] = Pc[j].p[n] = V0[j].p[n] = V1[j].p[n] = V2[j].p[n] = 0ull;
+                continue;
+            }
             if (sj < 0) sj = __shfl_sync(kFull, h.s, 0);   // past the row end: a valid address, the result is discarded
             const float *xs = xm + (size_t)sj * F3;
             const float *vs = vm + (size_t)sj * F3;
@@ -454,7 +468,7 @@ edge_bwd_dst_quad_kernel(const hn_edge_params P, const float *__restrict__ xh, c
         int kmin;
         u64 mask;
         const int cnt = tile_setup<T, true>(P, offset, h, e1 - eb, lane, tab, kmin, mask);
-        const Head<T> hn = load_head<T>(geom, col, eb + cnt, e1, lane);
+        const Head<T> hn = load_head<T, MASKED>(geom, col, eb + cnt, e1, lane);
         u64 qa[T][NP], qb[T][NP], qc[T][NP], fc[T][NP], ds[T];
         float rc_[T][VEC];    // Pc / sqrt(F): the u-independent factor of dL/du
 #pragma unroll
@@ -583,7 +597,8 @@ edge_bwd_dst_quad_kernel(const hn_edge_params P, const float *__restrict__ xh, c
         val[0] += __shfl_xor_sync(kFull, val[0], 1);
         // lane holds the total of value index idx = lane >> 2: edge idx >> 2, component idx & 3
         const int idx = lane >> 2;
-        if ((lane & 3) == 0 && (idx >> 2) < cnt) reinterpret_cast<float *>(out + eb)[idx] = val[0];
+        if ((lane & 3) == 0 && (idx >> 2) < cnt)
+            reinterpret_cast<float *>(out + eb)[idx] = ((live >> (idx >> 2)) & 1u) ? val[0] : 0.f;
         eb += cnt;
         h = hn;
     }
@@ -600,7 +615,7 @@ edge_bwd_dst_quad_kernel(const hn_edge_params P, const float *__restrict__ xh, c
 // band values come from a 12-entry shared-memory table (one LDS.64 per basis function instead of a shuffle) and
 // the FMAs are packed.
 // ---------------------------------------------------------------------------------------------------------------
-template <int F, int NP>
+template <int F, int NP, bool MASKED>
 __global__ void __launch_bounds__(32 * kWarps, 2)
 edge_bwd_src_sweep_kernel(const hn_edge_params P, const float *__restrict__ xh, const float *__restrict__ vec,
                           const float4 *__restrict__ geom, const int *__restrict__ t_rowptr, const int *__restrict__ t_eid,
@@ -684,7 +699,7 @@ edge_bwd_src_sweep_kernel(const hn_edge_params P, const float *__restrict__ xh, 
             gB = __ldg(geom + eA);
         }
         if (q + 3 < q1) eA = __ldg(t_eid + q + 3);
-        if (m >= 0) {
+        if (m >= 0 && (!MASKED || g.w >= 0.f)) {     // MASKED: a dead entry of a Verlet-skin list (g.w = -d) is skipped
             if (off != cur_off) {
                 flush();
                 cur_off = off;
@@ -784,32 +799,37 @@ bool supported(const hn_edge_params *p) { return p->hidden == 64 || p->hidden ==
 
 int bwd_dst_slices(int hidden) { return hidden == 64 ? 1 : hidden / 128; }
 
-#define HN_QUAD_DISPATCH(KERNEL, ...)                                                         \
-    switch (p->hidden) {                                                                      \
-        case 64: KERNEL<64, 1><<<grid(1), 32 * kWarps, 0, stream>>>(__VA_ARGS__); break;      \
-        case 128: KERNEL<128, 2><<<grid(1), 32 * kWarps, 0, stream>>>(__VA_ARGS__); break;    \
-        case 256: KERNEL<256, 2><<<grid(2), 32 * kWarps, 0, stream>>>(__VA_ARGS__); break;    \
-        default: KERNEL<512, 2><<<grid(4), 32 * kWarps, 0, stream>>>(__VA_ARGS__); break;     \
+// MASKED: flags bit 0 (Verlet-skin superset list, dead entries stored as -d in geom), a template argument so that the
+// kernels of plain lists are the ones they were before masking existed
+#define HN_QUAD_DISPATCH(KERNEL, MASKED, ...)                                                         \
+    switch (p->hidden) {                                                                              \
+        case 64: KERNEL<64, 1, MASKED><<<grid(1), 32 * kWarps, 0, stream>>>(__VA_ARGS__); break;      \
+        case 128: KERNEL<128, 2, MASKED><<<grid(1), 32 * kWarps, 0, stream>>>(__VA_ARGS__); break;    \
+        case 256: KERNEL<256, 2, MASKED><<<grid(2), 32 * kWarps, 0, stream>>>(__VA_ARGS__); break;    \
+        default: KERNEL<512, 2, MASKED><<<grid(4), 32 * kWarps, 0, stream>>>(__VA_ARGS__); break;     \
     }
-#define HN_QUAD_DISPATCH_HV(KERNEL, HV, ...)                                                      \
-    switch (p->hidden) {                                                                          \
-        case 64: KERNEL<64, 1, HV><<<grid(1), 32 * kWarps, 0, stream>>>(__VA_ARGS__); break;      \
-        case 128: KERNEL<128, 2, HV><<<grid(1), 32 * kWarps, 0, stream>>>(__VA_ARGS__); break;    \
-        case 256: KERNEL<256, 2, HV><<<grid(2), 32 * kWarps, 0, stream>>>(__VA_ARGS__); break;    \
-        default: KERNEL<512, 2, HV><<<grid(4), 32 * kWarps, 0, stream>>>(__VA_ARGS__); break;     \
+#define HN_QUAD_DISPATCH_HV(KERNEL, HV, MASKED, ...)                                                      \
+    switch (p->hidden) {                                                                                  \
+        case 64: KERNEL<64, 1, HV, MASKED><<<grid(1), 32 * kWarps, 0, stream>>>(__VA_ARGS__); break;      \
+        case 128: KERNEL<128, 2, HV, MASKED><<<grid(1), 32 * kWarps, 0, stream>>>(__VA_ARGS__); break;    \
+        case 256: KERNEL<256, 2, HV, MASKED><<<grid(2), 32 * kWarps, 0, stream>>>(__VA_ARGS__); break;    \
+        default: KERNEL<512, 2, HV, MASKED><<<grid(4), 32 * kWarps, 0, stream>>>(__VA_ARGS__); break;     \
     }
 
 int fwd(const hn_edge_params *p, const float *xh, const float *vec, const float *geom, const int32_t *rowptr,
         const int32_t *col, const int32_t *row_mod, const int64_t *row_xoff, const float *Wt, const float *bias,
         const float *offset, float *dx, float *dvec, cudaStream_t stream) {
     auto grid = [&](int ns) { return (unsigned)(((long long)p->n_rows * ns + kWarps - 1) / kWarps); };
-    if (vec != nullptr) {
-        HN_QUAD_DISPATCH_HV(edge_fwd_quad_kernel, true, *p, xh, vec, (const float4 *)geom, rowptr, col, row_mod,
-                            (const long long *)row_xoff, Wt, bias, offset, dx, dvec)
-    } else {
-        HN_QUAD_DISPATCH_HV(edge_fwd_quad_kernel, false, *p, xh, vec, (const float4 *)geom, rowptr, col, row_mod,
-                            (const long long *)row_xoff, Wt, bias, offset, dx, dvec)
-    }
+    dispatch_bool(p->flags & 1, [&](auto masked) {
+        constexpr bool MASKED = decltype(masked)::value;
+        if (vec != nullptr) {
+            HN_QUAD_DISPATCH_HV(edge_fwd_quad_kernel, true, MASKED, *p, xh, vec, (const float4 *)geom, rowptr, col, row_mod,
+                                (const long long *)row_xoff, Wt, bias, offset, dx, dvec)
+        } else {
+            HN_QUAD_DISPATCH_HV(edge_fwd_quad_kernel, false, MASKED, *p, xh, vec, (const float4 *)geom, rowptr, col, row_mod,
+                                (const long long *)row_xoff, Wt, bias, offset, dx, dvec)
+        }
+    });
     return 0;
 }
 
@@ -817,13 +837,16 @@ int bwd_dst(const hn_edge_params *p, const float *xh, const float *vec, const fl
             const int32_t *col, const int32_t *row_mod, const int64_t *row_xoff, const float *Wt, const float *bias,
             const float *offset, const float *g_dx, const float *g_dvec, float *g_geom, int64_t n_edges, cudaStream_t stream) {
     auto grid = [&](int ns) { return (unsigned)(((long long)p->n_rows * ns + kWarps - 1) / kWarps); };
-    if (vec != nullptr) {
-        HN_QUAD_DISPATCH_HV(edge_bwd_dst_quad_kernel, true, *p, xh, vec, (const float4 *)geom, rowptr, col, row_mod,
-                            (const long long *)row_xoff, Wt, bias, offset, g_dx, g_dvec, (float4 *)g_geom, (long long)n_edges)
-    } else {
-        HN_QUAD_DISPATCH_HV(edge_bwd_dst_quad_kernel, false, *p, xh, vec, (const float4 *)geom, rowptr, col, row_mod,
-                            (const long long *)row_xoff, Wt, bias, offset, g_dx, g_dvec, (float4 *)g_geom, (long long)n_edges)
-    }
+    dispatch_bool(p->flags & 1, [&](auto masked) {
+        constexpr bool MASKED = decltype(masked)::value;
+        if (vec != nullptr) {
+            HN_QUAD_DISPATCH_HV(edge_bwd_dst_quad_kernel, true, MASKED, *p, xh, vec, (const float4 *)geom, rowptr, col, row_mod,
+                                (const long long *)row_xoff, Wt, bias, offset, g_dx, g_dvec, (float4 *)g_geom, (long long)n_edges)
+        } else {
+            HN_QUAD_DISPATCH_HV(edge_bwd_dst_quad_kernel, false, MASKED, *p, xh, vec, (const float4 *)geom, rowptr, col, row_mod,
+                                (const long long *)row_xoff, Wt, bias, offset, g_dx, g_dvec, (float4 *)g_geom, (long long)n_edges)
+        }
+    });
     return 0;
 }
 
@@ -832,8 +855,11 @@ int bwd_src(const hn_edge_params *p, const float *xh, const float *vec, const fl
             const float *bias, const float *offset, const float *g_dx, const float *g_dvec, float *grad_xh, float *grad_vec,
             cudaStream_t stream) {
     auto grid = [&](int ns) { return (unsigned)(((long long)p->n_atoms * ns + kWarps - 1) / kWarps); };
-    HN_QUAD_DISPATCH(edge_bwd_src_sweep_kernel, *p, xh, vec, (const float4 *)geom, t_rowptr, t_eid, edge_row, row_mod,
-                     (const long long *)row_xoff, Wt, bias, offset, g_dx, g_dvec, grad_xh, grad_vec)
+    dispatch_bool(p->flags & 1, [&](auto masked) {
+        constexpr bool MASKED = decltype(masked)::value;
+        HN_QUAD_DISPATCH(edge_bwd_src_sweep_kernel, MASKED, *p, xh, vec, (const float4 *)geom, t_rowptr, t_eid, edge_row, row_mod,
+                         (const long long *)row_xoff, Wt, bias, offset, g_dx, g_dvec, grad_xh, grad_vec)
+    });
     return 0;
 }
 

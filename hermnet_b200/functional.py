@@ -98,7 +98,9 @@ def edge_geometry(pos: Tensor, cell: Optional[Tensor], g: RowGraph) -> Tensor:
 class _PaiNNEdge(Function):
     """Edge side of one layer.  F == 128: the tensor-core kernels of csrc/hn_edge_tc.cu over the graph's tile plans
     (``tileplan``); otherwise the C ABI picks the tile-sweep kernels (F in {64, 256, 512}) or the row-per-warp kernels
-    (any F % 32 == 0)."""
+    (any F % 32 == 0).  Every family takes Verlet-skin superset lists (``p.flags`` bit 0 with the ``p.live`` mask): the
+    entries marked dead contribute nothing, not even the filter bias -- the tensor-core kernels through the tile plans'
+    windows, the others through the signed geometry ``ops`` builds once per evaluation."""
 
     @staticmethod
     def forward(ctx, xh, vec, geom, Wt, bias, offset, g: RowGraph, p, vec_zero=False):
@@ -114,9 +116,6 @@ class _PaiNNEdge(Function):
             dx, dvec = ops.tc_edge_fwd(p, dst, xh, None if ctx.vec_null else vec, geom, wsplit, wscale, bias, offset, p.n_rows)
             ctx.wsplit = (wsplit, wscale)
         else:
-            if p.flags & 1:
-                raise RuntimeError("hermnet_b200: Verlet-skin graphs need the tensor-core edge kernels (hidden_channels == 128) "
-                                   "or the composite path (model.edge_path = 'composite')")
             dx, dvec = ops.painn_edge_fwd(p, xh, None if ctx.vec_null else vec, geom, g, Wt, bias, offset)
         ctx.g, ctx.p = g, p
         ctx.save_for_backward(xh, vec, geom, Wt, bias, offset)

@@ -266,7 +266,35 @@ def edge_use_tc(hidden: int, num_rbf: int) -> bool:
     return EDGE_VARIANT["v"] in ("auto", "tc") and tc_supported(hidden, num_rbf)
 
 
+def _kernel_geom(name: str, p: EdgeParams, geom):
+    """Geometry the row and tile-sweep kernels read: ``geom`` itself, or for a Verlet-skin list (``p.flags`` bit 0) a copy
+    whose distance is ``-d`` on the entries ``p.live`` (uint8 [E]) marks dead -- the sign is how the C ABI passes the mask
+    (a real distance is >= 1e-6).  The copy is cached on ``p``, keyed on the identity and version of ``geom`` and
+    ``p.live``, so that every layer's forward and backward calls of one evaluation share it.  Device ops only: capturable
+    in a CUDA graph."""
+    import weakref
+    if not p.flags & 1:
+        return geom
+    live = getattr(p, "live", None)
+    if not isinstance(live, torch.Tensor) or live.dtype != torch.uint8 or live.numel() != geom.size(0):
+        raise TypeError(f"hermnet_b200.{name}: live must be uint8 [E]")
+    _chk(name, geom, live)
+    stamp = (geom._version, geom.data_ptr(), live._version, live.data_ptr(), tuple(geom.shape))
+    hit = getattr(p, "_signed_geom", None)
+    if hit is not None and hit[0]() is geom and hit[1]() is live and hit[2] == stamp:
+        return hit[3]
+    with torch.no_grad():
+        signed = geom.detach().clone()
+        signed[:, 3] = torch.where(live.bool(), geom[:, 3], -geom[:, 3])
+    p._signed_geom = (weakref.ref(geom), weakref.ref(live), stamp, signed)
+    return signed
+
+
 def painn_edge_fwd(p: EdgeParams, xh, vec, geom, g, Wt, bias, offset):
+    """A Verlet-skin list (``p.flags`` bit 0) needs ``p.live``, as for ``painn_edge_bwd_w``: entries marked 0 contribute
+    nothing, not even the filter bias.  The same holds for ``painn_edge_bwd_dst`` (zero ``g_geom`` rows) and
+    ``painn_edge_bwd_src``."""
+    geom = _kernel_geom("painn_edge_fwd", p, geom)      # first: a missing mask is the error to report
     lib = _lib.load()
     _stamp(p)
     dev = _chk("painn_edge_fwd", xh, vec, geom, Wt, bias, offset)
@@ -282,6 +310,7 @@ def painn_edge_fwd(p: EdgeParams, xh, vec, geom, g, Wt, bias, offset):
 
 
 def painn_edge_bwd_dst(p: EdgeParams, xh, vec, geom, g, Wt, bias, offset, g_dx, g_dvec):
+    geom = _kernel_geom("painn_edge_bwd_dst", p, geom)      # first: a missing mask is the error to report
     lib = _lib.load()
     _stamp(p)
     dev = _chk("painn_edge_bwd_dst", xh, vec, geom, Wt, bias, offset, g_dx, g_dvec)
@@ -295,6 +324,7 @@ def painn_edge_bwd_dst(p: EdgeParams, xh, vec, geom, g, Wt, bias, offset, g_dx, 
 
 
 def painn_edge_bwd_src(p: EdgeParams, xh, vec, geom, g, Wt, bias, offset, g_dx, g_dvec):
+    geom = _kernel_geom("painn_edge_bwd_src", p, geom)      # first: a missing mask is the error to report
     lib = _lib.load()
     _stamp(p)
     dev = _chk("painn_edge_bwd_src", xh, vec, geom, Wt, bias, offset, g_dx, g_dvec)

@@ -135,10 +135,14 @@ typedef struct {
     float coeff;          /* Gaussian coefficient */
     int32_t variant;      /* kernel family of hn_painn_edge_{fwd,bwd_dst,bwd_src}: 0 = auto (quad-tile kernels for F % 64 == 0,
                              else row-per-warp), 1 = row-per-warp only (A/B measurements).  Per call: no library state. */
-    int32_t flags;        /* bit 0: the edge list is a Verlet-skin SUPERSET (built with rc + skin): the entries marked dead
-                             by hn_tc_tile_windows(live) must contribute nothing -- not even the filter bias (rmnet.py:55:
-                             the reference has no such edge).  Honoured by the hn_tc_edge_* kernels and by
-                             hn_painn_edge_bwd_w (through its live argument); the other families reject it. */
+    int32_t flags;        /* bit 0: the edge list is a Verlet-skin SUPERSET (built with rc + skin): its dead entries must
+                             contribute nothing -- not even the filter bias (rmnet.py:55: the reference has no such edge).
+                             Every family reads the mask from its own input:
+                               hn_tc_edge_*: the sign of tile_geom[.].w (-d for dead, written by hn_tc_tile_windows(live));
+                               hn_painn_edge_{fwd,bwd_dst,bwd_src}: the sign of geom[e].w (the caller stores -d for a
+                                 dead entry; a real distance is >= 1e-6).  bwd_dst writes exact zeros to the g_geom rows
+                                 of dead entries in every slice plane;
+                               hn_painn_edge_bwd_w, hn_layer0_basis_*: their live argument (uint8 [E]). */
 } hn_edge_params;
 
 /* Planes of g_geom that hn_painn_edge_bwd_dst writes for this F and kernel family (the caller sums them); 0 = unsupported F. */
