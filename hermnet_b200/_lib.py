@@ -44,6 +44,7 @@ SIGNATURES = {
     "hn_triplet_dots": (c_int32, [P, c_int32, P, P, P, c_int32, P, P]),
     "hn_edge_geom_fwd": (c_int32, [P, P, P, P, c_int32, P, P, c_float, c_int64, P, P]),
     "hn_edge_geom_bwd": (c_int32, [P, P, c_int32, P, P, c_int32, P, P, c_float, c_int64, c_int64, P, P, P]),
+    "hn_edge_virial_atom": (c_int32, [P, P, P, c_int32, P, P, c_int64, c_int64, P, P]),
     "hn_painn_edge_num_slices": (c_int32, [c_int32, c_int32]),
     "hn_painn_edge_fwd": (c_int32, [POINTER(EdgeParams)] + [P] * 13),
     "hn_painn_edge_bwd_dst": (c_int32, [POINTER(EdgeParams)] + [P] * 13 + [c_int64, P]),

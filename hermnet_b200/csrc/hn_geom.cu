@@ -92,6 +92,34 @@ __global__ void edge_geom_bwd_kernel(const float4 *__restrict__ geom, const floa
     }
 }
 
+// per-atom virial: every row-edge e gives -1/2 D_e (x) gD_e to each endpoint, D_e = d * u (clamped edges too).  Same
+// traversal as edge_geom_bwd_kernel (row CSR, then its transpose), so the summation order is fixed
+__global__ void edge_virial_atom_kernel(const float4 *__restrict__ geom, const float4 *__restrict__ g_geom,
+                                        const int *__restrict__ rowptr, int rows_per_atom, const int *__restrict__ t_rowptr,
+                                        const int *__restrict__ t_eid, int n_atoms, long long n_edges,
+                                        float *__restrict__ virial) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n_atoms) return;
+    float w[9];
+#pragma unroll
+    for (int k = 0; k < 9; ++k) w[k] = 0.f;
+    auto add = [&](long long e) {
+        const float4 g = __ldg(geom + e);
+        const float3 gD = edge_grad_D(geom, g_geom, 1, n_edges, e);
+        const float D[3] = {g.w * g.x, g.w * g.y, g.w * g.z};
+#pragma unroll
+        for (int a = 0; a < 3; ++a) {
+            w[3 * a] += D[a] * gD.x; w[3 * a + 1] += D[a] * gD.y; w[3 * a + 2] += D[a] * gD.z;
+        }
+    };
+    const int e0 = rowptr[(size_t)i * rows_per_atom], e1 = rowptr[(size_t)(i + 1) * rows_per_atom];
+    for (int e = e0; e < e1; ++e) add(e);
+    const int q0 = t_rowptr[i], q1 = t_rowptr[i + 1];
+    for (int q = q0; q < q1; ++q) add(t_eid[q]);
+#pragma unroll
+    for (int k = 0; k < 9; ++k) virial[9 * (size_t)i + k] = -0.5f * w[k];
+}
+
 __global__ void gather_rows_kernel(const float *__restrict__ X, const int *__restrict__ idx, long long total, int C,
                                    float *__restrict__ out) {
     long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
@@ -185,6 +213,16 @@ extern "C" int hn_edge_geom_bwd(const float *geom, const float *g_geom, int32_t 
         (const float4 *)geom, (const float4 *)g_geom, n_parts, (const char4 *)shift, rowptr, rows_per_atom, t_rowptr, t_eid,
         sign, (int)n_atoms, n_edges, grad_pos, cellw);
     return hn::check_launch("hn_edge_geom_bwd");
+}
+
+extern "C" int hn_edge_virial_atom(const float *geom, const float *g_geom, const int32_t *rowptr, int32_t rows_per_atom,
+                                   const int32_t *t_rowptr, const int32_t *t_eid, int64_t n_atoms, int64_t n_edges,
+                                   float *virial, void *stream) {
+    if (n_atoms <= 0) return 0;
+    HN_REQUIRE(rows_per_atom >= 1, "hn_edge_virial_atom", "rows_per_atom must be >= 1");
+    edge_virial_atom_kernel<<<(unsigned)((n_atoms + 127) / 128), 128, 0, (cudaStream_t)stream>>>(
+        (const float4 *)geom, (const float4 *)g_geom, rowptr, rows_per_atom, t_rowptr, t_eid, (int)n_atoms, n_edges, virial);
+    return hn::check_launch("hn_edge_virial_atom");
 }
 
 extern "C" int hn_gather_rows(const float *X, const int32_t *idx, int64_t n_out, int32_t C, float *out, void *stream) {

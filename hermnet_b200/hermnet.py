@@ -159,21 +159,61 @@ class _HermNet(nn.Module):
         pos = data.pos
         ops.require_cuda(pos, f"{self.KIND}.forward")
         g = self._graph_of(data)
-        cell = data.get("cell")
-        if cell is not None and data.get("edge_shift") is None and data.get("edge_index") is not None:
-            cell = None               # hermnet.py:138: the shift term needs both cell and edge_shift
-        if cell is not None:
-            cell = cell.reshape(-1, 3, 3)
-        energy, x, vec = self.forward_graph(pos, data.atomic_number, cell, g)
+        energy, x, vec = self.forward_graph(pos, data.atomic_number, self._cell_of(data), g)
         if self.store_features:
             data.x, data.vec = x[g.inv_perm], vec[g.inv_perm]
         return energy
+
+    @staticmethod
+    def _cell_of(data):
+        cell = data.get("cell")
+        if cell is not None and data.get("edge_shift") is None and data.get("edge_index") is not None:
+            cell = None               # hermnet.py:138: the shift term needs both cell and edge_shift
+        return None if cell is None else cell.reshape(-1, 3, 3)
+
+    def energy_forces_virial(self, data) -> Dict[str, torch.Tensor]:
+        """Energies, forces, per-atom energies and per-atom / per-graph virials of ``data`` from ONE backward pass
+        (first order; detached device tensors, caller's atom order):
+
+        ``energy [G]`` (= ``model(data)``), ``forces [N,3]`` (-dE/dpos), ``energies [N]`` (readout energy of each atom; with
+        ``intensive`` divided by its graph's atom count, so they always sum to ``energy``), ``virials [N,3,3]`` and
+        ``virial [G,3,3]``.  ``virial[g] = sum_i pos_i (x) F_i - cell^T dE/dcell`` (row = position component, not
+        symmetrised), obtained as ``-sum_e D_e (x) dE/dD_e`` over the edge vectors.  ``virials[i]`` gives each edge's term
+        half to each of its two atoms: a convention, as for any many-body potential -- an atom's share is not unique, the
+        per-graph sums are.  It is not a heat-flux estimator for this message-passing model."""
+        ops.require_cuda(data.pos, f"{self.KIND}.energy_forces_virial")
+        g = self._graph_of(data)
+        return self.energy_forces_virial_graph(data.pos, data.atomic_number, self._cell_of(data), g)
+
+    def energy_forces_virial_graph(self, pos, atomic_number, cell, g: RowGraph) -> Dict[str, torch.Tensor]:
+        """``energy_forces_virial`` on a prebuilt ``RowGraph`` (``forward_graph``'s arguments)."""
+        pos_leaf = pos.detach().requires_grad_(True)
+        with torch.enable_grad():
+            energy, _, _, geom, e_atom = self._forward_graph(pos_leaf, atomic_number,
+                                                             None if cell is None else cell.detach(), g)
+            grad_pos, g_geom = torch.autograd.grad(energy.sum(), (pos_leaf, geom), allow_unused=True)
+        if g_geom is None:            # no edges: the energy does not depend on the geometry
+            g_geom = torch.zeros_like(geom)
+        virials = ops.edge_virial_atom(geom.detach().float().contiguous(), g_geom.float().contiguous(), g)
+        sb = g.seg_batch
+        virial = ops.segment_sum(virials, sb.rowptr, sb.perm, sb.n_rows)[: g.n_graphs].view(-1, 3, 3)
+        e_atom = e_atom.detach().squeeze(1)
+        if self.intensive:
+            e_atom = e_atom / (sb.rowptr[1:] - sb.rowptr[:-1]).clamp(min=1).to(e_atom.dtype)[g.atom_graph.long()]
+        inv = g.inv_perm
+        return {"energy": energy.detach(), "forces": -grad_pos, "energies": e_atom[inv],
+                "virials": virials.view(-1, 3, 3)[inv], "virial": virial}
 
     def forward_graph(self, pos, atomic_number, cell, g: RowGraph, halo=None, atom_weight=None):
         """Hot path on a prebuilt ``RowGraph``: energies ``[num_graphs]`` plus final features (internal order).
         ``halo`` (domain decomposition, ``parallel.Halo``) refreshes the ghost rows between layers.
         ``atom_weight [N]`` (caller's atom order): the readout sums ``w_i e_i`` instead of ``e_i`` -- partial energies of a
         region, whose gradient only involves atoms within ``num_layers * rc`` of it (used by the cut-out parity check)."""
+        return self._forward_graph(pos, atomic_number, cell, g, halo, atom_weight)[:3]
+
+    def _forward_graph(self, pos, atomic_number, cell, g: RowGraph, halo=None, atom_weight=None):
+        """``forward_graph`` plus the edge geometry ``geom [E,4]`` (the only way positions and cell enter the energy) and
+        the readout energies ``e_atom [N,1]`` (internal order)."""
         F = self.hidden_channels
         fused = self._use_fused(pos)
         pos_i = pos[g.perm]
@@ -221,7 +261,7 @@ class _HermNet(nn.Module):
             for t in (pos, cell):
                 if t is not None and t.requires_grad:
                     energy = energy + 0.0 * t.sum()
-        return energy, x, vec
+        return energy, x, vec, geom, e_atom
 
     # ------------------------------------------------------------------------------------------------
     def _layer(self, conv, x, vec, geom, g: RowGraph, p, vec_zero: bool = False, z0=None, ckpt: bool = False, live=None):

@@ -228,6 +228,22 @@ def edge_geom_bwd(geom: Tensor, g_geom: Tensor, g, want_cell: bool):
     return grad_pos, cellw
 
 
+def edge_virial_atom(geom: Tensor, g_geom: Tensor, g) -> Tensor:
+    """Per-atom virial ``[N, 9]`` (internal atom order, row = position component) from ``geom [E,4]`` and its gradient
+    ``g_geom [E,4]``: each edge gives ``-1/2 D_e (x) dE/dD_e`` to both of its atoms."""
+    lib = _lib.load()
+    dev = _chk("edge_virial_atom", geom, g_geom)
+    _f32("edge_virial_atom", geom, g_geom)
+    if tuple(geom.shape) != (g.n_edges, 4) or tuple(g_geom.shape) != (g.n_edges, 4):
+        raise RuntimeError(f"hermnet_b200.edge_virial_atom: geom / g_geom must be [{g.n_edges}, 4]")
+    virial = torch.empty((g.n_atoms, 9), dtype=torch.float32, device=dev)
+    with torch.cuda.device(dev), _timed("edge_virial_atom", dev):
+        _lib.check(lib.hn_edge_virial_atom(_ptr(geom), _ptr(g_geom), _ptr(g.rowptr), g.rows_per_atom, _ptr(g.t_rowptr),
+                                           _ptr(g.t_eid), g.n_atoms, g.n_edges, _ptr(virial), _stream(dev)),
+                   "hn_edge_virial_atom")
+    return virial
+
+
 # ----------------------------------------------------------------------------------------------------
 # fused PaiNN edge kernels
 # ----------------------------------------------------------------------------------------------------

@@ -18,7 +18,7 @@ from torch import nn
 
 from ..data import Data
 from ..symbols import atomic_numbers
-from ..utils import virial_calc
+from ..utils import NKTV2P, virial_calc
 
 try:  # pragma: no cover - ASE is absent from the build image
     from ase.calculators.calculator import Calculator, all_changes
@@ -46,6 +46,14 @@ except Exception:  # noqa: BLE001
             self.calculate(atoms or self.atoms, ["stress"])
             return self.results["stress"]
 
+        def get_potential_energies(self, atoms=None):
+            self.calculate(atoms or self.atoms, ["energies"])
+            return self.results["energies"]
+
+        def get_stresses(self, atoms=None):
+            self.calculate(atoms or self.atoms, ["stresses"])
+            return self.results["stresses"]
+
 
 def build_graph(cell, elements, pos, rc, device="cuda"):
     """calculator.py:10-27 made functional: numpy in, device-resident ``Data`` out.  The neighbour list is NOT built
@@ -59,7 +67,7 @@ def build_graph(cell, elements, pos, rc, device="cuda"):
 
 
 class NNCalculator(Calculator):
-    implemented_properties = ['energy', 'free_energy', 'forces', 'stress']
+    implemented_properties = ['energy', 'free_energy', 'forces', 'stress', 'energies', 'stresses']
 
     def __init__(self, model: nn.Module, model_path: Optional[str], trn_mean: float, device_: str = 'cuda',
                  ensemble: str = 'NVT', compat_stress: bool = False, skin: float = 0.0):
@@ -87,6 +95,9 @@ class NNCalculator(Calculator):
         pbc = bool(np.any(atoms.pbc))
         data = build_graph(cell=cell if pbc else None, elements=elems, pos=atoms.positions, rc=self.model.rc,
                            device=self.device_)
+        if properties is not None and ('energies' in properties or 'stresses' in properties):
+            self.results.update(self.model_calc_per_atom(data, self.device_, pbc))
+            return
         energy, forces, virial = self.model_calc(data=data, device=self.device_, pbc=pbc, ensemble=self.ensemble)
         self.results['energy'] = energy
         self.results['free_energy'] = energy
@@ -95,9 +106,7 @@ class NNCalculator(Calculator):
 
     def model_calc(self, data, device, pbc, ensemble='NVT'):
         """calculator.py:59-99: ``(float energy, ndarray[N,3] forces, ndarray[6] virial)``."""
-        data = data.to(torch.device(device))
-        if pbc and self.verlet.skin > 0.0 and data.get("edge_index") is None:
-            data.graph = self.verlet.get(data.pos, data.atomic_number, data.get("cell"))
+        data = self._prepare(data, device, pbc)
         data.pos.requires_grad_(True)
         npt = ensemble.lower() == 'npt'
         if npt and pbc:
@@ -108,10 +117,34 @@ class NNCalculator(Calculator):
             cell = data.cell if pbc else None
             v = virial_calc(cell=cell, pos=data.pos.detach(), forces=forces, energy=energy, units='metal',
                             pbc=pbc).detach().cpu().numpy()
-            if self.compat_stress:   # the reference's ordering, kept for bit-compatibility with its consumers
-                virial = np.array([v[0, 1], v[1, 1], v[2, 2], v[0, 1], v[0, 2], v[1, 2]])
-            else:
-                virial = np.array([v[0, 0], v[1, 1], v[2, 2], v[1, 2], v[0, 2], v[0, 1]])
+            virial = self._stress_vector(v)
         else:
             virial = np.array([0., 0., 0., 0., 0., 0.], dtype=np.float32)
         return energy.detach().cpu().item(), forces.detach().cpu().view(-1).numpy().reshape(-1, 3), virial
+
+    def model_calc_per_atom(self, data, device, pbc):
+        """Every result of ``calculate`` from ONE backward pass (``model.energy_forces_virial``), for any ensemble:
+        ``energy`` / ``free_energy``, ``forces``, ``energies [N]`` (``trn_mean`` spread evenly, so they sum to ``energy``),
+        ``stresses [N,6]`` (symmetrised per-atom virials in ``stress``'s units and ordering) and ``stress`` (their sum)."""
+        data = self._prepare(data, device, pbc)
+        out = self.model.energy_forces_virial(data)
+        n = out["energies"].numel()
+        W = out["virials"].detach().cpu().double().numpy()
+        W = 0.5 * (W + W.transpose(0, 2, 1)) * NKTV2P['metal']
+        stresses = self._stress_vector(W.transpose(1, 2, 0)).T
+        energy = (out["energy"] + self.trn_mean).cpu().item()
+        return {'energy': energy, 'free_energy': energy, 'forces': out["forces"].cpu().numpy().reshape(-1, 3),
+                'energies': out["energies"].cpu().double().numpy() + self.trn_mean / max(n, 1),
+                'stresses': stresses, 'stress': stresses.sum(0)}
+
+    def _prepare(self, data, device, pbc):
+        data = data.to(torch.device(device))
+        if pbc and self.verlet.skin > 0.0 and data.get("edge_index") is None:
+            data.graph = self.verlet.get(data.pos, data.atomic_number, data.get("cell"))
+        return data
+
+    def _stress_vector(self, v):
+        """6-vector of a symmetric 3x3 virial ``v[a, b, ...]``."""
+        if self.compat_stress:   # the reference's ordering, kept for bit-compatibility with its consumers
+            return np.array([v[0, 1], v[1, 1], v[2, 2], v[0, 1], v[0, 2], v[1, 2]])
+        return np.array([v[0, 0], v[1, 1], v[2, 2], v[1, 2], v[0, 2], v[0, 1]])

@@ -84,8 +84,9 @@ class VerletGraph:
     (Sub-networks are treated as active when the SUPERSET list has an edge for them -- hermnet.py:56-57 can only differ
     for a sub-network whose every edge sits in the skin shell.)"""
 
-    def __init__(self, model, skin: float = 0.0, cuda_graph: bool = False):
+    def __init__(self, model, skin: float = 0.0, cuda_graph: bool = False, virial: bool = False):
         self.model, self.skin = model, float(skin)
+        self.virial = bool(virial)    # captured evaluation also returns the per-graph virial (energy_forces_virial)
         self.graph, self.ref_pos, self.ref_cell, self.ref_Z = None, None, None, None
         self.builds = self.reuses = 0
         # cuda_graph: while a list is re-used, replay the whole evaluation (forward + backward, ~200 launches + torch glue) as
@@ -95,12 +96,13 @@ class VerletGraph:
 
     def energy_and_gradient(self, pos, Z, cell):
         """``(E [num_graphs], dE/dpos)`` at ``pos`` through the re-used (or rebuilt) list; with ``cuda_graph`` the evaluation is
-        captured once per list build and replayed afterwards (the returned tensors are then the capture's static outputs)."""
+        captured once per list build and replayed afterwards (the returned tensors are then the capture's static outputs;
+        with ``virial`` the capture returns the virial ``[num_graphs,3,3]`` as a third one)."""
         g = self.get(pos, Z, cell)
         if self.cuda_graph and pos.is_cuda:
             if self._captured_for is not g:
                 from ..graphed import graphed_forces
-                self._captured = graphed_forces(self.model, pos, Z, cell, g, warmup=1)
+                self._captured = graphed_forces(self.model, pos, Z, cell, g, warmup=1, virial=self.virial)
                 self._captured_for = g
             return self._captured(pos)
         p = pos.detach().requires_grad_(True)
@@ -125,10 +127,12 @@ class VerletGraph:
 
 
 def velocity_verlet_device(model, numbers, positions, cell, velocities, steps: int, dt_fs: float = 0.5, device="cuda",
-                           skin: float = 0.0, stats: dict = None, cuda_graph: bool = False):
+                           skin: float = 0.0, stats: dict = None, cuda_graph: bool = False, virial: bool = False):
     """Device-resident MD (SURVEY 8(f) rank 1): positions, velocities and forces never leave the GPU; with ``skin > 0`` the
     neighbour list / row CSR / tile plans are re-used across steps (``VerletGraph``), otherwise rebuilt per step (device
-    cell list).  ``stats`` (optional dict) receives the build / re-use counts."""
+    cell list).  ``stats`` (optional dict) receives the build / re-use counts and, with ``virial``, ``stats["virial"]``: the
+    global virial after each step's force evaluation, ``[steps, 3, 3]`` on the device (``model.energy_forces_virial``: the
+    same single backward pass plus one per-atom virial kernel and its sum)."""
     dev = torch.device(device)
     Z = torch.as_tensor(np.asarray(numbers)).long().to(dev)
     pos = torch.as_tensor(np.asarray(positions), dtype=torch.float32).to(dev)
@@ -136,26 +140,33 @@ def velocity_verlet_device(model, numbers, positions, cell, velocities, steps: i
     c = torch.as_tensor(np.asarray(cell), dtype=torch.float32).reshape(1, 3, 3).to(dev)
     masses = np.array([MASSES.get(int(z), 2.0 * int(z)) for z in np.asarray(numbers)])
     inv_m = torch.as_tensor(1.0 / (masses * AMU_A2_FS2_TO_EV), dtype=torch.float32).to(dev)[:, None]
-    vg = VerletGraph(model, skin, cuda_graph)
+    vg = VerletGraph(model, skin, cuda_graph, virial)
 
     def forces(p):
         if vg.cuda_graph:
-            e, g = vg.energy_and_gradient(p, Z, c)
-            return e.clone(), -g                 # (static outputs of the capture: copy what outlives the next call)
+            out = vg.energy_and_gradient(p, Z, c)
+            # (static outputs of the capture: copy what outlives the next call)
+            return (out[0].clone(), -out[1]) + ((out[2].clone(),) if virial else ())
         d = Data(pos=p.detach().requires_grad_(True), atomic_number=Z, cell=c)
         d.graph = vg.get(d.pos, Z, c)
+        if virial:
+            out = model.energy_forces_virial(d)
+            return out["energy"], out["forces"], out["virial"]
         e = model(d)
         (g,) = torch.autograd.grad(e.sum(), d.pos)
         return e.detach(), -g
 
-    e, f = forces(pos)
-    energies = []
+    e, f = forces(pos)[:2]
+    energies, virials = [], []
     for _ in range(steps):
         _kick(vel, f, inv_m, dt_fs)
         pos = pos + dt_fs * vel
-        e, f = forces(pos)
+        e, f, *w = forces(pos)
         _kick(vel, f, inv_m, dt_fs)
         energies.append(e)
+        virials += w
     if stats is not None:
         stats.update(builds=vg.builds, reuses=vg.reuses)
+        if virial:
+            stats["virial"] = torch.cat(virials) if virials else c.new_zeros((0, 3, 3))
     return pos, vel, torch.cat(energies)

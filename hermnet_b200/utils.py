@@ -38,11 +38,13 @@ def in_subgraph(data, nids: Any):
     return rel
 
 
+NKTV2P = {'metal': 1.6021765e6, 'real': 68568.415, 'electron': 2.94210108e13}
+
+
 def virial_calc(cell, pos, forces, energy, units='metal', pbc=False):
     """utils.py:138-160 (same unit table, same symmetrisation)."""
-    table = {'metal': 1.6021765e6, 'real': 68568.415, 'electron': 2.94210108e13}
-    if units in table:
-        nktv2p = table[units]
+    if units in NKTV2P:
+        nktv2p = NKTV2P[units]
     elif units in ['lj', 'si', 'cgs', 'micro', 'nano']:
         nktv2p = 1.0
     else:

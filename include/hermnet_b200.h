@@ -105,6 +105,17 @@ int hn_edge_geom_bwd(const float *geom, const float *g_geom, int32_t n_parts, co
                      const int32_t *rowptr, int32_t rows_per_atom, const int32_t *t_rowptr, const int32_t *t_eid,
                      float sign, int64_t n_atoms, int64_t n_edges, float *grad_pos /*[N,3]*/,
                      float *cellw /*[N,9] or NULL*/, void *stream);
+/* Per-atom virial from the same gradient (one part, g_geom[E] as above):
+ *   virial[i][a][b] = -1/2 sum_{e in rows(i)} D_e[a]*gD_e[b] - 1/2 sum_{e : col[e] = i} D_e[a]*gD_e[b],
+ *   D_e = d*u (clamped edges too); rows(i) = rowptr[i*R] .. rowptr[(i+1)*R], sources from the transpose
+ *   (t_rowptr, t_eid).  Row = position component, column = force component; not symmetrised.  Summed
+ *   over a graph's atoms: W = sum_i pos_i (x) F_i - cell^T dE/dcell = -sum_e D_e (x) gD_e.  One thread
+ *   per atom, fixed order, no atomics (bitwise reproducible); zero g_geom rows (dead Verlet-skin
+ *   entries) add nothing; n_edges == 0 writes zeros.
+ * ------------------------------------------------------------------------------------------- */
+int hn_edge_virial_atom(const float *geom /*[E,4]*/, const float *g_geom /*[E,4]*/, const int32_t *rowptr,
+                        int32_t rows_per_atom, const int32_t *t_rowptr, const int32_t *t_eid, int64_t n_atoms,
+                        int64_t n_edges, float *virial /*[N][9]*/, void *stream);
 
 /* ---------------------------------------------------------------------------------------------
  * Fused PaiNN edge kernel.  Replaces, per layer and per sub-network, HermNet/rmnet.py:55-73
