@@ -85,6 +85,8 @@ SIGNATURES = {
     "hn_halo_unpack": (c_int32, [P, P, c_int64, c_int32, P, P, P]),
     "hn_segment_sum_workspace_bytes": (c_int64, [c_int32, c_int32]),
     "hn_segment_sum": (c_int32, [P, P, P, c_int32, c_int32, P, P, c_int64, P]),
+    "hn_md_langevin_baoa": (c_int32, [P, P, P, P, P, P, c_int32, P, P, P, c_float, c_float, c_float, c_int64, P]),
+    "hn_md_kick": (c_int32, [P, P, P, c_float, c_int64, P, P, P]),
 }
 
 

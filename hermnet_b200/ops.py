@@ -515,6 +515,62 @@ def segment_sum(Y: Tensor, rowptr: Tensor, perm: Optional[Tensor], n_rows: int) 
 
 
 # ----------------------------------------------------------------------------------------------------
+# Langevin MD step (csrc/hn_md.cu)
+# ----------------------------------------------------------------------------------------------------
+def _i64(name, *ts):
+    for t in ts:
+        if t is not None and t.dtype != torch.int64:
+            raise RuntimeError(f"hermnet_b200.{name}: seed / step tensors must be int64 (got {t.dtype})")
+
+
+def _md_shapes(name, n: int, vel: Tensor, force: Tensor, inv_mass: Tensor):
+    if tuple(vel.shape) != (n, 3) or tuple(force.shape) != (n, 3) or inv_mass.numel() != n:
+        raise RuntimeError(f"hermnet_b200.{name}: expected vel / force [{n},3] and inv_mass [{n}]")
+
+
+def md_langevin_baoa(pos: Tensor, vel: Tensor, force: Tensor, inv_mass: Tensor, replica: Tensor, replica_ptr: Tensor,
+                     kT: Tensor, seed: Tensor, step: Tensor, c1: float, c2: float, dt: float) -> None:
+    """B-A-O-A half of a BAOAB Langevin step, in place on ``pos`` / ``vel [N,3]`` (``hn_md_langevin_baoa``): ``replica int32
+    [N]``, ``replica_ptr int32 [G+1]`` (contiguous replicas), per-replica ``kT float32 [G]`` (eV) and ``seed int64 [G]``,
+    ``step int64 [1]`` (read, not advanced).  ``c1 = exp(-gamma dt)``, ``c2 = sqrt(1 - c1^2)``."""
+    lib = _lib.load()
+    dev = _chk("md_langevin_baoa", pos, vel, force, inv_mass, replica, replica_ptr, kT, seed, step)
+    _f32("md_langevin_baoa", pos, vel, force, inv_mass, kT)
+    _i32("md_langevin_baoa", replica, replica_ptr)
+    _i64("md_langevin_baoa", seed, step)
+    n, G = pos.size(0), replica_ptr.numel() - 1
+    _md_shapes("md_langevin_baoa", n, vel, force, inv_mass)
+    if tuple(pos.shape) != (n, 3) or replica.numel() != n or kT.numel() != G or seed.numel() != G or step.numel() != 1:
+        raise RuntimeError(f"hermnet_b200.md_langevin_baoa: expected pos [N,3], replica [N], kT / seed [G={G}], step [1]")
+    with torch.cuda.device(dev), _timed("md_langevin_baoa", dev):
+        _lib.check(lib.hn_md_langevin_baoa(_ptr(pos), _ptr(vel), _ptr(force), _ptr(inv_mass), _ptr(replica), _ptr(replica_ptr), G,
+                                           _ptr(kT), _ptr(seed), _ptr(step), float(c1), float(c2), float(dt), n, _stream(dev)),
+                   "hn_md_langevin_baoa")
+    # written through raw pointers: version-keyed caches (graphs, signed geometry, tile windows) must see the change
+    torch.autograd.graph.increment_version(pos)
+    torch.autograd.graph.increment_version(vel)
+
+
+def md_kick(vel: Tensor, force: Tensor, inv_mass: Tensor, half_dt: float, kinetic: Optional[Tensor], step: Tensor) -> None:
+    """Closing B of a BAOAB step, in place on ``vel [N,3]`` (``hn_md_kick``); ``kinetic [N]`` (optional) receives
+    ``1/2 |v_i|^2 / inv_m_i`` in eV; ``step int64 [1]`` is advanced by one."""
+    lib = _lib.load()
+    dev = _chk("md_kick", vel, force, inv_mass, kinetic, step)
+    _f32("md_kick", vel, force, inv_mass, kinetic)
+    _i64("md_kick", step)
+    n = vel.size(0)
+    _md_shapes("md_kick", n, vel, force, inv_mass)
+    if (kinetic is not None and kinetic.numel() != n) or step.numel() != 1:
+        raise RuntimeError(f"hermnet_b200.md_kick: expected kinetic [{n}] and step [1]")
+    with torch.cuda.device(dev), _timed("md_kick", dev):
+        _lib.check(lib.hn_md_kick(_ptr(vel), _ptr(force), _ptr(inv_mass), float(half_dt), n, _ptr(kinetic), _ptr(step), _stream(dev)),
+                   "hn_md_kick")
+    for t in (vel, kinetic, step):
+        if t is not None:
+            torch.autograd.graph.increment_version(t)
+
+
+# ----------------------------------------------------------------------------------------------------
 # tensor-core dense layer (3xTF32 split on tcgen05)
 # ----------------------------------------------------------------------------------------------------
 def split_tf32(w: Tensor) -> Tuple[Tensor, Tensor]:

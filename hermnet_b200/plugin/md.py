@@ -5,9 +5,12 @@ would drive it (``atoms.get_forces()`` -> ``calc.calculate(atoms)``).  ``device_
 positions stay on the GPU and only the graph is rebuilt per step."""
 from __future__ import annotations
 
+import math
+
 import numpy as np
 import torch
 
+from .. import ops
 from ..data import Data
 from ..symbols import atomic_numbers, chemical_symbols
 
@@ -84,8 +87,9 @@ class VerletGraph:
     (Sub-networks are treated as active when the SUPERSET list has an edge for them -- hermnet.py:56-57 can only differ
     for a sub-network whose every edge sits in the skin shell.)"""
 
-    def __init__(self, model, skin: float = 0.0, cuda_graph: bool = False, virial: bool = False):
+    def __init__(self, model, skin: float = 0.0, cuda_graph: bool = False, virial: bool = False, batch=None):
         self.model, self.skin = model, float(skin)
+        self.batch = batch            # [N] replica of each atom (contiguous), passed to build_graph; None: one system
         self.virial = bool(virial)    # captured evaluation also returns the per-graph virial (energy_forces_virial)
         self.graph, self.ref_pos, self.ref_cell, self.ref_Z = None, None, None, None
         self.builds = self.reuses = 0
@@ -118,12 +122,36 @@ class VerletGraph:
             if moved < 0.5 * self.skin:
                 self.reuses += 1
                 return self.graph
-        self.graph = self.model.build_graph(p, Z, cell, None, skin=self.skin) if self.skin > 0.0 else \
-            self.model.build_graph(p, Z, cell, None)
+        self.graph = self.model.build_graph(p, Z, cell, self.batch, skin=self.skin) if self.skin > 0.0 else \
+            self.model.build_graph(p, Z, cell, self.batch)
         self.ref_pos, self.ref_Z = p.clone(), Z
         self.ref_cell = None if cell is None else cell.detach().clone()
         self.builds += 1
         return self.graph
+
+
+def _evaluator(model, vg: VerletGraph, Z, c, virial: bool):
+    """``forces(p) -> (energy [G], forces [N,3][, virial [G,3,3]])`` at positions ``p`` through ``vg``: the captured
+    replay with ``vg.cuda_graph``, else one eager forward + backward (``model.energy_forces_virial`` with ``virial``)."""
+    def forces(p):
+        if vg.cuda_graph:
+            out = vg.energy_and_gradient(p, Z, c)
+            # (static outputs of the capture: copy what outlives the next call)
+            return (out[0].clone(), -out[1]) + ((out[2].clone(),) if virial else ())
+        d = Data(pos=p.detach().requires_grad_(True), atomic_number=Z, cell=c)
+        d.graph = vg.get(d.pos, Z, c)
+        if virial:
+            out = model.energy_forces_virial(d)
+            return out["energy"], out["forces"], out["virial"]
+        e = model(d)
+        (g,) = torch.autograd.grad(e.sum(), d.pos)
+        return e.detach(), -g
+    return forces
+
+
+def _inv_mass(numbers, dev):
+    masses = np.array([MASSES.get(int(z), 2.0 * int(z)) for z in np.asarray(numbers)])
+    return torch.as_tensor(1.0 / (masses * AMU_A2_FS2_TO_EV), dtype=torch.float32).to(dev)
 
 
 def velocity_verlet_device(model, numbers, positions, cell, velocities, steps: int, dt_fs: float = 0.5, device="cuda",
@@ -138,23 +166,9 @@ def velocity_verlet_device(model, numbers, positions, cell, velocities, steps: i
     pos = torch.as_tensor(np.asarray(positions), dtype=torch.float32).to(dev)
     vel = torch.as_tensor(np.asarray(velocities), dtype=torch.float32).to(dev).clone()      # (never the caller's buffer)
     c = torch.as_tensor(np.asarray(cell), dtype=torch.float32).reshape(1, 3, 3).to(dev)
-    masses = np.array([MASSES.get(int(z), 2.0 * int(z)) for z in np.asarray(numbers)])
-    inv_m = torch.as_tensor(1.0 / (masses * AMU_A2_FS2_TO_EV), dtype=torch.float32).to(dev)[:, None]
+    inv_m = _inv_mass(numbers, dev)[:, None]
     vg = VerletGraph(model, skin, cuda_graph, virial)
-
-    def forces(p):
-        if vg.cuda_graph:
-            out = vg.energy_and_gradient(p, Z, c)
-            # (static outputs of the capture: copy what outlives the next call)
-            return (out[0].clone(), -out[1]) + ((out[2].clone(),) if virial else ())
-        d = Data(pos=p.detach().requires_grad_(True), atomic_number=Z, cell=c)
-        d.graph = vg.get(d.pos, Z, c)
-        if virial:
-            out = model.energy_forces_virial(d)
-            return out["energy"], out["forces"], out["virial"]
-        e = model(d)
-        (g,) = torch.autograd.grad(e.sum(), d.pos)
-        return e.detach(), -g
+    forces = _evaluator(model, vg, Z, c, virial)
 
     e, f = forces(pos)[:2]
     energies, virials = [], []
@@ -170,3 +184,103 @@ def velocity_verlet_device(model, numbers, positions, cell, velocities, steps: i
         if virial:
             stats["virial"] = torch.cat(virials) if virials else c.new_zeros((0, 3, 3))
     return pos, vel, torch.cat(energies)
+
+
+def _replicas(batch, n: int):
+    """``(G, replica_ptr int64 [G+1])`` of a PyG-style batch vector: non-decreasing, every replica 0..G-1 non-empty."""
+    if batch is None:
+        return 1, np.array([0, n], dtype=np.int64)
+    b = (batch.detach().cpu().numpy() if isinstance(batch, torch.Tensor) else np.asarray(batch)).astype(np.int64).reshape(-1)
+    if b.size != n or n == 0:
+        raise ValueError(f"langevin_device: batch must have one entry per atom ({n}), got {b.size}")
+    step = np.diff(b)
+    if b[0] != 0 or (step < 0).any() or (step > 1).any():
+        raise ValueError("langevin_device: batch must be sorted with replicas 0..G-1 all non-empty (a PyG batch vector)")
+    G = int(b[-1]) + 1
+    return G, np.concatenate([[0], np.cumsum(np.bincount(b, minlength=G))]).astype(np.int64)
+
+
+def _per_replica(value, G: int, what: str) -> np.ndarray:
+    v = value.detach().cpu().numpy() if isinstance(value, torch.Tensor) else np.asarray(value)
+    v = np.full(G, v) if v.ndim == 0 else v.reshape(-1)
+    if v.size != G:
+        raise ValueError(f"langevin_device: {what} has {v.size} values for {G} replicas")
+    return v
+
+
+def langevin_device(model, numbers, positions, cell, velocities, steps: int, dt_fs: float = 0.5, temperature_K=300.0,
+                    friction_per_fs: float = 0.01, seed=0, batch=None, step0: int = 0, device="cuda", skin: float = 0.0,
+                    stats: dict = None, cuda_graph: bool = False, virial: bool = False):
+    """Device-resident Langevin (NVT) MD: BAOAB (Leimkuhler-Matthews) with friction ``gamma = friction_per_fs`` (1/fs) over
+    ``G`` independent replicas integrated together, each at its own temperature.  Returns ``(pos [N,3], vel [N,3],
+    energies [steps, G])``; positions, velocities and forces never leave the GPU.
+
+    ``batch``: ``None`` (one replica) or ``[N]`` replica of each atom, non-decreasing with every replica ``0..G-1``
+    non-empty (a PyG batch vector).  ``cell``: ``[3,3]`` (shared) or ``[G,3,3]``.  ``temperature_K``: a float or ``G``
+    values.  ``seed``: an int (replica ``g`` gets ``seed + g``) or ``G`` ints in ``[0, 2^63)``.  ``step0``: the first value
+    of the noise counter -- a run continued from returned ``pos`` / ``vel`` with ``step0 = stats["step"]`` reproduces the
+    uninterrupted trajectory bitwise (same skin / evaluation mode).
+
+    Noise is Philox4x32-10 keyed on (replica seed, replica-local atom index, step) (``hn_md_langevin_baoa``): trajectories
+    are bitwise reproducible, identical eager and with ``cuda_graph``, and a replica's noise does not depend on the batch it
+    is run in.  The step is two fused kernels (``ops.md_langevin_baoa`` before the force evaluation, ``ops.md_kick`` after
+    it) around the same evaluation as ``velocity_verlet_device``: ``skin`` list re-use, ``cuda_graph`` replay of the
+    evaluation (the two integrator kernels stay eager around it) and ``virial``.  The counter and the temperatures live in
+    device memory, so the loop adds no host synchronisation beyond the skin check.
+
+    ``stats`` (optional dict) receives ``builds`` / ``reuses``, ``temperature [steps, G]`` (``2 KE_g / (3 n_g k_B)`` after
+    each step, no centre-of-mass correction: Langevin dynamics does not conserve momentum), ``virial [steps, G, 3, 3]``
+    with ``virial=True`` and ``step``, the final counter value."""
+    if not dt_fs > 0.0:
+        raise ValueError(f"langevin_device: dt_fs must be > 0 (got {dt_fs})")
+    if not friction_per_fs >= 0.0:
+        raise ValueError(f"langevin_device: friction_per_fs must be >= 0 (got {friction_per_fs})")
+    numbers = numbers.cpu().numpy() if isinstance(numbers, torch.Tensor) else np.asarray(numbers)
+    n = len(numbers)
+    G, rptr = _replicas(batch, n)
+    T = _per_replica(temperature_K, G, "temperature_K").astype(np.float64)
+    if not (T >= 0.0).all():
+        raise ValueError("langevin_device: temperatures must be >= 0")
+    seeds = [int(seed) + g for g in range(G)] if np.ndim(seed) == 0 else [int(s) for s in _per_replica(seed, G, "seed")]
+    if not all(0 <= s < 2 ** 63 for s in seeds):
+        raise ValueError("langevin_device: seeds must be in [0, 2^63)")
+    if not 0 <= int(step0) < 2 ** 63:
+        raise ValueError("langevin_device: step0 must be in [0, 2^63)")
+    c_np = (cell.cpu().numpy() if isinstance(cell, torch.Tensor) else np.asarray(cell)).astype(np.float32).reshape(-1, 3, 3)
+    if c_np.shape[0] not in (1, G):
+        raise ValueError(f"langevin_device: cell must be [3,3] or [{G},3,3]")
+
+    dev = torch.device(device)
+    Z = torch.as_tensor(numbers).long().to(dev)
+    # (never the caller's buffers; device tensors are accepted, e.g. the pos / vel of a previous call to continue from)
+    pos = torch.as_tensor(positions, dtype=torch.float32, device=dev).clone()
+    vel = torch.as_tensor(velocities, dtype=torch.float32, device=dev).clone()
+    c = torch.from_numpy(np.repeat(c_np, G // c_np.shape[0], axis=0)).to(dev)
+    inv_m = _inv_mass(numbers, dev)
+    replica_ptr = torch.from_numpy(rptr).to(dev, torch.int32)
+    replica = torch.repeat_interleave(torch.arange(G, dtype=torch.int32), torch.from_numpy(np.diff(rptr))).to(dev)
+    kT = torch.from_numpy(KB_EV * T).to(dev, torch.float32)
+    seed_t = torch.tensor(seeds, dtype=torch.int64, device=dev)
+    step = torch.tensor([int(step0)], dtype=torch.int64, device=dev)
+    kinetic = torch.empty(n, dtype=torch.float32, device=dev)
+    t_scale = torch.from_numpy(2.0 / (3.0 * np.diff(rptr) * KB_EV)).to(dev, torch.float32)
+    gdt = float(friction_per_fs) * float(dt_fs)
+    c1, c2 = math.exp(-gdt), math.sqrt(-math.expm1(-2.0 * gdt))
+
+    vg = VerletGraph(model, skin, cuda_graph, virial, batch=None if batch is None else replica.long())
+    forces = _evaluator(model, vg, Z, c, virial)
+    e, f = forces(pos)[:2]
+    energies, temps, virials = [], [], []
+    for _ in range(steps):
+        ops.md_langevin_baoa(pos, vel, f, inv_m, replica, replica_ptr, kT, seed_t, step, c1, c2, dt_fs)
+        e, f, *w = forces(pos)
+        ops.md_kick(vel, f, inv_m, 0.5 * dt_fs, kinetic, step)
+        energies.append(e)
+        temps.append(ops.segment_sum(kinetic[:, None], replica_ptr, None, G)[:, 0] * t_scale)
+        virials += w
+    if stats is not None:
+        stats.update(builds=vg.builds, reuses=vg.reuses, step=int(step.item()),
+                     temperature=torch.stack(temps) if temps else kT.new_zeros((0, G)))
+        if virial:
+            stats["virial"] = torch.stack(virials) if virials else kT.new_zeros((0, G, 3, 3))
+    return pos, vel, torch.stack(energies) if energies else kT.new_zeros((0, G))

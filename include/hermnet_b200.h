@@ -377,6 +377,38 @@ int hn_node_mid_bwd(int64_t n, int32_t F, const float *g_vdot, const float *g_ca
 int hn_node_pre_bwd(int64_t n, int32_t F, const float *g_xn, const float *g_cat, const float *g_vecn,
                     const float *g_vecp, float *g_x, float *g_vec, void *stream);
 
+/* ---------------------------------------------------------------------------------------------
+ * Langevin (NVT) step of the device MD loop: BAOAB (Leimkuhler-Matthews), units A, fs, eV.  With
+ * c1 = exp(-gamma dt), c2 = sqrt(1 - c1^2) (computed by the caller in float64), inv_m = 1/(mass * 103.642697):
+ *   hn_md_langevin_baoa   B  v += dt/2 F(x_n) inv_m;  A  x += dt/2 v;
+ *                         O  v = c1 v + c2 sqrt(kT[g] inv_m) xi;  A  x += dt/2 v      (pos, vel in place)
+ *   -- the caller evaluates F(x_{n+1}) --
+ *   hn_md_kick            B  v += half_dt F(x_{n+1}) inv_m;  kinetic[i] = 1/2 |v_i|^2 / inv_m_i (eV; kinetic may be
+ *                         NULL);  one thread advances *step by 1.
+ * One thread per atom, caller's atom order.  Replica g owns the contiguous atoms replica_ptr[g] .. replica_ptr[g+1]
+ * (replica[N] int32 names each atom's replica, replica_ptr[G+1] int32); kT[G] (eV) and seed[G] (int64, bits read as
+ * uint64) are per-replica device arrays; step is a device int64 that baoa reads and only kick writes.  Keeping step and
+ * kT in device memory lets a captured CUDA graph replay without any host argument changing: every replay draws fresh
+ * noise, and a temperature ramp is a copy into kT.
+ *
+ * Noise (normative): for atom i of replica g, j = i - replica_ptr[g] (replica-local index),
+ *   r = Philox4x32-10(counter = (j, lo32(step), hi32(step), 0), key = (lo32(seed[g]), hi32(seed[g])))
+ *       (curand_Philox4x32_10 of <curand_philox4x32_x.h>),
+ *   u_k = float((r_k >> 9) * 2 + 1) * 2^-24        (k = 0..3: exact in fp32, in [2^-24, 1 - 2^-24]),
+ *   xi_x = sqrt(-2 ln u0) cos(2 pi u1),  xi_y = sqrt(-2 ln u0) sin(2 pi u1),  xi_z = sqrt(-2 ln u2) cos(2 pi u3)
+ *       (fp32 logf / sincospif; |xi| <= 5.77).
+ * The noise of a replica is a function of its seed, the local index and the step alone: independent of the batch it sits
+ * in and of the launch configuration, so a trajectory is bitwise reproducible and restartable from any step.
+ * Checks: 0 <= n_atoms < 2^31, n_replicas >= 1, dt > 0, 0 <= c1 <= 1, non-null pointers when n_atoms > 0
+ * (n_atoms == 0: no-op, step is not advanced).
+ * ------------------------------------------------------------------------------------------- */
+int hn_md_langevin_baoa(float *pos /*[N,3]*/, float *vel /*[N,3]*/, const float *force /*[N,3]*/, const float *inv_mass /*[N]*/,
+                        const int32_t *replica /*[N]*/, const int32_t *replica_ptr /*[G+1]*/, int32_t n_replicas,
+                        const float *kT /*[G]*/, const int64_t *seed /*[G]*/, const int64_t *step /*[1]*/, float c1, float c2,
+                        float dt, int64_t n_atoms, void *stream);
+int hn_md_kick(float *vel /*[N,3]*/, const float *force /*[N,3]*/, const float *inv_mass /*[N]*/, float half_dt, int64_t n_atoms,
+               float *kinetic /*[N] or NULL*/, int64_t *step /*[1]*/, void *stream);
+
 #ifdef __cplusplus
 }
 #endif
