@@ -87,6 +87,8 @@ SIGNATURES = {
     "hn_segment_sum": (c_int32, [P, P, P, c_int32, c_int32, P, P, c_int64, P]),
     "hn_md_langevin_baoa": (c_int32, [P, P, P, P, P, P, c_int32, P, P, P, c_float, c_float, c_float, c_int64, P]),
     "hn_md_kick": (c_int32, [P, P, P, c_float, c_int64, P, P, P]),
+    "hn_md_scr_barostat": (c_int32, [P, P, P, P, P, P, P, P, c_int32, c_float, c_float, P, P, P]),
+    "hn_md_affine_scale": (c_int32, [P, P, P, P, c_int64, P]),
 }
 
 

@@ -515,7 +515,7 @@ def segment_sum(Y: Tensor, rowptr: Tensor, perm: Optional[Tensor], n_rows: int) 
 
 
 # ----------------------------------------------------------------------------------------------------
-# Langevin MD step (csrc/hn_md.cu)
+# Langevin and constant-pressure MD steps (csrc/hn_md.cu)
 # ----------------------------------------------------------------------------------------------------
 def _i64(name, *ts):
     for t in ts:
@@ -568,6 +568,44 @@ def md_kick(vel: Tensor, force: Tensor, inv_mass: Tensor, half_dt: float, kineti
     for t in (vel, kinetic, step):
         if t is not None:
             torch.autograd.graph.increment_version(t)
+
+
+def md_scr_barostat(cell: Tensor, kinetic: Tensor, virial: Tensor, P0: Tensor, kT: Tensor, beta: Tensor, seed: Tensor,
+                    step: Tensor, dt: float, tau_p: float, mu: Tensor, pressure: Tensor) -> None:
+    """Stochastic cell rescaling of ``G`` replicas (``hn_md_scr_barostat``): ``cell [G,3,3]`` is scaled in place by
+    ``mu [G]`` (written), from the per-replica kinetic energy ``kinetic [G]`` (eV), ``virial [G,3,3]`` (eV), target
+    pressure ``P0 [G]`` (eV/A^3), ``kT [G]`` (eV), compressibility ``beta [G]`` (A^3/eV, >= 0), ``seed int64 [G]`` and
+    ``step int64 [1]`` (read).  ``pressure [G]`` receives the internal pressure (eV/A^3) of the unscaled cell."""
+    lib = _lib.load()
+    dev = _chk("md_scr_barostat", cell, kinetic, virial, P0, kT, beta, seed, step, mu, pressure)
+    _f32("md_scr_barostat", cell, kinetic, virial, P0, kT, beta, mu, pressure)
+    _i64("md_scr_barostat", seed, step)
+    G = kinetic.numel()
+    if (tuple(cell.shape) != (G, 3, 3) or tuple(virial.shape) != (G, 3, 3) or step.numel() != 1
+            or any(t.numel() != G for t in (P0, kT, beta, seed, mu, pressure))):
+        raise RuntimeError(f"hermnet_b200.md_scr_barostat: expected cell / virial [G={G},3,3], kinetic / P0 / kT / beta / seed / "
+                           "mu / pressure [G] and step [1]")
+    with torch.cuda.device(dev), _timed("md_scr_barostat", dev):
+        _lib.check(lib.hn_md_scr_barostat(_ptr(cell), _ptr(kinetic), _ptr(virial), _ptr(P0), _ptr(kT), _ptr(beta), _ptr(seed),
+                                          _ptr(step), G, float(dt), float(tau_p), _ptr(mu), _ptr(pressure), _stream(dev)),
+                   "hn_md_scr_barostat")
+    for t in (cell, mu, pressure):
+        torch.autograd.graph.increment_version(t)
+
+
+def md_affine_scale(pos: Tensor, vel: Tensor, replica: Tensor, mu: Tensor) -> None:
+    """``pos *= mu[replica]``, ``vel /= mu[replica]`` in place on ``[N,3]`` (``hn_md_affine_scale``; ``replica int32 [N]``)."""
+    lib = _lib.load()
+    dev = _chk("md_affine_scale", pos, vel, replica, mu)
+    _f32("md_affine_scale", pos, vel, mu)
+    _i32("md_affine_scale", replica)
+    n = pos.size(0)
+    if tuple(pos.shape) != (n, 3) or tuple(vel.shape) != (n, 3) or replica.numel() != n:
+        raise RuntimeError(f"hermnet_b200.md_affine_scale: expected pos / vel [{n},3] and replica [{n}]")
+    with torch.cuda.device(dev), _timed("md_affine_scale", dev):
+        _lib.check(lib.hn_md_affine_scale(_ptr(pos), _ptr(vel), _ptr(replica), _ptr(mu), n, _stream(dev)), "hn_md_affine_scale")
+    torch.autograd.graph.increment_version(pos)
+    torch.autograd.graph.increment_version(vel)
 
 
 # ----------------------------------------------------------------------------------------------------

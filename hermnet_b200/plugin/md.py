@@ -6,6 +6,7 @@ positions stay on the GPU and only the graph is rebuilt per step."""
 from __future__ import annotations
 
 import math
+from types import SimpleNamespace
 
 import numpy as np
 import torch
@@ -87,9 +88,13 @@ class VerletGraph:
     (Sub-networks are treated as active when the SUPERSET list has an edge for them -- hermnet.py:56-57 can only differ
     for a sub-network whose every edge sits in the skin shell.)"""
 
-    def __init__(self, model, skin: float = 0.0, cuda_graph: bool = False, virial: bool = False, batch=None):
+    def __init__(self, model, skin: float = 0.0, cuda_graph: bool = False, virial: bool = False, batch=None,
+                 deforming: bool = False):
         self.model, self.skin = model, float(skin)
         self.batch = batch            # [N] replica of each atom (contiguous), passed to build_graph; None: one system
+        # deforming: the cell may change between calls (constant-pressure MD); a list is then re-used under the
+        # affine criterion of ``_fits_deformed`` instead of being rebuilt whenever the cell differs
+        self.deforming = bool(deforming)
         self.virial = bool(virial)    # captured evaluation also returns the per-graph virial (energy_forces_virial)
         self.graph, self.ref_pos, self.ref_cell, self.ref_Z = None, None, None, None
         self.builds = self.reuses = 0
@@ -117,9 +122,13 @@ class VerletGraph:
     def get(self, pos, Z, cell):
         p = pos.detach()
         if (self.graph is not None and self.skin > 0.0 and p.shape == self.ref_pos.shape and (Z is self.ref_Z or torch.equal(Z, self.ref_Z))
-                and ((cell is None) == (self.ref_cell is None)) and (cell is None or torch.equal(cell.detach(), self.ref_cell))):
-            moved = float((p - self.ref_pos).norm(dim=1).max())          # one scalar read-back per step
-            if moved < 0.5 * self.skin:
+                and ((cell is None) == (self.ref_cell is None))):
+            if cell is None or torch.equal(cell.detach(), self.ref_cell):
+                moved = float((p - self.ref_pos).norm(dim=1).max())          # one scalar read-back per step
+                if moved < 0.5 * self.skin:
+                    self.reuses += 1
+                    return self.graph
+            elif self.deforming and cell.shape == self.ref_cell.shape and self._fits_deformed(p, cell.detach()):
                 self.reuses += 1
                 return self.graph
         self.graph = self.model.build_graph(p, Z, cell, self.batch, skin=self.skin) if self.skin > 0.0 else \
@@ -128,6 +137,42 @@ class VerletGraph:
         self.ref_cell = None if cell is None else cell.detach().clone()
         self.builds += 1
         return self.graph
+
+    def _fits_deformed(self, p, cell) -> bool:
+        """Whether the list built at ``(ref_pos, ref_cell)`` still holds every pair closer than ``rc`` at ``(p, cell)``.
+        Per replica ``M = ref_cell^-1 cell`` (row vectors) and ``u_i = p_i - ref_pos_i M``; for fixed integer shifts every
+        edge vector is then exactly ``D = D_ref M + u_src - u_dst``, so a pair left out of the list (``|D_ref| >= rc +
+        skin``) has ``|D| >= (rc + skin) sigma_min(M) - 2 max|u|``, and the list is complete while that bound exceeds
+        ``rc`` in every replica.  float64; one scalar read-back."""
+        c0, c1 = self.ref_cell.reshape(-1, 3, 3).double(), cell.reshape(-1, 3, 3).double()
+        inv0 = torch.stack([torch.linalg.cross(c0[:, 1], c0[:, 2]), torch.linalg.cross(c0[:, 2], c0[:, 0]),
+                            torch.linalg.cross(c0[:, 0], c0[:, 1])], -1) / _det3(c0)[:, None, None]
+        M = (inv0[:, :, :, None] * c1[:, None, :, :]).sum(2)
+        s_min = _sigma_min3(M)
+        rep = self.batch if self.batch is not None else torch.zeros(p.size(0), dtype=torch.long, device=p.device)
+        u = p.double() - (self.ref_pos.double()[:, :, None] * M[rep]).sum(1)
+        u_max = torch.zeros(M.size(0), dtype=torch.float64, device=p.device).scatter_reduce(
+            0, rep, u.norm(dim=1), "amax", include_self=True)
+        rc = self.graph.list_rc - self.skin
+        return float(((rc + self.skin) * s_min - 2.0 * u_max - rc).min()) > 0.0
+
+
+def _sigma_min3(M):
+    """Smallest singular value of ``[..., 3, 3]``: square root of the smallest eigenvalue of ``M^T M`` in closed form
+    (trigonometric solution of the symmetric 3x3 eigenproblem; exact for ``M ~ I`` too, where it reduces to ``tr / 3``)."""
+    A = (M[..., :, :, None] * M[..., :, None, :]).sum(-3)
+    q = A.diagonal(dim1=-2, dim2=-1).sum(-1) / 3.0
+    B = A - q[..., None, None] * torch.eye(3, dtype=A.dtype, device=A.device)
+    sd = torch.sqrt((B * B).sum((-2, -1)) / 6.0)
+    r = (_det3(B / torch.where(sd > 0, sd, 1.0)[..., None, None]) / 2.0).clamp(-1.0, 1.0)
+    return torch.sqrt((q + 2.0 * sd * torch.cos(torch.acos(r) / 3.0 + 2.0 * math.pi / 3.0)).clamp(min=0.0))
+
+
+def _det3(a):
+    """Determinant of ``[..., 3, 3]`` (element-wise; row or column convention alike)."""
+    return (a[..., 0, 0] * (a[..., 1, 1] * a[..., 2, 2] - a[..., 1, 2] * a[..., 2, 1])
+            - a[..., 0, 1] * (a[..., 1, 0] * a[..., 2, 2] - a[..., 1, 2] * a[..., 2, 0])
+            + a[..., 0, 2] * (a[..., 1, 0] * a[..., 2, 1] - a[..., 1, 1] * a[..., 2, 0]))
 
 
 def _evaluator(model, vg: VerletGraph, Z, c, virial: bool):
@@ -186,26 +231,69 @@ def velocity_verlet_device(model, numbers, positions, cell, velocities, steps: i
     return pos, vel, torch.cat(energies)
 
 
-def _replicas(batch, n: int):
+def _replicas(batch, n: int, name: str = "langevin_device"):
     """``(G, replica_ptr int64 [G+1])`` of a PyG-style batch vector: non-decreasing, every replica 0..G-1 non-empty."""
     if batch is None:
         return 1, np.array([0, n], dtype=np.int64)
     b = (batch.detach().cpu().numpy() if isinstance(batch, torch.Tensor) else np.asarray(batch)).astype(np.int64).reshape(-1)
     if b.size != n or n == 0:
-        raise ValueError(f"langevin_device: batch must have one entry per atom ({n}), got {b.size}")
+        raise ValueError(f"{name}: batch must have one entry per atom ({n}), got {b.size}")
     step = np.diff(b)
     if b[0] != 0 or (step < 0).any() or (step > 1).any():
-        raise ValueError("langevin_device: batch must be sorted with replicas 0..G-1 all non-empty (a PyG batch vector)")
+        raise ValueError(f"{name}: batch must be sorted with replicas 0..G-1 all non-empty (a PyG batch vector)")
     G = int(b[-1]) + 1
     return G, np.concatenate([[0], np.cumsum(np.bincount(b, minlength=G))]).astype(np.int64)
 
 
-def _per_replica(value, G: int, what: str) -> np.ndarray:
+def _per_replica(value, G: int, what: str, name: str = "langevin_device") -> np.ndarray:
     v = value.detach().cpu().numpy() if isinstance(value, torch.Tensor) else np.asarray(value)
     v = np.full(G, v) if v.ndim == 0 else v.reshape(-1)
     if v.size != G:
-        raise ValueError(f"langevin_device: {what} has {v.size} values for {G} replicas")
+        raise ValueError(f"{name}: {what} has {v.size} values for {G} replicas")
     return v
+
+
+def _langevin_state(name, numbers, positions, cell, velocities, dt_fs, temperature_K, friction_per_fs, seed, batch, step0,
+                    device):
+    """Validated inputs and device state shared by ``langevin_device`` and ``langevin_npt_device``."""
+    if not dt_fs > 0.0:
+        raise ValueError(f"{name}: dt_fs must be > 0 (got {dt_fs})")
+    if not friction_per_fs >= 0.0:
+        raise ValueError(f"{name}: friction_per_fs must be >= 0 (got {friction_per_fs})")
+    numbers = numbers.cpu().numpy() if isinstance(numbers, torch.Tensor) else np.asarray(numbers)
+    n = len(numbers)
+    G, rptr = _replicas(batch, n, name)
+    T = _per_replica(temperature_K, G, "temperature_K", name).astype(np.float64)
+    if not (T >= 0.0).all():
+        raise ValueError(f"{name}: temperatures must be >= 0")
+    seeds = [int(seed) + g for g in range(G)] if np.ndim(seed) == 0 else [int(s) for s in _per_replica(seed, G, "seed", name)]
+    if not all(0 <= s < 2 ** 63 for s in seeds):
+        raise ValueError(f"{name}: seeds must be in [0, 2^63)")
+    if not 0 <= int(step0) < 2 ** 63:
+        raise ValueError(f"{name}: step0 must be in [0, 2^63)")
+    c_np = (cell.cpu().numpy() if isinstance(cell, torch.Tensor) else np.asarray(cell)).astype(np.float32).reshape(-1, 3, 3)
+    if c_np.shape[0] not in (1, G):
+        raise ValueError(f"{name}: cell must be [3,3] or [{G},3,3]")
+
+    st = SimpleNamespace(n=n, G=G)
+    dev = torch.device(device)
+    st.Z = torch.as_tensor(numbers).long().to(dev)
+    # (never the caller's buffers; device tensors are accepted, e.g. the pos / vel of a previous call to continue from)
+    st.pos = torch.as_tensor(positions, dtype=torch.float32, device=dev).clone()
+    st.vel = torch.as_tensor(velocities, dtype=torch.float32, device=dev).clone()
+    st.c = torch.from_numpy(np.repeat(c_np, G // c_np.shape[0], axis=0)).to(dev)
+    st.inv_m = _inv_mass(numbers, dev)
+    st.replica_ptr = torch.from_numpy(rptr).to(dev, torch.int32)
+    st.replica = torch.repeat_interleave(torch.arange(G, dtype=torch.int32), torch.from_numpy(np.diff(rptr))).to(dev)
+    st.kT = torch.from_numpy(KB_EV * T).to(dev, torch.float32)
+    st.seed = torch.tensor(seeds, dtype=torch.int64, device=dev)
+    st.step = torch.tensor([int(step0)], dtype=torch.int64, device=dev)
+    st.kinetic = torch.empty(n, dtype=torch.float32, device=dev)
+    st.t_scale = torch.from_numpy(2.0 / (3.0 * np.diff(rptr) * KB_EV)).to(dev, torch.float32)
+    gdt = float(friction_per_fs) * float(dt_fs)
+    st.c1, st.c2 = math.exp(-gdt), math.sqrt(-math.expm1(-2.0 * gdt))
+    st.batch = None if batch is None else st.replica.long()
+    return st
 
 
 def langevin_device(model, numbers, positions, cell, velocities, steps: int, dt_fs: float = 0.5, temperature_K=300.0,
@@ -231,52 +319,19 @@ def langevin_device(model, numbers, positions, cell, velocities, steps: int, dt_
     ``stats`` (optional dict) receives ``builds`` / ``reuses``, ``temperature [steps, G]`` (``2 KE_g / (3 n_g k_B)`` after
     each step, no centre-of-mass correction: Langevin dynamics does not conserve momentum), ``virial [steps, G, 3, 3]``
     with ``virial=True`` and ``step``, the final counter value."""
-    if not dt_fs > 0.0:
-        raise ValueError(f"langevin_device: dt_fs must be > 0 (got {dt_fs})")
-    if not friction_per_fs >= 0.0:
-        raise ValueError(f"langevin_device: friction_per_fs must be >= 0 (got {friction_per_fs})")
-    numbers = numbers.cpu().numpy() if isinstance(numbers, torch.Tensor) else np.asarray(numbers)
-    n = len(numbers)
-    G, rptr = _replicas(batch, n)
-    T = _per_replica(temperature_K, G, "temperature_K").astype(np.float64)
-    if not (T >= 0.0).all():
-        raise ValueError("langevin_device: temperatures must be >= 0")
-    seeds = [int(seed) + g for g in range(G)] if np.ndim(seed) == 0 else [int(s) for s in _per_replica(seed, G, "seed")]
-    if not all(0 <= s < 2 ** 63 for s in seeds):
-        raise ValueError("langevin_device: seeds must be in [0, 2^63)")
-    if not 0 <= int(step0) < 2 ** 63:
-        raise ValueError("langevin_device: step0 must be in [0, 2^63)")
-    c_np = (cell.cpu().numpy() if isinstance(cell, torch.Tensor) else np.asarray(cell)).astype(np.float32).reshape(-1, 3, 3)
-    if c_np.shape[0] not in (1, G):
-        raise ValueError(f"langevin_device: cell must be [3,3] or [{G},3,3]")
-
-    dev = torch.device(device)
-    Z = torch.as_tensor(numbers).long().to(dev)
-    # (never the caller's buffers; device tensors are accepted, e.g. the pos / vel of a previous call to continue from)
-    pos = torch.as_tensor(positions, dtype=torch.float32, device=dev).clone()
-    vel = torch.as_tensor(velocities, dtype=torch.float32, device=dev).clone()
-    c = torch.from_numpy(np.repeat(c_np, G // c_np.shape[0], axis=0)).to(dev)
-    inv_m = _inv_mass(numbers, dev)
-    replica_ptr = torch.from_numpy(rptr).to(dev, torch.int32)
-    replica = torch.repeat_interleave(torch.arange(G, dtype=torch.int32), torch.from_numpy(np.diff(rptr))).to(dev)
-    kT = torch.from_numpy(KB_EV * T).to(dev, torch.float32)
-    seed_t = torch.tensor(seeds, dtype=torch.int64, device=dev)
-    step = torch.tensor([int(step0)], dtype=torch.int64, device=dev)
-    kinetic = torch.empty(n, dtype=torch.float32, device=dev)
-    t_scale = torch.from_numpy(2.0 / (3.0 * np.diff(rptr) * KB_EV)).to(dev, torch.float32)
-    gdt = float(friction_per_fs) * float(dt_fs)
-    c1, c2 = math.exp(-gdt), math.sqrt(-math.expm1(-2.0 * gdt))
-
-    vg = VerletGraph(model, skin, cuda_graph, virial, batch=None if batch is None else replica.long())
-    forces = _evaluator(model, vg, Z, c, virial)
+    st = _langevin_state("langevin_device", numbers, positions, cell, velocities, dt_fs, temperature_K, friction_per_fs, seed,
+                         batch, step0, device)
+    G, pos, vel, inv_m, replica_ptr, kT, step, kinetic = st.G, st.pos, st.vel, st.inv_m, st.replica_ptr, st.kT, st.step, st.kinetic
+    vg = VerletGraph(model, skin, cuda_graph, virial, batch=st.batch)
+    forces = _evaluator(model, vg, st.Z, st.c, virial)
     e, f = forces(pos)[:2]
     energies, temps, virials = [], [], []
     for _ in range(steps):
-        ops.md_langevin_baoa(pos, vel, f, inv_m, replica, replica_ptr, kT, seed_t, step, c1, c2, dt_fs)
+        ops.md_langevin_baoa(pos, vel, f, inv_m, st.replica, replica_ptr, kT, st.seed, step, st.c1, st.c2, dt_fs)
         e, f, *w = forces(pos)
         ops.md_kick(vel, f, inv_m, 0.5 * dt_fs, kinetic, step)
         energies.append(e)
-        temps.append(ops.segment_sum(kinetic[:, None], replica_ptr, None, G)[:, 0] * t_scale)
+        temps.append(ops.segment_sum(kinetic[:, None], replica_ptr, None, G)[:, 0] * st.t_scale)
         virials += w
     if stats is not None:
         stats.update(builds=vg.builds, reuses=vg.reuses, step=int(step.item()),
@@ -284,3 +339,89 @@ def langevin_device(model, numbers, positions, cell, velocities, steps: int, dt_
         if virial:
             stats["virial"] = torch.stack(virials) if virials else kT.new_zeros((0, G, 3, 3))
     return pos, vel, torch.stack(energies) if energies else kT.new_zeros((0, G))
+
+
+EV_A3_TO_BAR = 1.602176634e6       # 1 eV/A^3 in bar
+
+
+def langevin_npt_device(model, numbers, positions, cell, velocities, steps: int, dt_fs: float = 0.5, temperature_K=300.0,
+                        pressure_bar=1.0, compressibility_per_bar=4.5e-5, tau_p_fs: float = 1000.0,
+                        friction_per_fs: float = 0.01, seed=0, batch=None, step0: int = 0, device="cuda", skin: float = 0.0,
+                        stats: dict = None, cuda_graph: bool = False, forces=None):
+    """Device-resident constant-pressure (NPT) MD: the ``langevin_device`` step followed by isotropic stochastic cell
+    rescaling (Bernetti & Bussi 2020) of every replica towards its own pressure.  Returns ``(pos [N,3], vel [N,3],
+    cell [G,3,3], energies [steps, G])``; positions, velocities, cells and forces never leave the GPU.
+
+    ``batch``, ``cell`` (required, non-singular), ``temperature_K``, ``friction_per_fs``, ``seed`` and ``step0`` as in
+    ``langevin_device``.  ``pressure_bar`` (any finite value; negative is tension) and ``compressibility_per_bar`` (the
+    isothermal compressibility ``beta_T >= 0``; 0 keeps the cell fixed and reproduces ``langevin_device`` bitwise) are a
+    float or ``G`` values; ``tau_p_fs > 0`` is the barostat relaxation time.  Each step is BAOAB's B-A-O-A
+    (``ops.md_langevin_baoa``), the evaluation with the virial, the closing B (``ops.md_kick``), then per replica the
+    internal pressure ``(2 K + tr W) / 3V`` and the strain step (``ops.md_scr_barostat``, noise on counter word 3 = 1) and
+    the affine scaling of positions and velocities (``ops.md_affine_scale``).  The next step's first B uses the forces of
+    the unscaled positions (first order in the strain per step, as GROMACS's C-rescale).  Pressures, compressibilities,
+    temperatures, seeds, the step counter and the cells live in device memory: a captured evaluation keeps reading the
+    cell tensor the barostat scales in place.  ``skin`` lists are re-used across cell changes while the affine criterion of
+    ``VerletGraph(deforming=True)`` holds.  Because the first B of a step uses the forces of the previous step's unscaled
+    positions, the state of a run is ``pos`` / ``vel`` / ``cell`` plus those forces: a run continued from the returned
+    ``pos`` / ``vel`` / ``cell`` with ``step0 = stats["step"]`` and ``forces = stats["forces"]`` reproduces the
+    uninterrupted trajectory bitwise (same skin / evaluation mode).  ``forces=None`` evaluates them at ``positions``.
+
+    ``stats`` (optional dict) receives ``builds`` / ``reuses``, ``step``, ``temperature [steps, G]`` (K),
+    ``pressure [steps, G]`` (bar: the internal pressure of the post-kick state, before the cell step), ``volume
+    [steps, G]`` (A^3, after the cell step) and ``virial [steps, G, 3, 3]`` (eV)."""
+    name = "langevin_npt_device"
+    if cell is None:
+        raise ValueError(f"{name}: a periodic cell is required")
+    c_np = (cell.detach().cpu().numpy() if isinstance(cell, torch.Tensor) else np.asarray(cell, dtype=np.float64))
+    c_np = c_np.astype(np.float64).reshape(-1, 3, 3)
+    if not (np.isfinite(c_np).all() and (np.abs(np.linalg.det(c_np)) > 0.0).all()):
+        raise ValueError(f"{name}: the cell must be finite and non-singular")
+    if not tau_p_fs > 0.0:
+        raise ValueError(f"{name}: tau_p_fs must be > 0 (got {tau_p_fs})")
+    st = _langevin_state(name, numbers, positions, cell, velocities, dt_fs, temperature_K, friction_per_fs, seed, batch, step0,
+                         device)
+    G = st.G
+    P0 = _per_replica(pressure_bar, G, "pressure_bar", name).astype(np.float64)
+    if not np.isfinite(P0).all():
+        raise ValueError(f"{name}: pressures must be finite")
+    beta = _per_replica(compressibility_per_bar, G, "compressibility_per_bar", name).astype(np.float64)
+    if not (np.isfinite(beta).all() and (beta >= 0.0).all()):
+        raise ValueError(f"{name}: compressibilities must be finite and >= 0")
+
+    pos, vel, c, inv_m, replica_ptr, kT, step, kinetic = st.pos, st.vel, st.c, st.inv_m, st.replica_ptr, st.kT, st.step, st.kinetic
+    dev = pos.device
+    P0_t = torch.from_numpy(P0 / EV_A3_TO_BAR).to(dev, torch.float32)            # eV/A^3
+    beta_t = torch.from_numpy(beta * EV_A3_TO_BAR).to(dev, torch.float32)        # A^3/eV
+    mu, pressure = torch.ones(G, dtype=torch.float32, device=dev), torch.zeros(G, dtype=torch.float32, device=dev)
+
+    vg = VerletGraph(model, skin, cuda_graph, True, batch=st.batch, deforming=True)
+    evaluate = _evaluator(model, vg, st.Z, c, True)
+    if forces is None:
+        f = evaluate(pos)[1]
+    else:
+        f = torch.as_tensor(forces, dtype=torch.float32, device=dev).clone()
+        if tuple(f.shape) != (st.n, 3):
+            raise ValueError(f"{name}: forces must be [{st.n},3]")
+    energies, temps, virials, pressures, cells = [], [], [], [], []
+    for _ in range(steps):
+        ops.md_langevin_baoa(pos, vel, f, inv_m, st.replica, replica_ptr, kT, st.seed, step, st.c1, st.c2, dt_fs)
+        e, f, w = evaluate(pos)
+        ops.md_kick(vel, f, inv_m, 0.5 * dt_fs, kinetic, step)
+        ke = ops.segment_sum(kinetic[:, None], replica_ptr, None, G)[:, 0]
+        w = w.contiguous()
+        ops.md_scr_barostat(c, ke, w, P0_t, kT, beta_t, st.seed, step, dt_fs, tau_p_fs, mu, pressure)
+        ops.md_affine_scale(pos, vel, st.replica, mu)
+        energies.append(e)
+        temps.append(ke * st.t_scale)
+        virials.append(w)
+        pressures.append(pressure.clone())
+        cells.append(c.clone())
+    if stats is not None:
+        empty = kT.new_zeros((0, G))
+        stats.update(builds=vg.builds, reuses=vg.reuses, step=int(step.item()),
+                     temperature=torch.stack(temps) if temps else empty,
+                     pressure=torch.stack(pressures) * EV_A3_TO_BAR if pressures else empty,
+                     volume=_det3(torch.stack(cells).double()).abs().float() if cells else empty,
+                     virial=torch.stack(virials) if virials else kT.new_zeros((0, G, 3, 3)), forces=f)
+    return pos, vel, c, torch.stack(energies) if energies else kT.new_zeros((0, G))

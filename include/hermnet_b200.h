@@ -409,6 +409,37 @@ int hn_md_langevin_baoa(float *pos /*[N,3]*/, float *vel /*[N,3]*/, const float 
 int hn_md_kick(float *vel /*[N,3]*/, const float *force /*[N,3]*/, const float *inv_mass /*[N]*/, float half_dt, int64_t n_atoms,
                float *kinetic /*[N] or NULL*/, int64_t *step /*[1]*/, void *stream);
 
+/* ---------------------------------------------------------------------------------------------
+ * Constant-pressure cell step of the device MD loop: isotropic stochastic cell rescaling (Bernetti & Bussi,
+ * J. Chem. Phys. 153, 114107 (2020)), run after hn_md_kick and a per-replica sum of its kinetic energies.
+ * Units A, fs, eV; pressures in eV/A^3, beta (isothermal compressibility) in A^3/eV.
+ *   hn_md_scr_barostat    one thread per replica g, float64 inside:
+ *                           V = |det cell_g|,  P = (2 kinetic[g] + tr virial_g) / (3 V)   (virial as from the force
+ *                           pass: W = sum pos (x) F - cell^T dE/dcell, so tr W / 3V = -dU/dV),
+ *                           b = beta[g] dt / tau_p,
+ *                           de = -b (P0[g] - P) + sqrt(2 kT[g] b / V) xi,   mu = float(exp(de / 3)),
+ *                           cell_g = mu * cell_g (fp32, in place),  mu_out[g] = mu,  pressure[g] = float(P).
+ *                         The drift carries no +kT/V term: with the velocity scaling below and noise ~ V^-1/2
+ *                         (Ito), the zero-flux density is rho(V) ~ V^N exp(-(U + K + P0 V)/kT) (DESIGN.md).
+ *   hn_md_affine_scale    one thread per atom i of replica g = replica[i]:  pos_i = mu[g] pos_i,  vel_i = vel_i / mu[g]
+ *                         (fp32, in place; with the cell scaled by the same mu every edge vector scales exactly).
+ * Noise (normative): for replica g at counter value n = *step (read after hn_md_kick advanced it),
+ *   r = Philox4x32-10(counter = (0, lo32(n), hi32(n), 1), key = (lo32(seed[g]), hi32(seed[g]))),
+ *   u_k = float((r_k >> 9) * 2 + 1) * 2^-24 (k = 0, 1; as in hn_md_langevin_baoa),
+ *   xi = sqrt(-2 ln u0) cos(2 pi u1)        (float64 log / cospi of the exact fp32 uniforms).
+ * Counter word 3 = 1 keeps this stream disjoint from the Langevin noise (word 3 = 0) at every step.  P0, kT, beta, seed,
+ * step and cell live in device memory, so a captured replay needs no changing host argument and a pressure ramp is a
+ * copy into P0.  beta[g] >= 0 is the caller's precondition (device data are not read on the host).
+ * Checks: n_replicas >= 0, dt > 0, tau_p > 0 (so dt / tau_p > 0), 0 <= n_atoms < 2^31, non-null pointers when there
+ * is work (n_replicas == 0 / n_atoms == 0: no-op).
+ * ------------------------------------------------------------------------------------------- */
+int hn_md_scr_barostat(float *cell /*[G,3,3]*/, const float *kinetic /*[G]*/, const float *virial /*[G,3,3]*/,
+                       const float *P0 /*[G]*/, const float *kT /*[G]*/, const float *beta /*[G]*/, const int64_t *seed /*[G]*/,
+                       const int64_t *step /*[1]*/, int32_t n_replicas, float dt, float tau_p, float *mu /*[G]*/,
+                       float *pressure /*[G]*/, void *stream);
+int hn_md_affine_scale(float *pos /*[N,3]*/, float *vel /*[N,3]*/, const int32_t *replica /*[N]*/, const float *mu /*[G]*/,
+                       int64_t n_atoms, void *stream);
+
 #ifdef __cplusplus
 }
 #endif
