@@ -609,6 +609,104 @@ def md_affine_scale(pos: Tensor, vel: Tensor, replica: Tensor, mu: Tensor) -> No
 
 
 # ----------------------------------------------------------------------------------------------------
+# FIRE structure relaxation (csrc/hn_opt.cu)
+# ----------------------------------------------------------------------------------------------------
+def _f64(name, *ts):
+    for t in ts:
+        if t is not None and t.dtype != torch.float64:
+            raise RuntimeError(f"hermnet_b200.{name}: optimizer state tensors must be float64 (got {t.dtype})")
+
+
+def _g9(name, G: int, *ts):
+    for t in ts:
+        if t is not None and t.numel() != 9 * G:
+            raise RuntimeError(f"hermnet_b200.{name}: expected [G={G},3,3] (or [G,9]) matrices, got {tuple(t.shape)}")
+
+
+def opt_fire_reduce(force: Tensor, vel: Tensor, A: Optional[Tensor], replica: Tensor, replica_ptr: Tensor) -> Tensor:
+    """Per-replica float64 ``[G,4]``: ``(sum F'.v, sum |F'|^2, sum |v|^2, max |F'_i|^2)`` over the atoms with ``F'_i = f_i A^T``
+    (``hn_opt_fire_reduce``; ``A float64 [G,3,3]`` or ``None`` for ``A = I``).  Deterministic (fixed summation order)."""
+    lib = _lib.load()
+    dev = _chk("opt_fire_reduce", force, vel, A, replica, replica_ptr)
+    _f32("opt_fire_reduce", force, vel)
+    _f64("opt_fire_reduce", A)
+    _i32("opt_fire_reduce", replica, replica_ptr)
+    n, G = force.size(0), replica_ptr.numel() - 1
+    if tuple(force.shape) != (n, 3) or tuple(vel.shape) != (n, 3) or replica.numel() != n:
+        raise RuntimeError(f"hermnet_b200.opt_fire_reduce: expected force / vel [{n},3] and replica [{n}]")
+    _g9("opt_fire_reduce", G, A)
+    sums = (torch.empty if n else torch.zeros)((G, 4), dtype=torch.float64, device=dev)      # (n == 0: the launch is a no-op)
+    with torch.cuda.device(dev), _timed("opt_fire_reduce", dev, kernels=2):
+        ws_bytes = int(lib.hn_opt_fire_reduce_workspace_bytes(n, G))        # per-chunk partials: caller-owned
+        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev) if ws_bytes else None
+        _lib.check(lib.hn_opt_fire_reduce(_ptr(force), _ptr(vel), _ptr(A), _ptr(replica), _ptr(replica_ptr), G, n, _ptr(sums),
+                                          _ptr(ws), ws_bytes, _stream(dev)), "hn_opt_fire_reduce")
+    return sums
+
+
+def opt_fire_step(sums: Tensor, virial: Optional[Tensor], cell: Optional[Tensor], h0: Optional[Tensor], A: Optional[Tensor],
+                  A_prev: Optional[Tensor], vcell: Optional[Tensor], P0: Optional[Tensor], cell_factor: Optional[Tensor],
+                  dt: Tensor, alpha: Tensor, n_pos: Tensor, steps: Tensor, converged: Tensor, fmax: float, dt_max: float,
+                  max_step: float, move: bool, coef: Tensor, fmax_out: Tensor, n_active: Tensor) -> None:
+    """One FIRE step of ``G`` replicas in float64 (``hn_opt_fire_step``): convergence test, mixing, ``dt`` / ``alpha`` /
+    ``n_pos`` logic and the closed-form ``max_step`` cap; with ``A`` the three cell rows from ``virial [G,3,3]`` (fp32), the
+    cell ``[G,3,3]`` (fp32, rewritten in place as ``h0 A``), target pressure ``P0 [G]`` (eV/A^3) and ``cell_factor [G]``.
+    Writes ``coef [G,3]`` (for ``opt_fire_update``), ``fmax_out [G]`` and ``n_active int32 [1]``; ``move=False`` runs the
+    convergence test only.  State: ``dt``, ``alpha`` float64 ``[G]``, ``n_pos``, ``steps``, ``converged`` int32 ``[G]``,
+    ``A``, ``A_prev``, ``vcell``, ``h0`` float64 ``[G,3,3]``."""
+    lib = _lib.load()
+    dev = _chk("opt_fire_step", sums, virial, cell, h0, A, A_prev, vcell, P0, cell_factor, dt, alpha, n_pos, steps, converged, coef,
+               fmax_out, n_active)
+    G = dt.numel()
+    _f64("opt_fire_step", sums, h0, A, A_prev, vcell, P0, cell_factor, dt, alpha, coef, fmax_out)
+    _f32("opt_fire_step", virial, cell)
+    _i32("opt_fire_step", n_pos, steps, converged, n_active)
+    if (sums.numel() != 4 * G or coef.numel() != 3 * G or n_active.numel() != 1
+            or any(t.numel() != G for t in (alpha, n_pos, steps, converged, fmax_out))):
+        raise RuntimeError(f"hermnet_b200.opt_fire_step: expected sums [G={G},4], coef [G,3], dt / alpha / n_pos / steps / "
+                           "converged / fmax_out [G] and n_active [1]")
+    if A is not None:
+        if any(t is None for t in (virial, cell, h0, A_prev, vcell, P0, cell_factor)):
+            raise RuntimeError("hermnet_b200.opt_fire_step: the cell rows need virial, cell, h0, A_prev, vcell, P0 and cell_factor")
+        _g9("opt_fire_step", G, virial, cell, h0, A, A_prev, vcell)
+        if P0.numel() != G or cell_factor.numel() != G:
+            raise RuntimeError(f"hermnet_b200.opt_fire_step: expected P0 / cell_factor [G={G}]")
+    with torch.cuda.device(dev), _timed("opt_fire_step", dev):
+        _lib.check(lib.hn_opt_fire_step(_ptr(sums), _ptr(virial), _ptr(cell), _ptr(h0), _ptr(A), _ptr(A_prev), _ptr(vcell), _ptr(P0),
+                                        _ptr(cell_factor), _ptr(dt), _ptr(alpha), _ptr(n_pos), _ptr(steps), _ptr(converged), G,
+                                        float(fmax), float(dt_max), float(max_step), int(bool(move)), _ptr(coef), _ptr(fmax_out),
+                                        _ptr(n_active), _stream(dev)), "hn_opt_fire_step")
+    for t in (dt, alpha, n_pos, steps, converged, coef, fmax_out, n_active) + ((cell, A, A_prev, vcell) if A is not None else ()):
+        torch.autograd.graph.increment_version(t)
+
+
+def opt_fire_update(x: Optional[Tensor], rp: Tensor, vel: Tensor, force: Tensor, A_prev: Optional[Tensor], A: Optional[Tensor],
+                    replica: Tensor, converged: Tensor, coef: Tensor) -> None:
+    """Atom rows of a FIRE step in place (``hn_opt_fire_update``), for atoms of replicas not converged:
+    ``vel = c_v vel + c_f' f A_prev^T``, ``rp += s dt vel``, ``x = rp A``.  ``A = None``: positions only, ``rp`` is the
+    positions and ``x`` / ``A_prev`` are unused."""
+    lib = _lib.load()
+    dev = _chk("opt_fire_update", x, rp, vel, force, A_prev, A, replica, converged, coef)
+    _f32("opt_fire_update", x, rp, vel, force)
+    _f64("opt_fire_update", A_prev, A, coef)
+    _i32("opt_fire_update", replica, converged)
+    n, G = rp.size(0), converged.numel()
+    if (tuple(rp.shape) != (n, 3) or tuple(vel.shape) != (n, 3) or tuple(force.shape) != (n, 3) or replica.numel() != n
+            or coef.numel() != 3 * G):
+        raise RuntimeError(f"hermnet_b200.opt_fire_update: expected rp / vel / force [{n},3], replica [{n}] and coef [G={G},3]")
+    if A is not None:
+        if x is None or A_prev is None or tuple(x.shape) != (n, 3):
+            raise RuntimeError(f"hermnet_b200.opt_fire_update: A needs x [{n},3] and A_prev")
+        _g9("opt_fire_update", G, A, A_prev)
+    with torch.cuda.device(dev), _timed("opt_fire_update", dev):
+        _lib.check(lib.hn_opt_fire_update(_ptr(x if A is not None else None), _ptr(rp), _ptr(vel), _ptr(force), _ptr(A_prev),
+                                          _ptr(A), _ptr(replica), _ptr(converged), _ptr(coef), n, _stream(dev)),
+                   "hn_opt_fire_update")
+    for t in (rp, vel) + ((x,) if A is not None else ()):
+        torch.autograd.graph.increment_version(t)
+
+
+# ----------------------------------------------------------------------------------------------------
 # tensor-core dense layer (3xTF32 split on tcgen05)
 # ----------------------------------------------------------------------------------------------------
 def split_tf32(w: Tensor) -> Tuple[Tensor, Tensor]:

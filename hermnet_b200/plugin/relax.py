@@ -1,0 +1,114 @@
+"""Device-resident structure relaxation: FIRE over batched replicas, with the unit cell relaxed under a target pressure
+if asked for.  The optimizer is ASE's ``FIRE`` (its rules and defaults) applied per replica, over the generalized
+coordinates of ASE's ``UnitCellFilter`` -- the route ``FIRE(UnitCellFilter(atoms))`` over ``NNCalculator`` takes one
+structure at a time on the host; here every replica of a PyG-style batch relaxes at once and only one integer (the number
+of replicas still moving) comes back to the host per step."""
+from __future__ import annotations
+
+import numpy as np
+import torch
+
+from .. import ops
+from .md import EV_A3_TO_BAR, VerletGraph, _det3, _evaluator, _per_replica, _replicas
+
+
+def fire_relax_device(model, numbers, positions, cell, fmax=0.05, max_steps=1000, batch=None, relax_cell=False,
+                      pressure_bar=0.0, cell_factor=None, dt=0.1, dt_max=1.0, max_step=0.2, skin=0.0, cuda_graph=False,
+                      stats=None, device="cuda"):
+    """Relax ``G`` replicas to ``max_i |F_i| < fmax`` (eV/A) with FIRE, each on its own: own ``dt`` / ``alpha`` / ``n_pos``,
+    own convergence (sticky: a converged replica never moves again and keeps its coordinates bitwise), at most
+    ``max_steps`` steps.  Returns ``(pos [N,3], cell [G,3,3] or None, energy [G])``, the energy at the returned geometry.
+
+    ``batch``: ``None`` (one replica) or ``[N]`` replica of each atom, non-decreasing with every replica ``0..G-1``
+    non-empty.  ``cell``: ``None`` (clusters; not with ``relax_cell``), ``[3,3]`` (shared) or ``[G,3,3]``, rows are the
+    lattice vectors.  ``dt``, ``dt_max`` (>= dt), ``max_step`` (A, the cap on a replica's whole step) are ASE's parameters;
+    masses are ignored as in ASE.
+
+    ``relax_cell``: ASE's ``UnitCellFilter``.  With ``A = h0^-1 h`` (``h0`` the starting cell) the coordinates are the atom
+    rows ``x A^-1`` (forces ``f A^T``) and three cell rows ``c_f A^T`` whose force is ``(W_sym - P0 V I) A^-1 / c_f``:
+    ``W_sym`` the symmetrised virial of the force pass (``model.energy_forces_virial``; it is ASE's ``-V sigma``), ``P0`` the
+    target pressure (``pressure_bar``, a float or ``G`` values), ``V = |det h|`` and ``c_f`` = ``cell_factor`` (a float or
+    ``G`` values; default the replica's atom count, as ASE).  The cell rows count in the norms, in ``F.v`` and in the
+    convergence test like atom rows; the stationary point minimises the enthalpy ``E + P0 V``.
+
+    Each iteration is one evaluation (``skin`` lists re-used across steps and, with the cell relaxed, across cell changes;
+    ``cuda_graph`` replays the evaluation while a list is re-used), then ``ops.opt_fire_reduce`` (per-replica sums over the
+    atoms), ``ops.opt_fire_step`` (per replica in float64: convergence, mixing, ``dt`` / ``alpha``, the ``max_step`` cap in
+    closed form, the cell rows) and ``ops.opt_fire_update`` (the atom rows).
+
+    ``stats`` (optional dict) receives ``converged [G]`` (bool), ``steps [G]`` (steps taken), per-evaluation traces
+    ``energy``, ``fmax`` (the generalized max force) and, with ``relax_cell``, ``volume`` (A^3), all ``[iters, G]``; the
+    optimizer state after each iteration's step, ``dt``, ``alpha`` and ``n_pos [iters, G]``; and ``builds`` / ``reuses``."""
+    name = "fire_relax_device"
+    if not fmax > 0.0:
+        raise ValueError(f"{name}: fmax must be > 0 (got {fmax})")
+    if not dt > 0.0:
+        raise ValueError(f"{name}: dt must be > 0 (got {dt})")
+    if not dt_max >= dt:
+        raise ValueError(f"{name}: dt_max must be >= dt (got {dt_max} < {dt})")
+    if not max_step > 0.0:
+        raise ValueError(f"{name}: max_step must be > 0 (got {max_step})")
+    if not int(max_steps) >= 0:
+        raise ValueError(f"{name}: max_steps must be >= 0 (got {max_steps})")
+    max_steps = int(max_steps)
+    numbers = numbers.cpu().numpy() if isinstance(numbers, torch.Tensor) else np.asarray(numbers)
+    n = len(numbers)
+    G, rptr = _replicas(batch, n, name)
+    c_np = None
+    if cell is not None:
+        c_np = (cell.detach().cpu().numpy() if isinstance(cell, torch.Tensor) else np.asarray(cell)).astype(np.float64).reshape(-1, 3, 3)
+        if c_np.shape[0] not in (1, G):
+            raise ValueError(f"{name}: cell must be [3,3] or [{G},3,3]")
+    if relax_cell and (c_np is None or not np.isfinite(c_np).all() or not (np.abs(np.linalg.det(c_np)) > 0.0).all()):
+        raise ValueError(f"{name}: relax_cell needs a finite, non-singular cell")
+    P0 = _per_replica(pressure_bar, G, "pressure_bar", name).astype(np.float64)
+    if not np.isfinite(P0).all():
+        raise ValueError(f"{name}: pressures must be finite")
+    cf = np.diff(rptr).astype(np.float64) if cell_factor is None else \
+        _per_replica(cell_factor, G, "cell_factor", name).astype(np.float64)
+    if not (np.isfinite(cf).all() and (cf > 0.0).all()):
+        raise ValueError(f"{name}: cell_factor must be finite and > 0")
+
+    dev = torch.device(device)
+    Z = torch.as_tensor(numbers).long().to(dev)
+    # (never the caller's buffers)
+    pos = torch.as_tensor(positions, dtype=torch.float32, device=dev).reshape(n, 3).clone()
+    c = None if c_np is None else torch.from_numpy(np.repeat(c_np.astype(np.float32), G // c_np.shape[0], axis=0)).to(dev)
+    replica_ptr = torch.from_numpy(rptr).to(dev, torch.int32)
+    replica = torch.repeat_interleave(torch.arange(G, dtype=torch.int32), torch.from_numpy(np.diff(rptr))).to(dev)
+    vg = VerletGraph(model, skin, cuda_graph, relax_cell, batch=None if batch is None else replica.long(), deforming=relax_cell)
+    evaluate = _evaluator(model, vg, Z, c, relax_cell)
+
+    f64 = dict(dtype=torch.float64, device=dev)
+    dt_g, alpha = torch.full((G,), float(dt), **f64), torch.full((G,), 0.1, **f64)
+    n_pos, steps, converged = (torch.zeros(G, dtype=torch.int32, device=dev) for _ in range(3))
+    coef, fmax_g = torch.zeros((G, 3), **f64), torch.zeros(G, **f64)
+    n_active = torch.zeros(1, dtype=torch.int32, device=dev)
+    vel = torch.zeros_like(pos)
+    if relax_cell:
+        rp = pos.clone()                                        # r' = x A^-1 with A = I at the start
+        A = torch.eye(3, **f64).repeat(G, 1, 1)
+        A_prev, vcell, h0 = A.clone(), torch.zeros((G, 3, 3), **f64), c.double()
+        P0_t, cf_t = torch.from_numpy(P0 / EV_A3_TO_BAR).to(dev), torch.from_numpy(cf).to(dev)
+    else:
+        rp, A, A_prev, vcell, h0, P0_t, cf_t = pos, None, None, None, None, None, None     # positions only: x is r'
+
+    trace = {k: [] for k in ("energy", "fmax", "volume", "dt", "alpha", "n_pos")}
+    for it in range(max_steps + 1):
+        e, f, *w = evaluate(pos)
+        sums = ops.opt_fire_reduce(f, vel, A, replica, replica_ptr)
+        if relax_cell:
+            trace["volume"].append(_det3(c.double()).abs())      # of the evaluated cell, before the step moves it
+        ops.opt_fire_step(sums, w[0].contiguous() if relax_cell else None, c if relax_cell else None, h0, A, A_prev, vcell, P0_t,
+                          cf_t, dt_g, alpha, n_pos, steps, converged, fmax, dt_max, max_step, it < max_steps, coef, fmax_g,
+                          n_active)
+        trace["energy"].append(e)
+        for k, t in (("fmax", fmax_g), ("dt", dt_g), ("alpha", alpha), ("n_pos", n_pos)):
+            trace[k].append(t.clone())
+        if it == max_steps or int(n_active.item()) == 0:         # one int read-back per step
+            break
+        ops.opt_fire_update(pos if relax_cell else None, rp, vel, f, A_prev, A, replica, converged, coef)
+    if stats is not None:
+        stats.update(builds=vg.builds, reuses=vg.reuses, converged=converged.bool(), steps=steps.clone(),
+                     **{k: torch.stack(v) for k, v in trace.items() if v})
+    return pos, c, e

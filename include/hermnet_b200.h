@@ -440,6 +440,56 @@ int hn_md_scr_barostat(float *cell /*[G,3,3]*/, const float *kinetic /*[G]*/, co
 int hn_md_affine_scale(float *pos /*[N,3]*/, float *vel /*[N,3]*/, const int32_t *replica /*[N]*/, const float *mu /*[G]*/,
                        int64_t n_atoms, void *stream);
 
+/* ---------------------------------------------------------------------------------------------
+ * Structure relaxation: FIRE (Bitzek et al., PRL 97, 170201 (2006)) with ASE's rules, per replica g, over the generalized
+ * coordinates of ASE's UnitCellFilter in row-vector convention (lattice vectors = rows of h).  Masses are ignored.
+ * Replicas are contiguous as in hn_md_langevin_baoa (replica[N], replica_ptr[G+1]).
+ *   Deformation A_g = h0_g^-1 h_g (float64 [G][9], row-major).  Atom rows r'_i = x_i A^-1, generalized force F'_i = f_i A^T.
+ *   With the cell relaxed (A != NULL) three cell rows q_c = c_f A^T with generalized force
+ *     F_c = (W_sym - P0 V I) A^-1 / c_f,   W_sym = (W + W^T)/2,  W = sum pos (x) F - h^T dE/dh  (the per-graph virial of
+ *     the force pass; W - P0 V I is ASE's filter virial),  V = |det h|,  c_f = cell_factor[g].
+ *   A == NULL: positions only; A = I exactly, F' = f and x = r' bitwise (no multiplication).
+ * Fixed constants N_min = 5, f_inc = 1.1, f_dec = 0.5, alpha_start = 0.1, f_alpha = 0.99.  Per iteration, with F the
+ * generalized forces at the current coordinates and every sum over replica g's rows (atom rows and cell rows alike):
+ *   hn_opt_fire_reduce   one warp per chunk of 256 atoms, float64:  sums[g] = (sum F'.v, sum |F'|^2, sum |v|^2,
+ *                        max_i |F'_i|^2) over the atom rows.  The piece (chunk b) x (replica g) is written to workspace slot
+ *                        b + g and the pieces of a replica are summed in order (a warp per replica, or a block when replicas
+ *                        span many chunks): fixed summation order, no atomics, bitwise reproducible for a given (N, G).
+ *   hn_opt_fire_step     one thread per replica, float64.  Adds the cell rows (A != NULL), writes fmax_out[g] = max row |F|,
+ *                        then:  converged[g] set: nothing more.  max row |F|^2 < fmax^2: converged[g] = 1 (sticky; the
+ *                        replica never moves again).  Otherwise the replica counts in *n_active (zeroed by the call) and,
+ *                        with move != 0, takes a FIRE step:
+ *                          steps[g] == 0 (ASE's v is None):  c_v = 0, c_m = 0 (dt, alpha unchanged);
+ *                          P = F.v > 0:  c_v = 1 - alpha, c_m = alpha |v| / |F|;  if n_pos > N_min: dt = min(f_inc dt, dt_max),
+ *                                        alpha *= f_alpha;  n_pos += 1;
+ *                          else:         c_v = 0, c_m = 0, alpha = alpha_start, dt *= f_dec, n_pos = 0;
+ *                          v_new = c_v v + c_f' F with c_f' = c_m + dt, |v_new|^2 = c_v^2 |v|^2 + 2 c_v c_f' F.v + c_f'^2 |F|^2
+ *                          (closed form: no second atom pass), s = min(1, max_step / (dt |v_new|)),
+ *                          coef[g] = (c_v, c_f', s dt), steps[g] += 1;
+ *                        cell rows: vcell = c_v vcell + c_f' F_c, A_prev = A, A = ((c_f A^T + s dt vcell) / c_f)^T,
+ *                        cell = float(h0 A) in place.  move == 0: convergence test only (the last evaluation of a capped run).
+ *   hn_opt_fire_update   one thread per atom of a replica with converged[g] == 0:  v = c_v v + c_f' F'_i (F' at A_prev, the
+ *                        deformation the forces were evaluated at),  r' += s dt v (fp32 storage, float64 arithmetic),
+ *                        x = r' A (the new deformation; A == NULL: r' is the positions and x is not used).
+ * State (device memory, caller-owned): dt, alpha [G] float64, n_pos, steps, converged [G] int32, vcell, A, A_prev [G][9]
+ * float64, h0 [G][9] float64.  Initial values: dt = the user's dt, alpha = 0.1, zeros, A = I, v = 0, r' = x.
+ * Checks: 0 <= n_atoms < 2^31, n_replicas >= 0, fmax, dt_max, max_step > 0, non-null pointers when there is work
+ * (n_atoms == 0 / n_replicas == 0: no-op); the reduce workspace holds hn_opt_fire_reduce_workspace_bytes.
+ * ------------------------------------------------------------------------------------------- */
+int64_t hn_opt_fire_reduce_workspace_bytes(int64_t n_atoms, int32_t n_replicas);
+int hn_opt_fire_reduce(const float *force /*[N,3]*/, const float *vel /*[N,3]*/, const double *A /*[G,9] or NULL*/,
+                       const int32_t *replica /*[N]*/, const int32_t *replica_ptr /*[G+1]*/, int32_t n_replicas, int64_t n_atoms,
+                       double *sums /*[G,4]*/, void *workspace, int64_t workspace_bytes, void *stream);
+int hn_opt_fire_step(const double *sums /*[G,4]*/, const float *virial /*[G,3,3]*/, float *cell /*[G,3,3]*/,
+                     const double *h0 /*[G,9]*/, double *A /*[G,9] or NULL*/, double *A_prev /*[G,9]*/, double *vcell /*[G,9]*/,
+                     const double *P0 /*[G] eV/A^3*/, const double *cell_factor /*[G]*/, double *dt /*[G]*/, double *alpha /*[G]*/,
+                     int32_t *n_pos /*[G]*/, int32_t *steps /*[G]*/, int32_t *converged /*[G]*/, int32_t n_replicas, double fmax,
+                     double dt_max, double max_step, int32_t move, double *coef /*[G,3]*/, double *fmax_out /*[G]*/,
+                     int32_t *n_active /*[1]*/, void *stream);
+int hn_opt_fire_update(float *x /*[N,3]*/, float *rp /*[N,3]*/, float *vel /*[N,3]*/, const float *force /*[N,3]*/,
+                       const double *A_prev /*[G,9]*/, const double *A /*[G,9] or NULL*/, const int32_t *replica /*[N]*/,
+                       const int32_t *converged /*[G]*/, const double *coef /*[G,3]*/, int64_t n_atoms, void *stream);
+
 #ifdef __cplusplus
 }
 #endif
