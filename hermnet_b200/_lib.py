@@ -19,7 +19,21 @@ class EdgeParams(Structure):
                 ("num_rbf", c_int32), ("env_p", c_int32), ("inv_rc", c_float), ("coeff", c_float), ("variant", c_int32), ("flags", c_int32)]
 
 
-P = c_void_p  # every device pointer crosses the ABI as a plain address
+class P(c_void_p):
+    """Argument type of every device pointer: ctypes passes ``None`` (NULL) and ``c_void_p`` through, and the address of
+    anything with ``data_ptr()`` (a tensor) as a full-width pointer."""
+
+    @classmethod
+    def from_param(cls, obj):
+        if obj is None or type(obj) is c_void_p:
+            return obj
+        try:
+            data_ptr = obj.data_ptr
+        except AttributeError:
+            if isinstance(obj, c_void_p):
+                return obj
+            raise TypeError(f"expected a tensor, a c_void_p or None for a device pointer, got {type(obj).__name__}") from None
+        return c_void_p(data_ptr())     # never a bare int: ctypes would pass it as a 32-bit C int
 
 
 class TcPlan(Structure):
