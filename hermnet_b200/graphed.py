@@ -39,23 +39,3 @@ class GraphedForces:
         self.graph.replay()
         return self.outputs
 
-
-def graphed_forces(model, pos: Tensor, atomic_number: Tensor, cell: Optional[Tensor], graph, warmup: int = 2,
-                   virial: bool = False) -> GraphedForces:
-    """Captured ``energy, dE/dpos`` of ``model`` on the prebuilt ``graph`` (``model.build_graph``); parameters must be frozen
-    (inference) and the graph must stay valid for the positions passed later (same edges, or a Verlet-skin superset list).
-    ``virial``: the capture is ``model.energy_forces_virial_graph`` and returns the per-graph virial ``[G,3,3]`` as a third
-    output (same single backward pass, plus the per-atom virial kernel and its per-graph sum)."""
-    if any(p.requires_grad for p in model.parameters()):
-        raise RuntimeError("hermnet_b200.graphed_forces: freeze the parameters first (inference path)")
-    # (a Verlet-skin superset list works too: its per-call live mask is computed by device kernels inside the capture)
-
-    def fn(p):
-        if virial:
-            out = model.energy_forces_virial_graph(p, atomic_number, cell, graph)
-            return out["energy"], -out["forces"], out["virial"]
-        q = p.detach().requires_grad_(True)
-        e, _, _ = model.forward_graph(q, atomic_number, cell, graph)
-        (g,) = torch.autograd.grad(e.sum(), q)
-        return e.detach(), g
-    return GraphedForces(fn, pos, warmup)

@@ -1,8 +1,14 @@
-"""ASE-free MD driver for BASELINE.json configs[2] ("MD inference via the ASE calculator plugin"): ASE is not
-installed in this image, so this module supplies the two pieces of ASE the plugin path needs -- an ``Atoms``-like
-container and a velocity-Verlet loop -- with ASE's attribute names, so ``NNCalculator`` is exercised exactly as ASE
-would drive it (``atoms.get_forces()`` -> ``calc.calculate(atoms)``).  ``device_resident=True`` is SURVEY 8(f) rank 1:
-positions stay on the GPU and only the graph is rebuilt per step."""
+"""MD without ASE, on the host and on the device.
+
+Host: ASE is not installed in this image, so this module supplies the two pieces of ASE the calculator plugin path needs
+(BASELINE.json configs[2]) -- ``SimpleAtoms``, an ``Atoms``-like container, and ``velocity_verlet``, a host velocity-Verlet
+loop -- with ASE's attribute names, so ``NNCalculator`` is exercised exactly as ASE would drive it (``atoms.get_forces()``
+-> ``calc.calculate(atoms)``).
+
+Device (SURVEY 8(f) rank 1): positions, velocities and forces stay on the GPU.  ``velocity_verlet_device`` (NVE),
+``langevin_device`` (NVT), ``langevin_npt_device`` (NPT) and ``relax.fire_relax_device`` (FIRE) share the input set-up
+(``_setup``: atoms, replicas of a PyG-style batch, cell) and one evaluation, ``VerletGraph.evaluate``: a Verlet-skin list
+re-used across steps, eager or replayed as a captured CUDA graph."""
 from __future__ import annotations
 
 import math
@@ -12,7 +18,7 @@ import numpy as np
 import torch
 
 from .. import ops
-from ..data import Data
+from ..graphed import GraphedForces
 from ..symbols import atomic_numbers, chemical_symbols
 
 KB_EV = 8.617333262e-5
@@ -95,7 +101,7 @@ class VerletGraph:
         # deforming: the cell may change between calls (constant-pressure MD); a list is then re-used under the
         # affine criterion of ``_fits_deformed`` instead of being rebuilt whenever the cell differs
         self.deforming = bool(deforming)
-        self.virial = bool(virial)    # captured evaluation also returns the per-graph virial (energy_forces_virial)
+        self.virial = bool(virial)    # evaluate also returns the per-graph virial (energy_forces_virial)
         self.graph, self.ref_pos, self.ref_cell, self.ref_Z = None, None, None, None
         self.builds = self.reuses = 0
         # cuda_graph: while a list is re-used, replay the whole evaluation (forward + backward, ~200 launches + torch glue) as
@@ -103,19 +109,37 @@ class VerletGraph:
         self.cuda_graph = bool(cuda_graph) and self.skin > 0.0
         self._captured, self._captured_for = None, None
 
-    def energy_and_gradient(self, pos, Z, cell):
-        """``(E [num_graphs], dE/dpos)`` at ``pos`` through the re-used (or rebuilt) list; with ``cuda_graph`` the evaluation is
-        captured once per list build and replayed afterwards (the returned tensors are then the capture's static outputs;
-        with ``virial`` the capture returns the virial ``[num_graphs,3,3]`` as a third one)."""
+    def counts(self) -> dict:
+        """The ``builds`` / ``reuses`` entries of a driver's ``stats``."""
+        return dict(builds=self.builds, reuses=self.reuses)
+
+    def evaluate(self, pos, Z, cell):
+        """``(energy [num_graphs], forces [N,3])`` at ``pos`` (cell ``[num_graphs,3,3]`` or None) through the re-used (or
+        rebuilt) list, plus the virial ``[num_graphs,3,3]`` with ``virial``.  With ``cuda_graph`` and a CUDA ``pos``, the same
+        evaluation is captured once per list build and replayed afterwards (the parameters must be frozen); the returned
+        tensors are then copies of the capture's static outputs, so they outlive the next call.  Elsewhere it runs eagerly."""
         g = self.get(pos, Z, cell)
         if self.cuda_graph and pos.is_cuda:
             if self._captured_for is not g:
-                from ..graphed import graphed_forces
-                self._captured = graphed_forces(self.model, pos, Z, cell, g, warmup=1, virial=self.virial)
+                if any(p.requires_grad for p in self.model.parameters()):
+                    raise RuntimeError("hermnet_b200.VerletGraph: freeze the parameters first (cuda_graph is inference only)")
+                # (a Verlet-skin superset list works: its per-call live mask is computed by device kernels inside the capture)
+                self._captured = GraphedForces(lambda p: self._evaluate_on(p, Z, cell, g), pos, warmup=1)
                 self._captured_for = g
-            return self._captured(pos)
+            out = self._captured(pos)
+            out = tuple(t.clone() for t in out) if self.virial else (out[0].clone(), out[1])
+        else:
+            out = self._evaluate_on(pos, Z, cell, g)
+        return out if self.virial else (out[0], -out[1])     # (on a replay the negation is also the copy of dE/dpos)
+
+    def _evaluate_on(self, pos, Z, cell, g):
+        """``(energy, forces, virial)`` of ``model.energy_forces_virial_graph`` with ``virial``, else ``(energy, dE/dpos)`` of
+        ``model.forward_graph``: what ``model(data)`` / ``model.energy_forces_virial(data)`` compute on an attached graph."""
+        if self.virial:
+            out = self.model.energy_forces_virial_graph(pos, Z, cell, g)
+            return out["energy"], out["forces"], out["virial"]
         p = pos.detach().requires_grad_(True)
-        e, _, _ = self.model.forward_graph(p, Z, None if cell is None else cell.reshape(-1, 3, 3), g)
+        e, _, _ = self.model.forward_graph(p, Z, cell, g)
         (grad,) = torch.autograd.grad(e.sum(), p)
         return e.detach(), grad
 
@@ -175,25 +199,6 @@ def _det3(a):
             + a[..., 0, 2] * (a[..., 1, 0] * a[..., 2, 1] - a[..., 1, 1] * a[..., 2, 0]))
 
 
-def _evaluator(model, vg: VerletGraph, Z, c, virial: bool):
-    """``forces(p) -> (energy [G], forces [N,3][, virial [G,3,3]])`` at positions ``p`` through ``vg``: the captured
-    replay with ``vg.cuda_graph``, else one eager forward + backward (``model.energy_forces_virial`` with ``virial``)."""
-    def forces(p):
-        if vg.cuda_graph:
-            out = vg.energy_and_gradient(p, Z, c)
-            # (static outputs of the capture: copy what outlives the next call)
-            return (out[0].clone(), -out[1]) + ((out[2].clone(),) if virial else ())
-        d = Data(pos=p.detach().requires_grad_(True), atomic_number=Z, cell=c)
-        d.graph = vg.get(d.pos, Z, c)
-        if virial:
-            out = model.energy_forces_virial(d)
-            return out["energy"], out["forces"], out["virial"]
-        e = model(d)
-        (g,) = torch.autograd.grad(e.sum(), d.pos)
-        return e.detach(), -g
-    return forces
-
-
 def _inv_mass(numbers, dev):
     masses = np.array([MASSES.get(int(z), 2.0 * int(z)) for z in np.asarray(numbers)])
     return torch.as_tensor(1.0 / (masses * AMU_A2_FS2_TO_EV), dtype=torch.float32).to(dev)
@@ -206,36 +211,37 @@ def velocity_verlet_device(model, numbers, positions, cell, velocities, steps: i
     cell list).  ``stats`` (optional dict) receives the build / re-use counts and, with ``virial``, ``stats["virial"]``: the
     global virial after each step's force evaluation, ``[steps, 3, 3]`` on the device (``model.energy_forces_virial``: the
     same single backward pass plus one per-atom virial kernel and its sum)."""
-    dev = torch.device(device)
-    Z = torch.as_tensor(np.asarray(numbers)).long().to(dev)
-    pos = torch.as_tensor(np.asarray(positions), dtype=torch.float32).to(dev)
-    vel = torch.as_tensor(np.asarray(velocities), dtype=torch.float32).to(dev).clone()      # (never the caller's buffer)
-    c = torch.as_tensor(np.asarray(cell), dtype=torch.float32).reshape(1, 3, 3).to(dev)
-    inv_m = _inv_mass(numbers, dev)[:, None]
+    st = _setup("velocity_verlet_device", numbers, positions, cell, None, device)
+    pos = st.pos
+    vel = torch.as_tensor(velocities, dtype=torch.float32, device=pos.device).clone()      # (never the caller's buffer)
+    inv_m = _inv_mass(st.numbers, pos.device)[:, None]
     vg = VerletGraph(model, skin, cuda_graph, virial)
-    forces = _evaluator(model, vg, Z, c, virial)
 
-    e, f = forces(pos)[:2]
+    e, f = vg.evaluate(pos, st.Z, st.c)[:2]
     energies, virials = [], []
     for _ in range(steps):
         _kick(vel, f, inv_m, dt_fs)
         pos = pos + dt_fs * vel
-        e, f, *w = forces(pos)
+        e, f, *w = vg.evaluate(pos, st.Z, st.c)
         _kick(vel, f, inv_m, dt_fs)
         energies.append(e)
         virials += w
     if stats is not None:
-        stats.update(builds=vg.builds, reuses=vg.reuses)
+        stats.update(vg.counts())
         if virial:
-            stats["virial"] = torch.cat(virials) if virials else c.new_zeros((0, 3, 3))
+            stats["virial"] = torch.cat(virials) if virials else st.c.new_zeros((0, 3, 3))
     return pos, vel, torch.cat(energies)
 
 
-def _replicas(batch, n: int, name: str = "langevin_device"):
+def _host(x) -> np.ndarray:
+    return x.detach().cpu().numpy() if isinstance(x, torch.Tensor) else np.asarray(x)
+
+
+def _replicas(batch, n: int, name: str):
     """``(G, replica_ptr int64 [G+1])`` of a PyG-style batch vector: non-decreasing, every replica 0..G-1 non-empty."""
     if batch is None:
         return 1, np.array([0, n], dtype=np.int64)
-    b = (batch.detach().cpu().numpy() if isinstance(batch, torch.Tensor) else np.asarray(batch)).astype(np.int64).reshape(-1)
+    b = _host(batch).astype(np.int64).reshape(-1)
     if b.size != n or n == 0:
         raise ValueError(f"{name}: batch must have one entry per atom ({n}), got {b.size}")
     step = np.diff(b)
@@ -245,54 +251,80 @@ def _replicas(batch, n: int, name: str = "langevin_device"):
     return G, np.concatenate([[0], np.cumsum(np.bincount(b, minlength=G))]).astype(np.int64)
 
 
-def _per_replica(value, G: int, what: str, name: str = "langevin_device") -> np.ndarray:
-    v = value.detach().cpu().numpy() if isinstance(value, torch.Tensor) else np.asarray(value)
+def _per_replica(value, G: int, what: str, name: str) -> np.ndarray:
+    """``value`` (one value or ``G`` values) as ``G`` values, as given."""
+    v = _host(value)
     v = np.full(G, v) if v.ndim == 0 else v.reshape(-1)
     if v.size != G:
         raise ValueError(f"{name}: {what} has {v.size} values for {G} replicas")
     return v
 
 
+def _replica_floats(value, G: int, what: str, name: str, ok, must: str) -> np.ndarray:
+    """``value`` (a float or ``G`` values) as ``G`` float64 values; ``ValueError`` with ``must`` unless ``ok`` holds for all."""
+    v = _per_replica(value, G, what, name).astype(np.float64)
+    if not ok(v).all():
+        raise ValueError(f"{name}: {must}")
+    return v
+
+
+def _setup(name, numbers, positions, cell, batch, device, cell_error=None):
+    """Validated inputs of a device driver: ``n``, ``G``, ``sizes [G]`` and ``numbers`` on the host, ``replica_ptr [G+1]`` /
+    ``replica [N]`` (int32), ``batch`` for ``VerletGraph`` (None for one replica), ``Z``, a private float32 copy of ``pos`` and
+    the float32 cell ``c [G,3,3]`` (a ``[3,3]`` cell is shared) or None.  With ``cell_error``, a missing, non-finite or
+    singular cell raises ``ValueError`` with that message."""
+    numbers = _host(numbers)
+    n = len(numbers)
+    G, rptr = _replicas(batch, n, name)
+    c_np = None if cell is None else _host(cell).astype(np.float64).reshape(-1, 3, 3)
+    if c_np is not None and c_np.shape[0] not in (1, G):
+        raise ValueError(f"{name}: cell must be [3,3] or [{G},3,3]")
+    if cell_error and (c_np is None or not np.isfinite(c_np).all() or not (np.abs(np.linalg.det(c_np)) > 0.0).all()):
+        raise ValueError(f"{name}: {cell_error}")
+
+    dev = torch.device(device)
+    sizes = np.diff(rptr)
+    replica = torch.repeat_interleave(torch.arange(G, dtype=torch.int32), torch.from_numpy(sizes)).to(dev)
+    return SimpleNamespace(
+        n=n, G=G, sizes=sizes, numbers=numbers, replica_ptr=torch.from_numpy(rptr).to(dev, torch.int32), replica=replica,
+        batch=None if batch is None else replica.long(), Z=torch.as_tensor(numbers).long().to(dev),
+        # (never the caller's buffers; device tensors are accepted, e.g. the pos of a previous call to continue from)
+        pos=torch.as_tensor(positions, dtype=torch.float32, device=dev).reshape(n, 3).clone(),
+        c=None if c_np is None else torch.from_numpy(np.repeat(c_np.astype(np.float32), G // c_np.shape[0], axis=0)).to(dev))
+
+
+def _stack(trace, like, *shape):
+    """The per-step ``trace`` as one ``[steps, *shape]`` tensor (``like``'s dtype and device when there are no steps)."""
+    return torch.stack(trace) if trace else like.new_zeros((0, *shape))
+
+
 def _langevin_state(name, numbers, positions, cell, velocities, dt_fs, temperature_K, friction_per_fs, seed, batch, step0,
-                    device):
-    """Validated inputs and device state shared by ``langevin_device`` and ``langevin_npt_device``."""
+                    device, cell_error=None):
+    """``_setup`` plus the Langevin state shared by ``langevin_device`` and ``langevin_npt_device``: velocities, inverse
+    masses, ``kT``, seeds, the step counter, the per-atom kinetic energies, ``c1`` / ``c2`` and ``t_scale``."""
     if not dt_fs > 0.0:
         raise ValueError(f"{name}: dt_fs must be > 0 (got {dt_fs})")
     if not friction_per_fs >= 0.0:
         raise ValueError(f"{name}: friction_per_fs must be >= 0 (got {friction_per_fs})")
-    numbers = numbers.cpu().numpy() if isinstance(numbers, torch.Tensor) else np.asarray(numbers)
-    n = len(numbers)
-    G, rptr = _replicas(batch, n, name)
-    T = _per_replica(temperature_K, G, "temperature_K", name).astype(np.float64)
-    if not (T >= 0.0).all():
-        raise ValueError(f"{name}: temperatures must be >= 0")
+    st = _setup(name, numbers, positions, cell, batch, device, cell_error)
+    G = st.G
+    T = _replica_floats(temperature_K, G, "temperature_K", name, lambda t: t >= 0.0, "temperatures must be >= 0")
     seeds = [int(seed) + g for g in range(G)] if np.ndim(seed) == 0 else [int(s) for s in _per_replica(seed, G, "seed", name)]
     if not all(0 <= s < 2 ** 63 for s in seeds):
         raise ValueError(f"{name}: seeds must be in [0, 2^63)")
     if not 0 <= int(step0) < 2 ** 63:
         raise ValueError(f"{name}: step0 must be in [0, 2^63)")
-    c_np = (cell.cpu().numpy() if isinstance(cell, torch.Tensor) else np.asarray(cell)).astype(np.float32).reshape(-1, 3, 3)
-    if c_np.shape[0] not in (1, G):
-        raise ValueError(f"{name}: cell must be [3,3] or [{G},3,3]")
 
-    st = SimpleNamespace(n=n, G=G)
-    dev = torch.device(device)
-    st.Z = torch.as_tensor(numbers).long().to(dev)
-    # (never the caller's buffers; device tensors are accepted, e.g. the pos / vel of a previous call to continue from)
-    st.pos = torch.as_tensor(positions, dtype=torch.float32, device=dev).clone()
+    dev = st.pos.device
     st.vel = torch.as_tensor(velocities, dtype=torch.float32, device=dev).clone()
-    st.c = torch.from_numpy(np.repeat(c_np, G // c_np.shape[0], axis=0)).to(dev)
-    st.inv_m = _inv_mass(numbers, dev)
-    st.replica_ptr = torch.from_numpy(rptr).to(dev, torch.int32)
-    st.replica = torch.repeat_interleave(torch.arange(G, dtype=torch.int32), torch.from_numpy(np.diff(rptr))).to(dev)
+    st.inv_m = _inv_mass(st.numbers, dev)
     st.kT = torch.from_numpy(KB_EV * T).to(dev, torch.float32)
     st.seed = torch.tensor(seeds, dtype=torch.int64, device=dev)
     st.step = torch.tensor([int(step0)], dtype=torch.int64, device=dev)
-    st.kinetic = torch.empty(n, dtype=torch.float32, device=dev)
-    st.t_scale = torch.from_numpy(2.0 / (3.0 * np.diff(rptr) * KB_EV)).to(dev, torch.float32)
+    st.kinetic = torch.empty(st.n, dtype=torch.float32, device=dev)
+    st.t_scale = torch.from_numpy(2.0 / (3.0 * st.sizes * KB_EV)).to(dev, torch.float32)
     gdt = float(friction_per_fs) * float(dt_fs)
     st.c1, st.c2 = math.exp(-gdt), math.sqrt(-math.expm1(-2.0 * gdt))
-    st.batch = None if batch is None else st.replica.long()
     return st
 
 
@@ -323,22 +355,20 @@ def langevin_device(model, numbers, positions, cell, velocities, steps: int, dt_
                          batch, step0, device)
     G, pos, vel, inv_m, replica_ptr, kT, step, kinetic = st.G, st.pos, st.vel, st.inv_m, st.replica_ptr, st.kT, st.step, st.kinetic
     vg = VerletGraph(model, skin, cuda_graph, virial, batch=st.batch)
-    forces = _evaluator(model, vg, st.Z, st.c, virial)
-    e, f = forces(pos)[:2]
+    e, f = vg.evaluate(pos, st.Z, st.c)[:2]
     energies, temps, virials = [], [], []
     for _ in range(steps):
         ops.md_langevin_baoa(pos, vel, f, inv_m, st.replica, replica_ptr, kT, st.seed, step, st.c1, st.c2, dt_fs)
-        e, f, *w = forces(pos)
+        e, f, *w = vg.evaluate(pos, st.Z, st.c)
         ops.md_kick(vel, f, inv_m, 0.5 * dt_fs, kinetic, step)
         energies.append(e)
         temps.append(ops.segment_sum(kinetic[:, None], replica_ptr, None, G)[:, 0] * st.t_scale)
         virials += w
     if stats is not None:
-        stats.update(builds=vg.builds, reuses=vg.reuses, step=int(step.item()),
-                     temperature=torch.stack(temps) if temps else kT.new_zeros((0, G)))
+        stats.update(vg.counts(), step=int(step.item()), temperature=_stack(temps, kT, G))
         if virial:
-            stats["virial"] = torch.stack(virials) if virials else kT.new_zeros((0, G, 3, 3))
-    return pos, vel, torch.stack(energies) if energies else kT.new_zeros((0, G))
+            stats["virial"] = _stack(virials, kT, G, 3, 3)
+    return pos, vel, _stack(energies, kT, G)
 
 
 EV_A3_TO_BAR = 1.602176634e6       # 1 eV/A^3 in bar
@@ -371,23 +401,14 @@ def langevin_npt_device(model, numbers, positions, cell, velocities, steps: int,
     ``pressure [steps, G]`` (bar: the internal pressure of the post-kick state, before the cell step), ``volume
     [steps, G]`` (A^3, after the cell step) and ``virial [steps, G, 3, 3]`` (eV)."""
     name = "langevin_npt_device"
-    if cell is None:
-        raise ValueError(f"{name}: a periodic cell is required")
-    c_np = (cell.detach().cpu().numpy() if isinstance(cell, torch.Tensor) else np.asarray(cell, dtype=np.float64))
-    c_np = c_np.astype(np.float64).reshape(-1, 3, 3)
-    if not (np.isfinite(c_np).all() and (np.abs(np.linalg.det(c_np)) > 0.0).all()):
-        raise ValueError(f"{name}: the cell must be finite and non-singular")
     if not tau_p_fs > 0.0:
         raise ValueError(f"{name}: tau_p_fs must be > 0 (got {tau_p_fs})")
     st = _langevin_state(name, numbers, positions, cell, velocities, dt_fs, temperature_K, friction_per_fs, seed, batch, step0,
-                         device)
+                         device, cell_error="a finite, non-singular periodic cell is required")
     G = st.G
-    P0 = _per_replica(pressure_bar, G, "pressure_bar", name).astype(np.float64)
-    if not np.isfinite(P0).all():
-        raise ValueError(f"{name}: pressures must be finite")
-    beta = _per_replica(compressibility_per_bar, G, "compressibility_per_bar", name).astype(np.float64)
-    if not (np.isfinite(beta).all() and (beta >= 0.0).all()):
-        raise ValueError(f"{name}: compressibilities must be finite and >= 0")
+    P0 = _replica_floats(pressure_bar, G, "pressure_bar", name, np.isfinite, "pressures must be finite")
+    beta = _replica_floats(compressibility_per_bar, G, "compressibility_per_bar", name, lambda b: np.isfinite(b) & (b >= 0.0),
+                           "compressibilities must be finite and >= 0")
 
     pos, vel, c, inv_m, replica_ptr, kT, step, kinetic = st.pos, st.vel, st.c, st.inv_m, st.replica_ptr, st.kT, st.step, st.kinetic
     dev = pos.device
@@ -396,9 +417,8 @@ def langevin_npt_device(model, numbers, positions, cell, velocities, steps: int,
     mu, pressure = torch.ones(G, dtype=torch.float32, device=dev), torch.zeros(G, dtype=torch.float32, device=dev)
 
     vg = VerletGraph(model, skin, cuda_graph, True, batch=st.batch, deforming=True)
-    evaluate = _evaluator(model, vg, st.Z, c, True)
     if forces is None:
-        f = evaluate(pos)[1]
+        f = vg.evaluate(pos, st.Z, c)[1]
     else:
         f = torch.as_tensor(forces, dtype=torch.float32, device=dev).clone()
         if tuple(f.shape) != (st.n, 3):
@@ -406,7 +426,7 @@ def langevin_npt_device(model, numbers, positions, cell, velocities, steps: int,
     energies, temps, virials, pressures, cells = [], [], [], [], []
     for _ in range(steps):
         ops.md_langevin_baoa(pos, vel, f, inv_m, st.replica, replica_ptr, kT, st.seed, step, st.c1, st.c2, dt_fs)
-        e, f, w = evaluate(pos)
+        e, f, w = vg.evaluate(pos, st.Z, c)
         ops.md_kick(vel, f, inv_m, 0.5 * dt_fs, kinetic, step)
         ke = ops.segment_sum(kinetic[:, None], replica_ptr, None, G)[:, 0]
         w = w.contiguous()
@@ -418,10 +438,7 @@ def langevin_npt_device(model, numbers, positions, cell, velocities, steps: int,
         pressures.append(pressure.clone())
         cells.append(c.clone())
     if stats is not None:
-        empty = kT.new_zeros((0, G))
-        stats.update(builds=vg.builds, reuses=vg.reuses, step=int(step.item()),
-                     temperature=torch.stack(temps) if temps else empty,
-                     pressure=torch.stack(pressures) * EV_A3_TO_BAR if pressures else empty,
-                     volume=_det3(torch.stack(cells).double()).abs().float() if cells else empty,
-                     virial=torch.stack(virials) if virials else kT.new_zeros((0, G, 3, 3)), forces=f)
-    return pos, vel, c, torch.stack(energies) if energies else kT.new_zeros((0, G))
+        stats.update(vg.counts(), step=int(step.item()), temperature=_stack(temps, kT, G),
+                     pressure=_stack(pressures, kT, G) * EV_A3_TO_BAR,
+                     volume=_det3(_stack(cells, c, G, 3, 3).double()).abs().float(), virial=_stack(virials, kT, G, 3, 3), forces=f)
+    return pos, vel, c, _stack(energies, kT, G)

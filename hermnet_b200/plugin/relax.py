@@ -9,7 +9,7 @@ import numpy as np
 import torch
 
 from .. import ops
-from .md import EV_A3_TO_BAR, VerletGraph, _det3, _evaluator, _per_replica, _replicas
+from .md import EV_A3_TO_BAR, VerletGraph, _det3, _replica_floats, _setup
 
 
 def fire_relax_device(model, numbers, positions, cell, fmax=0.05, max_steps=1000, batch=None, relax_cell=False,
@@ -51,34 +51,15 @@ def fire_relax_device(model, numbers, positions, cell, fmax=0.05, max_steps=1000
     if not int(max_steps) >= 0:
         raise ValueError(f"{name}: max_steps must be >= 0 (got {max_steps})")
     max_steps = int(max_steps)
-    numbers = numbers.cpu().numpy() if isinstance(numbers, torch.Tensor) else np.asarray(numbers)
-    n = len(numbers)
-    G, rptr = _replicas(batch, n, name)
-    c_np = None
-    if cell is not None:
-        c_np = (cell.detach().cpu().numpy() if isinstance(cell, torch.Tensor) else np.asarray(cell)).astype(np.float64).reshape(-1, 3, 3)
-        if c_np.shape[0] not in (1, G):
-            raise ValueError(f"{name}: cell must be [3,3] or [{G},3,3]")
-    if relax_cell and (c_np is None or not np.isfinite(c_np).all() or not (np.abs(np.linalg.det(c_np)) > 0.0).all()):
-        raise ValueError(f"{name}: relax_cell needs a finite, non-singular cell")
-    P0 = _per_replica(pressure_bar, G, "pressure_bar", name).astype(np.float64)
-    if not np.isfinite(P0).all():
-        raise ValueError(f"{name}: pressures must be finite")
-    cf = np.diff(rptr).astype(np.float64) if cell_factor is None else \
-        _per_replica(cell_factor, G, "cell_factor", name).astype(np.float64)
-    if not (np.isfinite(cf).all() and (cf > 0.0).all()):
-        raise ValueError(f"{name}: cell_factor must be finite and > 0")
+    st = _setup(name, numbers, positions, cell, batch, device,
+                cell_error="relax_cell needs a finite, non-singular cell" if relax_cell else None)
+    G, Z, pos, c, replica, replica_ptr = st.G, st.Z, st.pos, st.c, st.replica, st.replica_ptr
+    P0 = _replica_floats(pressure_bar, G, "pressure_bar", name, np.isfinite, "pressures must be finite")
+    cf = _replica_floats(st.sizes if cell_factor is None else cell_factor, G, "cell_factor", name,
+                         lambda v: np.isfinite(v) & (v > 0.0), "cell_factor must be finite and > 0")
+    vg = VerletGraph(model, skin, cuda_graph, relax_cell, batch=st.batch, deforming=relax_cell)
 
-    dev = torch.device(device)
-    Z = torch.as_tensor(numbers).long().to(dev)
-    # (never the caller's buffers)
-    pos = torch.as_tensor(positions, dtype=torch.float32, device=dev).reshape(n, 3).clone()
-    c = None if c_np is None else torch.from_numpy(np.repeat(c_np.astype(np.float32), G // c_np.shape[0], axis=0)).to(dev)
-    replica_ptr = torch.from_numpy(rptr).to(dev, torch.int32)
-    replica = torch.repeat_interleave(torch.arange(G, dtype=torch.int32), torch.from_numpy(np.diff(rptr))).to(dev)
-    vg = VerletGraph(model, skin, cuda_graph, relax_cell, batch=None if batch is None else replica.long(), deforming=relax_cell)
-    evaluate = _evaluator(model, vg, Z, c, relax_cell)
-
+    dev = pos.device
     f64 = dict(dtype=torch.float64, device=dev)
     dt_g, alpha = torch.full((G,), float(dt), **f64), torch.full((G,), 0.1, **f64)
     n_pos, steps, converged = (torch.zeros(G, dtype=torch.int32, device=dev) for _ in range(3))
@@ -95,7 +76,7 @@ def fire_relax_device(model, numbers, positions, cell, fmax=0.05, max_steps=1000
 
     trace = {k: [] for k in ("energy", "fmax", "volume", "dt", "alpha", "n_pos")}
     for it in range(max_steps + 1):
-        e, f, *w = evaluate(pos)
+        e, f, *w = vg.evaluate(pos, Z, c)
         sums = ops.opt_fire_reduce(f, vel, A, replica, replica_ptr)
         if relax_cell:
             trace["volume"].append(_det3(c.double()).abs())      # of the evaluated cell, before the step moves it
@@ -109,6 +90,6 @@ def fire_relax_device(model, numbers, positions, cell, fmax=0.05, max_steps=1000
             break
         ops.opt_fire_update(pos if relax_cell else None, rp, vel, f, A_prev, A, replica, converged, coef)
     if stats is not None:
-        stats.update(builds=vg.builds, reuses=vg.reuses, converged=converged.bool(), steps=steps.clone(),
+        stats.update(vg.counts(), converged=converged.bool(), steps=steps.clone(),
                      **{k: torch.stack(v) for k, v in trace.items() if v})
     return pos, c, e

@@ -13,6 +13,7 @@ import hermnet_b200 as H
 from hermnet_b200 import ops, synthetic
 from hermnet_b200.plugin import md
 from tests import util
+from tests.test_atom_virial import _emu_edge_virial_atom
 from tests.util import lattice_system
 
 DEV = "cuda:0"
@@ -92,6 +93,7 @@ def emu_md_kick(vel, force, inv_mass, half_dt, kinetic, step):
 def emu_md(emu, monkeypatch):
     monkeypatch.setattr(ops, "md_langevin_baoa", emu_md_langevin_baoa)
     monkeypatch.setattr(ops, "md_kick", emu_md_kick)
+    monkeypatch.setattr(ops, "edge_virial_atom", _emu_edge_virial_atom)
     return emu
 
 
@@ -436,6 +438,16 @@ def test_emulated_stats_restart_and_replica_independence(emu_md):
     assert np.array_equal(vel, 0.002 * np.random.default_rng(1).standard_normal(pos.shape).astype(np.float32))  # input untouched
     ke = 0.5 * (v.double() ** 2).sum(1) / md._inv_mass(Z, "cpu").double()
     assert util.rel_err(st["temperature"][-1].double(), ke.view(2, n1).sum(1) * 2.0 / (3 * n1 * md.KB_EV)) < 1e-6
+    # with the virial, eager and cuda_graph (which evaluates eagerly on CPU tensors): the same run, bitwise
+    virials = []
+    for cg in (False, True):
+        st_w = {}
+        p_w, v_w, e_w = md.langevin_device(model, Z, pos, cell, vel, steps=6, stats=st_w, virial=True, cuda_graph=cg, **kw)
+        assert torch.equal(p_w, p) and torch.equal(v_w, v) and torch.equal(e_w, e)
+        assert torch.equal(st_w["temperature"], st["temperature"]) and st_w["virial"].shape == (6, 2, 3, 3)
+        assert (st_w["builds"], st_w["reuses"], st_w["step"]) == (st["builds"], st["reuses"], st["step"])
+        virials.append(st_w["virial"])
+    assert torch.equal(virials[0], virials[1])
     # restart: 4 + 2 steps equal 6 steps (fresh lists every step)
     kw0 = dict(kw, skin=0.0)
     p6, v6, e6 = md.langevin_device(model, Z, pos, cell, vel, steps=6, **kw0)
@@ -454,8 +466,9 @@ def test_emulated_stats_restart_and_replica_independence(emu_md):
     assert e_s.shape == (2, 1) and p_s.shape == (n1, 3)
 
 
-def test_emulated_velocity_verlet_device_unchanged(emu):
-    """The shared evaluation helper keeps the NVE loop's trajectory: the loop written out as before, bitwise."""
+def test_emulated_velocity_verlet_device_unchanged(emu_md):
+    """The shared evaluation helper keeps the NVE loop's trajectory: the loop written out as before, bitwise -- also with the
+    virial, eager and with ``cuda_graph``."""
     model = _cpu_model()
     pos, Z, cell, _ = _cpu_systems((22,))
     vel = 0.002 * np.random.default_rng(2).standard_normal(pos.shape).astype(np.float32)
@@ -481,6 +494,15 @@ def test_emulated_velocity_verlet_device_unchanged(emu):
         w.add_(f * inv_m, alpha=0.25)
         es.append(en)
     assert torch.equal(p, q) and torch.equal(v, w) and torch.equal(e, torch.cat(es))
+    virials = []
+    for cg in (False, True):
+        st = {}
+        p_w, v_w, e_w = md.velocity_verlet_device(model, Z, pos, cell, vel, steps=4, device="cpu", skin=0.5, stats=st,
+                                                  cuda_graph=cg, virial=True)
+        assert torch.equal(p_w, q) and torch.equal(v_w, w) and torch.equal(e_w, torch.cat(es))
+        assert st["virial"].shape == (4, 3, 3) and (st["builds"], st["reuses"]) == (1, 4)
+        virials.append(st["virial"])
+    assert torch.equal(virials[0], virials[1])
 
 
 @pytest.mark.parametrize("bad", [

@@ -404,6 +404,12 @@ def test_emulated_stats_restart_and_zero_compressibility(emu_npt):
     assert st["builds"] + st["reuses"] == 7 and st["reuses"] > 0
     assert not torch.equal(c, torch.from_numpy(cell))
     assert util.rel_err(st["volume"][-1].double(), torch.linalg.det(c.double()).abs()) < 1e-6
+    # cuda_graph (which evaluates eagerly on CPU tensors): the same run, bitwise
+    st_g = {}
+    out_g = md.langevin_npt_device(model, Z, pos, cell, vel, steps=6, stats=st_g, skin=0.5, cuda_graph=True, **kw)
+    assert all(torch.equal(a, b) for a, b in zip(out_g, (p, v, c, e)))
+    assert st_g.keys() == st.keys()
+    assert all(torch.equal(st_g[k], st[k]) if isinstance(st[k], torch.Tensor) else st_g[k] == st[k] for k in st)
     # restart: 4 + 2 steps equal 6 steps (fresh lists every step)
     p6, v6, c6, e6 = md.langevin_npt_device(model, Z, pos, cell, vel, steps=6, **kw)
     st4 = {}

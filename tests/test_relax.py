@@ -326,6 +326,17 @@ def test_emulated_driver_matches_host_fire(emu_relax):
     pos, Z, cell, batch = _cpu_systems((31, 32))
     check_against_host_fire(model, pos, Z, cell, batch, "cpu", False, 0.0, steps=8, fmax=1e-4)
     check_against_host_fire(model, pos, Z, cell, batch, "cpu", True, [2e4, -1e4], steps=8, fmax=1e-4, dt_max=0.12)
+    # the cell relaxed with a skin list, eager and with cuda_graph (which evaluates eagerly on CPU tensors): bitwise equal
+    runs = []
+    for cg in (False, True):
+        st = {}
+        out = fire_relax_device(model, Z, pos, cell, fmax=1e-4, max_steps=8, batch=batch, relax_cell=True, pressure_bar=[2e4, -1e4],
+                                dt_max=0.12, skin=0.5, cuda_graph=cg, stats=st, device="cpu")
+        runs.append((out, st))
+    (out0, st0), (out1, st1) = runs
+    assert st0["steps"].tolist() == [8, 8] and st0["reuses"] > 0 and st0.keys() == st1.keys()
+    assert all(torch.equal(a, b) for a, b in zip(out0, out1))
+    assert all(torch.equal(st0[k], st1[k]) if isinstance(st0[k], torch.Tensor) else st0[k] == st1[k] for k in st0)
 
 
 def test_emulated_stats_and_a_replica_that_starts_converged(emu_relax):
