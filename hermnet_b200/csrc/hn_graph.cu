@@ -15,7 +15,7 @@ namespace {
 
 constexpr int kMaxGroups = 16;
 constexpr int kMaxCap = 64;
-constexpr double kSkin = 1.0 + 1e-6;  // bins are sized for rc*(1+1e-6): rounding can never drop a pair
+constexpr double kSkin = 1.0 + 1e-6;  // bins are sized for rc*(1+1e-6) plus the fp32 bound below
 
 struct GraphMeta {
     double cell[9];    // row vectors (periodic) or diag(extent) (non-periodic)
@@ -115,9 +115,22 @@ __global__ void graph_setup_kernel(const float *__restrict__ pos, const float *_
                 }
             __syncthreads();
         }
+    } else {
+        // largest |coordinate| of the graph: bounds the rounding of the periodic pair test below
+        float big = 0.f;
+        for (long long q = 3ll * a0 + threadIdx.x; q < 3ll * a1; q += blockDim.x) big = fmaxf(big, fabsf(pos[q]));
+        smax[0][threadIdx.x] = big;
+        __syncthreads();
+        for (int s = blockDim.x / 2; s > 0; s >>= 1) {
+            if (threadIdx.x < s) smax[0][threadIdx.x] = fmaxf(smax[0][threadIdx.x], smax[0][threadIdx.x + s]);
+            __syncthreads();
+        }
     }
     if (threadIdx.x != 0) return;
-    const double rcs = rc * kSkin;
+    // The periodic test subtracts the positions in fp32 (ASE): each component of pos_j - pos_i is off by up to 2^-24 of
+    // itself, at most 2^-23 max|pos|, so a kept pair can lie up to sqrt(3) 2^-23 max|pos| beyond rc -- more than the
+    // 1e-6 relative margin once |pos| reaches a few hundred A (large boxes, unwrapped trajectories).  The bins cover it.
+    const double rcs = rc * kSkin + (cell != nullptr ? ldexp((double)smax[0][0], -22) : 0.0);
     const int n_atoms = a1 - a0;
     double h[3];
     if (cell != nullptr) {

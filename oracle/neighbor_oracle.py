@@ -44,6 +44,8 @@ def neighbor_list_pbc(pos: np.ndarray, cell: np.ndarray, rc: float, centres=None
     m = _image_range(c64, rc)
     cart_w = fw @ c64
     centres = np.arange(n) if centres is None else np.asarray(centres)
+    # the exact test rounds pos_j - pos_i to fp32 (up to 2^-23 max|pos| per component): the screen must not be tighter
+    margin = 1e-3 + 2.0 ** -21 * float(np.abs(pos).max(initial=0.0))
     out_i, out_j, out_s = [], [], []
     sig = np.array([(a, b, c) for a in range(-m[0], m[0] + 1) for b in range(-m[1], m[1] + 1)
                     for c in range(-m[2], m[2] + 1)], dtype=np.int64)
@@ -54,7 +56,7 @@ def neighbor_list_pbc(pos: np.ndarray, cell: np.ndarray, rc: float, centres=None
             ci = centres[a:a + chunk]
             # cheap float64 screen in wrapped coordinates with a safety margin
             d = cart_w[None, :, :] + off[None, None, :] - cart_w[ci][:, None, :]
-            cand = np.argwhere((d * d).sum(-1) < (rc + 1e-3) ** 2)
+            cand = np.argwhere((d * d).sum(-1) < (rc + margin) ** 2)
             if cand.size == 0:
                 continue
             ii = ci[cand[:, 0]]
