@@ -103,6 +103,9 @@ SIGNATURES = {
     "hn_md_kick": (c_int32, [P, P, P, c_float, c_int64, P, P, P]),
     "hn_md_scr_barostat": (c_int32, [P, P, P, P, P, P, P, P, c_int32, c_float, c_float, P, P, P]),
     "hn_md_affine_scale": (c_int32, [P, P, P, P, c_int64, P]),
+    "hn_md_kinetic_tensor": (c_int32, [P, P, c_int64, P, P]),
+    "hn_md_scr_barostat_tri": (c_int32, [P, P, P, P, P, P, P, P, c_int32, c_float, c_float, P, P, P, P]),
+    "hn_md_affine_deform": (c_int32, [P, P, P, P, P, c_int64, P]),
     "hn_opt_fire_reduce_workspace_bytes": (c_int64, [c_int64, c_int32]),
     "hn_opt_fire_reduce": (c_int32, [P, P, P, P, P, c_int32, c_int64, P, P, c_int64, P]),
     "hn_opt_fire_step": (c_int32, [P] * 14 + [c_int32, c_double, c_double, c_double, c_int32, P, P, P, P]),

@@ -508,6 +508,48 @@ def md_affine_scale(pos: Tensor, vel: Tensor, replica: Tensor, mu: Tensor) -> No
     _bump(pos, vel)
 
 
+def md_kinetic_tensor(vel: Tensor, inv_mass: Tensor) -> Tensor:
+    """Per-atom kinetic tensors ``[N,6]``: the lower triangle ``(00, 10, 11, 20, 21, 22)`` of ``m v (x) v`` (eV) with
+    ``m = 1 / inv_mass`` (``hn_md_kinetic_tensor``)."""
+    dev = _chk("md_kinetic_tensor", f32=(vel, inv_mass))
+    n = vel.size(0)
+    if tuple(vel.shape) != (n, 3) or inv_mass.numel() != n:
+        raise RuntimeError(f"hermnet_b200.md_kinetic_tensor: expected vel [{n},3] and inv_mass [{n}]")
+    out = torch.empty((n, 6), dtype=torch.float32, device=dev)
+    _launch("hn_md_kinetic_tensor", dev, "md_kinetic_tensor", vel, inv_mass, n, out)
+    return out
+
+
+def md_scr_barostat_tri(cell: Tensor, kin6: Tensor, virial: Tensor, P0: Tensor, kT: Tensor, beta: Tensor, seed: Tensor,
+                        step: Tensor, dt: float, tau_p: float, mu: Tensor, mu_inv_t: Tensor, pressure: Tensor) -> None:
+    """Triclinic stochastic cell rescaling of ``G`` lower-triangular cells (``hn_md_scr_barostat_tri``): ``cell [G,3,3]`` is
+    deformed in place to ``cell mu``; ``mu``, ``mu_inv_t`` (``mu^-T``) and ``pressure`` (the internal pressure tensor of the
+    undeformed cell, eV/A^3) ``[G,3,3]`` are written.  Inputs: per-replica kinetic tensors ``kin6 [G,6]`` (eV, packed lower
+    triangle), ``virial [G,3,3]`` (eV, lower triangle read), ``P0 [G]`` (eV/A^3), ``kT [G]`` (eV), ``beta [G]`` (A^3/eV,
+    >= 0), ``seed int64 [G]`` and ``step int64 [1]`` (read)."""
+    dev = _chk("md_scr_barostat_tri", f32=(cell, kin6, virial, P0, kT, beta, mu, mu_inv_t, pressure), i64=(seed, step))
+    G = P0.numel()
+    if (any(tuple(t.shape) != (G, 3, 3) for t in (cell, virial, mu, mu_inv_t, pressure)) or tuple(kin6.shape) != (G, 6)
+            or step.numel() != 1 or any(t.numel() != G for t in (kT, beta, seed))):
+        raise RuntimeError(f"hermnet_b200.md_scr_barostat_tri: expected cell / virial / mu / mu_inv_t / pressure [G={G},3,3], "
+                           "kin6 [G,6], P0 / kT / beta / seed [G] and step [1]")
+    _launch("hn_md_scr_barostat_tri", dev, "md_scr_barostat_tri", cell, kin6, virial, P0, kT, beta, seed, step, G, float(dt),
+            float(tau_p), mu, mu_inv_t, pressure)
+    _bump(cell, mu, mu_inv_t, pressure)
+
+
+def md_affine_deform(pos: Tensor, vel: Tensor, replica: Tensor, mu: Tensor, mu_inv_t: Tensor) -> None:
+    """``pos = pos mu[replica]``, ``vel = vel mu_inv_t[replica]`` in place on ``[N,3]`` (row vectors; ``hn_md_affine_deform``;
+    ``replica int32 [N]``, ``mu`` / ``mu_inv_t [G,3,3]``)."""
+    dev = _chk("md_affine_deform", f32=(pos, vel, mu, mu_inv_t), i32=(replica,))
+    n = pos.size(0)
+    if (tuple(pos.shape) != (n, 3) or tuple(vel.shape) != (n, 3) or replica.numel() != n or mu.dim() != 3
+            or tuple(mu.shape[1:]) != (3, 3) or mu_inv_t.shape != mu.shape):
+        raise RuntimeError(f"hermnet_b200.md_affine_deform: expected pos / vel [{n},3], replica [{n}] and mu / mu_inv_t [G,3,3]")
+    _launch("hn_md_affine_deform", dev, "md_affine_deform", pos, vel, replica, mu, mu_inv_t, n)
+    _bump(pos, vel)
+
+
 # ----------------------------------------------------------------------------------------------------
 # FIRE structure relaxation (csrc/hn_opt.cu)
 # ----------------------------------------------------------------------------------------------------

@@ -377,7 +377,7 @@ EV_A3_TO_BAR = 1.602176634e6       # 1 eV/A^3 in bar
 def langevin_npt_device(model, numbers, positions, cell, velocities, steps: int, dt_fs: float = 0.5, temperature_K=300.0,
                         pressure_bar=1.0, compressibility_per_bar=4.5e-5, tau_p_fs: float = 1000.0,
                         friction_per_fs: float = 0.01, seed=0, batch=None, step0: int = 0, device="cuda", skin: float = 0.0,
-                        stats: dict = None, cuda_graph: bool = False, forces=None):
+                        stats: dict = None, cuda_graph: bool = False, forces=None, cell_dof: str = "isotropic"):
     """Device-resident constant-pressure (NPT) MD: the ``langevin_device`` step followed by isotropic stochastic cell
     rescaling (Bernetti & Bussi 2020) of every replica towards its own pressure.  Returns ``(pos [N,3], vel [N,3],
     cell [G,3,3], energies [steps, G])``; positions, velocities, cells and forces never leave the GPU.
@@ -397,15 +397,32 @@ def langevin_npt_device(model, numbers, positions, cell, velocities, steps: int,
     ``pos`` / ``vel`` / ``cell`` with ``step0 = stats["step"]`` and ``forces = stats["forces"]`` reproduces the
     uninterrupted trajectory bitwise (same skin / evaluation mode).  ``forces=None`` evaluates them at ``positions``.
 
+    ``cell_dof="triclinic"`` frees the cell's shape under the hydrostatic target pressure: every replica's cell must then be
+    lower-triangular with a positive diagonal (``a`` along x, ``b`` in the xy plane; ``standard_cell`` rotates a system into
+    that form).  The cell step is then the triclinic stochastic cell rescaling of DESIGN.md: the per-replica kinetic tensor
+    (``ops.md_kinetic_tensor`` and a segment sum), a lower-triangular strain ``mu`` from the pressure tensor
+    (``ops.md_scr_barostat_tri``, noise on counter word 3 = 2) and ``x <- x mu``, ``v <- v mu^-T``
+    (``ops.md_affine_deform``).  Zero compressibility again reproduces ``langevin_device`` bitwise, and restarts, ``skin``
+    and ``cuda_graph`` work as in the isotropic mode.
+
     ``stats`` (optional dict) receives ``builds`` / ``reuses``, ``step``, ``temperature [steps, G]`` (K),
     ``pressure [steps, G]`` (bar: the internal pressure of the post-kick state, before the cell step), ``volume
-    [steps, G]`` (A^3, after the cell step) and ``virial [steps, G, 3, 3]`` (eV)."""
+    [steps, G]`` (A^3, after the cell step) and ``virial [steps, G, 3, 3]`` (eV); with ``cell_dof="triclinic"`` also
+    ``cell [steps, G, 3, 3]`` (after the cell step) and ``pressure_tensor [steps, G, 3, 3]`` (bar, of the post-kick state;
+    ``pressure`` is a third of its trace)."""
     name = "langevin_npt_device"
     if not tau_p_fs > 0.0:
         raise ValueError(f"{name}: tau_p_fs must be > 0 (got {tau_p_fs})")
+    if cell_dof not in ("isotropic", "triclinic"):
+        raise ValueError(f"{name}: cell_dof must be 'isotropic' or 'triclinic' (got {cell_dof!r})")
     st = _langevin_state(name, numbers, positions, cell, velocities, dt_fs, temperature_K, friction_per_fs, seed, batch, step0,
                          device, cell_error="a finite, non-singular periodic cell is required")
     G = st.G
+    if cell_dof == "triclinic":
+        h = st.c.detach().cpu().double()
+        if not (torch.equal(h.triu(1), torch.zeros_like(h)) and bool((h.diagonal(dim1=1, dim2=2) > 0.0).all())):
+            raise ValueError(f"{name}: cell_dof='triclinic' needs every cell lower-triangular with a positive diagonal "
+                             "(rotate the system with plugin.md.standard_cell)")
     P0 = _replica_floats(pressure_bar, G, "pressure_bar", name, np.isfinite, "pressures must be finite")
     beta = _replica_floats(compressibility_per_bar, G, "compressibility_per_bar", name, lambda b: np.isfinite(b) & (b >= 0.0),
                            "compressibilities must be finite and >= 0")
@@ -414,7 +431,6 @@ def langevin_npt_device(model, numbers, positions, cell, velocities, steps: int,
     dev = pos.device
     P0_t = torch.from_numpy(P0 / EV_A3_TO_BAR).to(dev, torch.float32)            # eV/A^3
     beta_t = torch.from_numpy(beta * EV_A3_TO_BAR).to(dev, torch.float32)        # A^3/eV
-    mu, pressure = torch.ones(G, dtype=torch.float32, device=dev), torch.zeros(G, dtype=torch.float32, device=dev)
 
     vg = VerletGraph(model, skin, cuda_graph, True, batch=st.batch, deforming=True)
     if forces is None:
@@ -423,6 +439,9 @@ def langevin_npt_device(model, numbers, positions, cell, velocities, steps: int,
         f = torch.as_tensor(forces, dtype=torch.float32, device=dev).clone()
         if tuple(f.shape) != (st.n, 3):
             raise ValueError(f"{name}: forces must be [{st.n},3]")
+    if cell_dof == "triclinic":
+        return _npt_triclinic(st, vg, f, steps, dt_fs, tau_p_fs, P0_t, beta_t, stats)
+    mu, pressure = torch.ones(G, dtype=torch.float32, device=dev), torch.zeros(G, dtype=torch.float32, device=dev)
     energies, temps, virials, pressures, cells = [], [], [], [], []
     for _ in range(steps):
         ops.md_langevin_baoa(pos, vel, f, inv_m, st.replica, replica_ptr, kT, st.seed, step, st.c1, st.c2, dt_fs)
@@ -442,3 +461,60 @@ def langevin_npt_device(model, numbers, positions, cell, velocities, steps: int,
                      pressure=_stack(pressures, kT, G) * EV_A3_TO_BAR,
                      volume=_det3(_stack(cells, c, G, 3, 3).double()).abs().float(), virial=_stack(virials, kT, G, 3, 3), forces=f)
     return pos, vel, c, _stack(energies, kT, G)
+
+
+def _npt_triclinic(st, vg, f, steps, dt_fs, tau_p_fs, P0_t, beta_t, stats):
+    """The step loop of ``langevin_npt_device(cell_dof="triclinic")`` from its validated state ``st``, evaluation ``vg`` and
+    first forces ``f``."""
+    G, pos, vel, c, inv_m, replica_ptr, kT, step, kinetic = st.G, st.pos, st.vel, st.c, st.inv_m, st.replica_ptr, st.kT, st.step, \
+        st.kinetic
+    mu, mu_inv_t, ptensor = (torch.zeros(G, 3, 3, dtype=torch.float32, device=pos.device) for _ in range(3))
+    energies, temps, virials, ptensors, cells = [], [], [], [], []
+    for _ in range(steps):
+        ops.md_langevin_baoa(pos, vel, f, inv_m, st.replica, replica_ptr, kT, st.seed, step, st.c1, st.c2, dt_fs)
+        e, f, w = vg.evaluate(pos, st.Z, c)
+        ops.md_kick(vel, f, inv_m, 0.5 * dt_fs, kinetic, step)
+        ke = ops.segment_sum(kinetic[:, None], replica_ptr, None, G)[:, 0]
+        kin6 = ops.segment_sum(ops.md_kinetic_tensor(vel, inv_m), replica_ptr, None, G)
+        w = w.contiguous()
+        ops.md_scr_barostat_tri(c, kin6, w, P0_t, kT, beta_t, st.seed, step, dt_fs, tau_p_fs, mu, mu_inv_t, ptensor)
+        ops.md_affine_deform(pos, vel, st.replica, mu, mu_inv_t)
+        energies.append(e)
+        temps.append(ke * st.t_scale)
+        virials.append(w)
+        ptensors.append(ptensor.clone())
+        cells.append(c.clone())
+    if stats is not None:
+        pt = _stack(ptensors, kT, G, 3, 3) * EV_A3_TO_BAR
+        cs = _stack(cells, c, G, 3, 3)
+        stats.update(vg.counts(), step=int(step.item()), temperature=_stack(temps, kT, G),
+                     pressure=pt.diagonal(dim1=2, dim2=3).sum(-1) / 3.0, volume=_det3(cs.double()).abs().float(),
+                     virial=_stack(virials, kT, G, 3, 3), forces=f, cell=cs, pressure_tensor=pt)
+    return pos, vel, c, _stack(energies, kT, G)
+
+
+def standard_cell(positions, cell, velocities=None, batch=None):
+    """Rotate each replica into the lower-triangular cell form ``langevin_npt_device(cell_dof="triclinic")`` needs: lattice
+    vector ``a`` along x, ``b`` in the xy plane, positive diagonal (ASE's and LAMMPS's standard orientation).  Per replica
+    ``g`` the LQ factorisation ``h = L Q`` (lattice vectors = rows of ``h``, ``diag L > 0``) gives the rotation ``R = Q^T``,
+    and ``x R``, ``v R``, ``L`` are returned as float64 numpy ``(positions [N,3], cell, velocities [N,3] or None)``; the cell
+    keeps the input's ``[3,3]`` or ``[G,3,3]`` shape, with its upper triangle exactly 0.  ``batch`` as in the drivers (None:
+    one system).  Distances, energies and the model's forces (rotated by ``R``) are unchanged.  A left-handed cell
+    (``det h < 0``) raises ``ValueError``: no rotation makes it lower-triangular with a positive diagonal."""
+    x = _host(positions).astype(np.float64).reshape(-1, 3)
+    n = len(x)
+    G, rptr = _replicas(batch, n, "standard_cell")
+    h = _host(cell).astype(np.float64)
+    hs = h.reshape(-1, 3, 3)
+    if hs.shape[0] not in (1, G):
+        raise ValueError(f"standard_cell: cell must be [3,3] or [{G},3,3]")
+    if not np.isfinite(hs).all() or not (np.linalg.det(hs) > 0.0).all():
+        raise ValueError("standard_cell: every cell must be finite and right-handed (det h > 0)")
+    q, r = np.linalg.qr(np.swapaxes(hs, 1, 2))          # h^T = q r  ->  h = r^T q^T, L = r^T
+    sgn = np.sign(np.diagonal(r, axis1=1, axis2=2))
+    L = np.tril(np.swapaxes(r, 1, 2) * sgn[:, None, :])
+    R = q * sgn[:, None, :]                              # h R = L with R = q diag(sgn), a rotation since det h > 0
+    rep = np.repeat(np.arange(G) if hs.shape[0] == G else np.zeros(G, dtype=np.int64), np.diff(rptr))
+    rot = lambda a: np.einsum("ni,nij->nj", a, R[rep])  # noqa: E731
+    v = None if velocities is None else rot(_host(velocities).astype(np.float64).reshape(n, 3))
+    return rot(x), L.reshape(h.shape), v

@@ -441,6 +441,48 @@ int hn_md_affine_scale(float *pos /*[N,3]*/, float *vel /*[N,3]*/, const int32_t
                        int64_t n_atoms, void *stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * Constant pressure with the cell shape free: triclinic stochastic cell rescaling of lower-triangular cells (lattice
+ * vectors = rows of h, h upper triangle 0, diagonal > 0: a along x, b in the xy plane), run after hn_md_kick.  Units and
+ * per-replica device arrays as in hn_md_scr_barostat.  Lower triangles are packed (00, 10, 11, 20, 21, 22).
+ *   hn_md_kinetic_tensor     one thread per atom:  out[i] = (m v (x) v) lower triangle, m = 1 / inv_mass[i] (fp32); the
+ *                            caller sums it per replica (hn_segment_sum) into kin6[g] = sum_i m v (x) v.
+ *   hn_md_scr_barostat_tri   one thread per replica g, float64 inside:
+ *                              V = h00 h11 h22,  P = (kin6[g] + W_g) / V on the lower triangle (only the lower triangle of
+ *                              virial is read; the force pass's W = sum pos (x) F - h^T dE/dh is symmetric to rounding),
+ *                              b = beta[g] dt / tau_p,
+ *                              delta = (b/3) (P - P0[g] I) + (b kT[g] / 3V) diag(2, 0, -2) + sqrt(2 b kT[g] / 3V) xi
+ *                              (lower-triangular; xi = 6 unit normals),
+ *                              mu = expm(delta) in closed form (diagonal exponentials, divided differences of exp for the
+ *                              off-diagonal entries, expm1-based / series forms for close diagonal entries),
+ *                              cell_g = float(h mu) (lower triangle; the upper triangle is written as exact zeros),
+ *                              mu_out[g] = float(mu), mu_inv_t[g] = float(expm(-delta)^T) (upper-triangular),
+ *                              pressure[g] = the symmetric tensor with lower triangle float(P) (eV/A^3).
+ *                            The drift's diag(2, 0, -2) makes rho ~ exp(-(U + K + P0 V)/kT) / (h11 h22^2) in (h, s = x h^-1,
+ *                            pi = p h^T) stationary (DESIGN.md, "Triclinic constant pressure"); tr delta has the law of the
+ *                            isotropic barostat's strain.  beta = 0 gives mu = I and the cell unchanged bitwise.
+ *   hn_md_affine_deform      one thread per atom i of replica g = replica[i] (fp32, in place, row vectors):
+ *                              pos_i = pos_i mu[g],  vel_i = vel_i mu_inv_t[g];  mu = I leaves pos / vel bitwise unchanged.
+ *                            With the cell deformed by the same mu every edge vector becomes D mu exactly.
+ * Noise (normative): for replica g at counter value n = *step (read after hn_md_kick advanced it),
+ *   r_k = Philox4x32-10(counter = (k, lo32(n), hi32(n), 2), key = (lo32(seed[g]), hi32(seed[g])))   (k = 0, 1),
+ *   u = float((r >> 9) * 2 + 1) * 2^-24 of each word (as in hn_md_langevin_baoa),
+ *   per k: z = sqrt(-2 ln u0) cos(2 pi u1), sqrt(-2 ln u0) sin(2 pi u1), sqrt(-2 ln u2) cos(2 pi u3), sqrt(-2 ln u2) sin(2 pi u3)
+ *   (float64), and xi = the first 6 of the 8 values in the packed order.  Counter word 3 = 2 keeps this stream disjoint from
+ *   the Langevin noise (0) and the isotropic barostat's (1).
+ * Lower-triangular cells with a positive diagonal and beta[g] >= 0 are the caller's precondition.
+ * Checks: n_replicas >= 0, dt > 0, tau_p > 0, 0 <= n_atoms < 2^31, non-null pointers when there is work (n_replicas == 0 /
+ * n_atoms == 0: no-op).
+ * ------------------------------------------------------------------------------------------- */
+int hn_md_kinetic_tensor(const float *vel /*[N,3]*/, const float *inv_mass /*[N]*/, int64_t n_atoms, float *out /*[N,6]*/,
+                         void *stream);
+int hn_md_scr_barostat_tri(float *cell /*[G,3,3]*/, const float *kin6 /*[G,6]*/, const float *virial /*[G,3,3]*/,
+                           const float *P0 /*[G]*/, const float *kT /*[G]*/, const float *beta /*[G]*/, const int64_t *seed /*[G]*/,
+                           const int64_t *step /*[1]*/, int32_t n_replicas, float dt, float tau_p, float *mu /*[G,3,3]*/,
+                           float *mu_inv_t /*[G,3,3]*/, float *pressure /*[G,3,3]*/, void *stream);
+int hn_md_affine_deform(float *pos /*[N,3]*/, float *vel /*[N,3]*/, const int32_t *replica /*[N]*/, const float *mu /*[G,3,3]*/,
+                        const float *mu_inv_t /*[G,3,3]*/, int64_t n_atoms, void *stream);
+
+/* ---------------------------------------------------------------------------------------------
  * Structure relaxation: FIRE (Bitzek et al., PRL 97, 170201 (2006)) with ASE's rules, per replica g, over the generalized
  * coordinates of ASE's UnitCellFilter in row-vector convention (lattice vectors = rows of h).  Masses are ignored.
  * Replicas are contiguous as in hn_md_langevin_baoa (replica[N], replica_ptr[G+1]).
