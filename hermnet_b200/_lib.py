@@ -110,6 +110,10 @@ SIGNATURES = {
     "hn_opt_fire_reduce": (c_int32, [P, P, P, P, P, c_int32, c_int64, P, P, c_int64, P]),
     "hn_opt_fire_step": (c_int32, [P] * 14 + [c_int32, c_double, c_double, c_double, c_int32, P, P, P, P]),
     "hn_opt_fire_update": (c_int32, [P] * 9 + [c_int64, P]),
+    "hn_neb_reduce_workspace_bytes": (c_int64, [c_int64, c_int32]),
+    "hn_neb_reduce": (c_int32, [P] * 7 + [c_int32, c_int32, c_int64, P, P, c_int64, P]),
+    "hn_neb_step": (c_int32, [P] * 4 + [c_int32, c_int32, c_int32, P, P, P]),
+    "hn_neb_project": (c_int32, [P] * 7 + [c_int32, c_int32, P, c_int64, P]),
 }
 
 

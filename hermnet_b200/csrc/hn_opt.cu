@@ -6,26 +6,22 @@
 //                        max_step cap in closed form from the three sums (no second pass over the atoms)
 //   update  per atom:    v = c_v v + c_f F',  r' += s dt v,  x = r' A
 #include "hn_common.cuh"
+#include "hn_reduce.cuh"
 
 namespace {
 
-constexpr int OPT_CHUNK = 256;        // atoms of one warp's piece in the reduce (8 per lane)
 constexpr int OPT_N_MIN = 5;
 constexpr double OPT_F_INC = 1.1, OPT_F_DEC = 0.5, OPT_ALPHA_START = 0.1, OPT_F_ALPHA = 0.99;
 
-struct Sums {
+// (F'.v, |F'|^2, |v|^2, max |F'_i|^2); 32-byte aligned: one vector access per workspace slot
+struct alignas(32) Sums {
     double fv, ff, vv, fm;
-};
-
-__device__ __forceinline__ void warp_reduce(Sums &s) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-        s.fv += __shfl_xor_sync(0xffffffffu, s.fv, o);
-        s.ff += __shfl_xor_sync(0xffffffffu, s.ff, o);
-        s.vv += __shfl_xor_sync(0xffffffffu, s.vv, o);
-        s.fm = fmax(s.fm, __shfl_xor_sync(0xffffffffu, s.fm, o));
+    __device__ __forceinline__ void merge(const Sums &o) { fv += o.fv, ff += o.ff, vv += o.vv, fm = fmax(fm, o.fm); }
+    __device__ __forceinline__ Sums shfl_xor(int o) const {
+        return {__shfl_xor_sync(0xffffffffu, fv, o), __shfl_xor_sync(0xffffffffu, ff, o), __shfl_xor_sync(0xffffffffu, vv, o),
+                __shfl_xor_sync(0xffffffffu, fm, o)};
     }
-}
+};
 
 // F' = f A^T (row vector): F'_j = sum_k f_k A[j][k];  A == nullptr: F' = f
 __device__ __forceinline__ void gen_force(const float *__restrict__ f, const double *__restrict__ A, double out[3]) {
@@ -38,26 +34,17 @@ __device__ __forceinline__ void gen_force(const float *__restrict__ f, const dou
     for (int j = 0; j < 3; ++j) out[j] = f0 * A[3 * j] + f1 * A[3 * j + 1] + f2 * A[3 * j + 2];
 }
 
-// One warp per OPT_CHUNK-atom chunk b; the piece (chunk b) x (replica g) goes to slot b + g, which is unique because b + g
-// strictly increases along the atoms.  Lanes stride over the piece, then a fixed xor tree: deterministic.
 __global__ void opt_fire_reduce_pieces_kernel(const float *__restrict__ force, const float *__restrict__ vel,
                                               const double *__restrict__ A, const int *__restrict__ replica,
                                               const int *__restrict__ replica_ptr, int n_atoms, int n_chunks,
-                                              double4 *__restrict__ part) {
-    const int b = (int)((blockIdx.x * (size_t)blockDim.x + threadIdx.x) >> 5), lane = threadIdx.x & 31;
-    if (b >= n_chunks) return;
-    const int a0 = b * OPT_CHUNK, a1 = min(a0 + OPT_CHUNK, n_atoms);
-    const int g_last = __ldg(replica + a1 - 1);
-    for (int g = __ldg(replica + a0); g <= g_last; ++g) {
-        const int s = max(a0, __ldg(replica_ptr + g)), e = min(a1, __ldg(replica_ptr + g + 1));
-        if (s >= e) continue;
+                                              Sums *__restrict__ part) {
+    hn::reduce_pieces<Sums>(replica, replica_ptr, n_atoms, n_chunks, part, [&](int g) {
         double Ag[9];
         if (A != nullptr) {
 #pragma unroll
             for (int k = 0; k < 9; ++k) Ag[k] = __ldg(A + 9 * (size_t)g + k);
         }
-        Sums acc{0.0, 0.0, 0.0, 0.0};
-        for (int i = s + lane; i < e; i += 32) {
+        return [=](Sums &acc, int i) {
             double F[3];
             gen_force(force + 3 * (size_t)i, A != nullptr ? Ag : nullptr, F);
             const double v0 = vel[3 * (size_t)i], v1 = vel[3 * (size_t)i + 1], v2 = vel[3 * (size_t)i + 2];
@@ -66,43 +53,16 @@ __global__ void opt_fire_reduce_pieces_kernel(const float *__restrict__ force, c
             acc.ff += f2;
             acc.vv += v0 * v0 + v1 * v1 + v2 * v2;
             acc.fm = fmax(acc.fm, f2);
-        }
-        warp_reduce(acc);
-        if (lane == 0) part[b + g] = make_double4(acc.fv, acc.ff, acc.vv, acc.fm);
-    }
+        };
+    });
 }
 
-// `per` threads (32 or 256) sum the slots of one replica in a fixed order; out[g] = (F'.v, |F'|^2, |v|^2, max |F'_i|^2)
-__global__ void opt_fire_reduce_final_kernel(const double4 *__restrict__ part, const int *__restrict__ replica_ptr,
+// out[g] = (F'.v, |F'|^2, |v|^2, max |F'_i|^2)
+__global__ void opt_fire_reduce_final_kernel(const Sums *__restrict__ part, const int *__restrict__ replica_ptr,
                                              int n_replicas, int per, double *__restrict__ out) {
-    __shared__ Sums warp_acc[8];
-    const int g = (int)((blockIdx.x * (size_t)blockDim.x + threadIdx.x) / per), t = threadIdx.x % per;
-    Sums acc{0.0, 0.0, 0.0, 0.0};
-    if (g < n_replicas) {
-        const int p0 = __ldg(replica_ptr + g), p1 = __ldg(replica_ptr + g + 1);
-        if (p1 > p0) {
-            const int b1 = (p1 - 1) / OPT_CHUNK;
-#pragma unroll 4
-            for (int b = p0 / OPT_CHUNK + t; b <= b1; b += per) {
-                const double4 d = part[b + g];
-                acc.fv += d.x, acc.ff += d.y, acc.vv += d.z, acc.fm = fmax(acc.fm, d.w);
-            }
-        }
-    }
-    warp_reduce(acc);
-    if (per > 32) {                           // one replica per block: combine the 8 warps in order
-        if ((threadIdx.x & 31) == 0) warp_acc[threadIdx.x >> 5] = acc;
-        __syncthreads();
-        if (threadIdx.x != 0) return;
-        acc = warp_acc[0];
-        for (int w = 1; w < 8; ++w) {
-            acc.fv += warp_acc[w].fv, acc.ff += warp_acc[w].ff, acc.vv += warp_acc[w].vv;
-            acc.fm = fmax(acc.fm, warp_acc[w].fm);
-        }
-    } else if (t != 0) {
-        return;
-    }
-    if (g >= n_replicas) return;
+    int g;
+    Sums acc;
+    if (!hn::reduce_slots(part, replica_ptr, n_replicas, per, g, acc)) return;
     double *o = out + 4 * (size_t)g;
     o[0] = acc.fv, o[1] = acc.ff, o[2] = acc.vv, o[3] = acc.fm;
 }
@@ -237,13 +197,11 @@ __global__ void opt_fire_update_kernel(float *__restrict__ x, float *__restrict_
     for (int k = 0; k < 3; ++k) x[b + k] = (float)(r[0] * __ldg(Ag + k) + r[1] * __ldg(Ag + 3 + k) + r[2] * __ldg(Ag + 6 + k));
 }
 
-inline int64_t opt_chunks(int64_t n_atoms) { return (n_atoms + OPT_CHUNK - 1) / OPT_CHUNK; }
-
 }  // namespace
 
 extern "C" int64_t hn_opt_fire_reduce_workspace_bytes(int64_t n_atoms, int32_t n_replicas) {
     if (n_atoms <= 0 || n_replicas <= 0) return 0;
-    return (opt_chunks(n_atoms) + n_replicas) * (int64_t)sizeof(double4);
+    return (hn::reduce_chunks(n_atoms) + n_replicas) * (int64_t)sizeof(Sums);
 }
 
 extern "C" int hn_opt_fire_reduce(const float *force, const float *vel, const double *A, const int32_t *replica,
@@ -256,13 +214,12 @@ extern "C" int hn_opt_fire_reduce(const float *force, const float *vel, const do
     cudaStream_t s = (cudaStream_t)stream;
     HN_REQUIRE(workspace && workspace_bytes >= hn_opt_fire_reduce_workspace_bytes(n_atoms, n_replicas), "hn_opt_fire_reduce",
                "workspace smaller than hn_opt_fire_reduce_workspace_bytes");
-    const int64_t chunks = opt_chunks(n_atoms);
-    double4 *part = (double4 *)workspace;
+    const int64_t chunks = hn::reduce_chunks(n_atoms);
+    Sums *part = (Sums *)workspace;
     opt_fire_reduce_pieces_kernel<<<(unsigned)((chunks * 32 + 255) / 256), 256, 0, s>>>(force, vel, A, replica, replica_ptr,
                                                                                          (int)n_atoms, (int)chunks, part);
     HN_CUDA(cudaGetLastError(), "hn_opt_fire_reduce");
-    // a block per replica when replicas span many chunks on average, else a warp per replica
-    const int per = chunks >= 64 * (int64_t)n_replicas ? 256 : 32;
+    const int per = hn::reduce_slot_threads(chunks, n_replicas);
     opt_fire_reduce_final_kernel<<<(unsigned)(((int64_t)n_replicas * per + 255) / 256), 256, 0, s>>>(part, replica_ptr, n_replicas,
                                                                                                     per, sums);
     return hn::check_launch("hn_opt_fire_reduce");

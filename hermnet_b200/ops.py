@@ -622,6 +622,69 @@ def opt_fire_update(x: Optional[Tensor], rp: Tensor, vel: Tensor, force: Tensor,
 
 
 # ----------------------------------------------------------------------------------------------------
+# nudged elastic band forces (csrc/hn_neb.cu)
+# ----------------------------------------------------------------------------------------------------
+def _neb_layout(name: str, pos: Tensor, initial: Tensor, final: Tensor, image: Tensor, image_ptr: Tensor, band_ptr: Tensor,
+                n_images: int):
+    """``(M, B)`` of the band-major layout: ``pos [M,3]`` with ``M = K N``, endpoints ``[N,3]``, ``image [M]``,
+    ``image_ptr [B K + 1]``, ``band_ptr [B+1]``."""
+    m, B, K = pos.size(0), band_ptr.numel() - 1, int(n_images)
+    n = initial.size(0)
+    if (K < 1 or tuple(pos.shape) != (m, 3) or tuple(initial.shape) != (n, 3) or tuple(final.shape) != (n, 3) or m != K * n
+            or image.numel() != m or image_ptr.numel() != B * K + 1):
+        raise RuntimeError(f"hermnet_b200.{name}: expected pos [K N,3], initial / final [N,3], image [K N], "
+                           f"image_ptr [B K+1] and band_ptr [B+1] with K = n_images >= 1 (got K={K}, pos {tuple(pos.shape)}, "
+                           f"initial {tuple(initial.shape)}, final {tuple(final.shape)}, image {image.numel()}, "
+                           f"image_ptr {image_ptr.numel()}, band_ptr {band_ptr.numel()})")
+    return m, B
+
+
+def neb_reduce(pos: Tensor, force: Tensor, initial: Tensor, final: Tensor, image: Tensor, image_ptr: Tensor, band_ptr: Tensor,
+               n_images: int) -> Tensor:
+    """Per-image float64 ``[B K,5]``: ``(|D+|^2, |D-|^2, D+.D-, F.D+, F.D-)`` of the band-major images (``hn_neb_reduce``;
+    ``D+ = R_{k+1} - R_k``, ``D- = R_k - R_{k-1}``, endpoints from ``initial`` / ``final``).  Deterministic."""
+    dev = _chk("neb_reduce", f32=(pos, force, initial, final), i32=(image, image_ptr, band_ptr))
+    m, B = _neb_layout("neb_reduce", pos, initial, final, image, image_ptr, band_ptr, n_images)
+    if tuple(force.shape) != (m, 3):
+        raise RuntimeError(f"hermnet_b200.neb_reduce: expected force [{m},3], got {tuple(force.shape)}")
+    n_img = B * int(n_images)
+    sums = (torch.empty if m else torch.zeros)((n_img, 5), dtype=torch.float64, device=dev)
+    ws_bytes = int(_lib.load().hn_neb_reduce_workspace_bytes(m, n_img))
+    ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev) if ws_bytes else None
+    _launch("hn_neb_reduce", dev, "neb_reduce", pos, force, initial, final, image, image_ptr, band_ptr, B, int(n_images), m, sums,
+            ws, ws_bytes, kernels=2)
+    return sums
+
+
+def neb_step(sums: Tensor, energy: Tensor, end_energy: Tensor, spring: Tensor, climb: bool, coef: Tensor, imax: Tensor) -> None:
+    """Tangent weights, climbing image and projection coefficients of ``B`` bands of ``K`` images (``hn_neb_step``, float64):
+    ``sums [B K,5]`` of ``neb_reduce``, image energies ``energy [B K]`` and ``end_energy [B,2]`` (fp32), ``spring [B]``
+    (eV/A^2, float64).  Writes ``coef [B K,2]`` (float64) and ``imax [B]`` (int32, the first highest image, 1..K)."""
+    dev = _chk("neb_step", f32=(energy, end_energy), f64=(sums, spring, coef), i32=(imax,))
+    B = spring.numel()
+    n_img = energy.numel()
+    if (B == 0 and n_img) or (B and n_img % B) or end_energy.numel() != 2 * B or imax.numel() != B \
+            or sums.numel() != 5 * n_img or coef.numel() != 2 * n_img:
+        raise RuntimeError(f"hermnet_b200.neb_step: expected sums [B K,5], energy [B K], end_energy [B,2], spring / imax [B] "
+                           f"and coef [B K,2] (got B={B}, energy {n_img}, sums {sums.numel()}, coef {coef.numel()})")
+    K = n_img // B if B else 1
+    _launch("hn_neb_step", dev, "neb_step", sums, energy, end_energy, spring, int(bool(climb)), B, K, coef, imax)
+    _bump(coef, imax)
+
+
+def neb_project(force: Tensor, pos: Tensor, initial: Tensor, final: Tensor, image: Tensor, image_ptr: Tensor, band_ptr: Tensor,
+                n_images: int, coef: Tensor) -> None:
+    """``force <- force + coef[g,0] D+ + coef[g,1] D-`` in place for every atom of the band-major images (``hn_neb_project``;
+    float64 arithmetic, fp32 storage)."""
+    dev = _chk("neb_project", f32=(force, pos, initial, final), f64=(coef,), i32=(image, image_ptr, band_ptr))
+    m, B = _neb_layout("neb_project", pos, initial, final, image, image_ptr, band_ptr, n_images)
+    if tuple(force.shape) != (m, 3) or coef.numel() != 2 * B * int(n_images):
+        raise RuntimeError(f"hermnet_b200.neb_project: expected force [{m},3] and coef [B K,2]")
+    _launch("hn_neb_project", dev, "neb_project", force, pos, initial, final, image, image_ptr, band_ptr, B, int(n_images), coef, m)
+    _bump(force)
+
+
+# ----------------------------------------------------------------------------------------------------
 # tensor-core dense layer (3xTF32 split on tcgen05)
 # ----------------------------------------------------------------------------------------------------
 def split_tf32(w: Tensor) -> Tuple[Tensor, Tensor]:

@@ -6,9 +6,9 @@ loop -- with ASE's attribute names, so ``NNCalculator`` is exercised exactly as 
 -> ``calc.calculate(atoms)``).
 
 Device (SURVEY 8(f) rank 1): positions, velocities and forces stay on the GPU.  ``velocity_verlet_device`` (NVE),
-``langevin_device`` (NVT), ``langevin_npt_device`` (NPT) and ``relax.fire_relax_device`` (FIRE) share the input set-up
-(``_setup``: atoms, replicas of a PyG-style batch, cell) and one evaluation, ``VerletGraph.evaluate``: a Verlet-skin list
-re-used across steps, eager or replayed as a captured CUDA graph."""
+``langevin_device`` (NVT), ``langevin_npt_device`` (NPT), ``relax.fire_relax_device`` (FIRE) and ``neb.neb_device`` (NEB)
+share the input set-up (``_setup``: atoms, replicas of a PyG-style batch, cell) and one evaluation,
+``VerletGraph.evaluate``: a Verlet-skin list re-used across steps, eager or replayed as a captured CUDA graph."""
 from __future__ import annotations
 
 import math

@@ -40,17 +40,7 @@ def fire_relax_device(model, numbers, positions, cell, fmax=0.05, max_steps=1000
     ``energy``, ``fmax`` (the generalized max force) and, with ``relax_cell``, ``volume`` (A^3), all ``[iters, G]``; the
     optimizer state after each iteration's step, ``dt``, ``alpha`` and ``n_pos [iters, G]``; and ``builds`` / ``reuses``."""
     name = "fire_relax_device"
-    if not fmax > 0.0:
-        raise ValueError(f"{name}: fmax must be > 0 (got {fmax})")
-    if not dt > 0.0:
-        raise ValueError(f"{name}: dt must be > 0 (got {dt})")
-    if not dt_max >= dt:
-        raise ValueError(f"{name}: dt_max must be >= dt (got {dt_max} < {dt})")
-    if not max_step > 0.0:
-        raise ValueError(f"{name}: max_step must be > 0 (got {max_step})")
-    if not int(max_steps) >= 0:
-        raise ValueError(f"{name}: max_steps must be >= 0 (got {max_steps})")
-    max_steps = int(max_steps)
+    max_steps = _fire_params(name, fmax, dt, dt_max, max_step, max_steps)
     st = _setup(name, numbers, positions, cell, batch, device,
                 cell_error="relax_cell needs a finite, non-singular cell" if relax_cell else None)
     G, Z, pos, c, replica, replica_ptr = st.G, st.Z, st.pos, st.c, st.replica, st.replica_ptr
@@ -61,35 +51,77 @@ def fire_relax_device(model, numbers, positions, cell, fmax=0.05, max_steps=1000
 
     dev = pos.device
     f64 = dict(dtype=torch.float64, device=dev)
-    dt_g, alpha = torch.full((G,), float(dt), **f64), torch.full((G,), 0.1, **f64)
-    n_pos, steps, converged = (torch.zeros(G, dtype=torch.int32, device=dev) for _ in range(3))
-    coef, fmax_g = torch.zeros((G, 3), **f64), torch.zeros(G, **f64)
-    n_active = torch.zeros(1, dtype=torch.int32, device=dev)
-    vel = torch.zeros_like(pos)
     if relax_cell:
         rp = pos.clone()                                        # r' = x A^-1 with A = I at the start
         A = torch.eye(3, **f64).repeat(G, 1, 1)
         A_prev, vcell, h0 = A.clone(), torch.zeros((G, 3, 3), **f64), c.double()
         P0_t, cf_t = torch.from_numpy(P0 / EV_A3_TO_BAR).to(dev), torch.from_numpy(cf).to(dev)
     else:
-        rp, A, A_prev, vcell, h0, P0_t, cf_t = pos, None, None, None, None, None, None     # positions only: x is r'
+        rp, A, A_prev = pos, None, None                         # positions only: x is r'
+    fire = _Fire(rp, replica, replica_ptr, G, fmax, dt, dt_max, max_step)
 
-    trace = {k: [] for k in ("energy", "fmax", "volume", "dt", "alpha", "n_pos")}
+    energy, volume = [], []
     for it in range(max_steps + 1):
         e, f, *w = vg.evaluate(pos, Z, c)
-        sums = ops.opt_fire_reduce(f, vel, A, replica, replica_ptr)
         if relax_cell:
-            trace["volume"].append(_det3(c.double()).abs())      # of the evaluated cell, before the step moves it
-        ops.opt_fire_step(sums, w[0].contiguous() if relax_cell else None, c if relax_cell else None, h0, A, A_prev, vcell, P0_t,
-                          cf_t, dt_g, alpha, n_pos, steps, converged, fmax, dt_max, max_step, it < max_steps, coef, fmax_g,
-                          n_active)
-        trace["energy"].append(e)
-        for k, t in (("fmax", fmax_g), ("dt", dt_g), ("alpha", alpha), ("n_pos", n_pos)):
-            trace[k].append(t.clone())
-        if it == max_steps or int(n_active.item()) == 0:         # one int read-back per step
+            volume.append(_det3(c.double()).abs())                # of the evaluated cell, before the step moves it
+        rows = (A, w[0].contiguous(), c, h0, A_prev, vcell, P0_t, cf_t) if relax_cell else ()
+        energy.append(e)
+        if fire.step(f, it < max_steps, *rows):
             break
-        ops.opt_fire_update(pos if relax_cell else None, rp, vel, f, A_prev, A, replica, converged, coef)
+        fire.update(f, pos if relax_cell else None, A_prev, A)
     if stats is not None:
-        stats.update(vg.counts(), converged=converged.bool(), steps=steps.clone(),
-                     **{k: torch.stack(v) for k, v in trace.items() if v})
+        trace = fire.trace
+        stats.update(vg.counts(), converged=fire.converged.bool(), steps=fire.steps.clone(), energy=torch.stack(energy),
+                     fmax=torch.stack(trace["fmax"]), **({"volume": torch.stack(volume)} if relax_cell else {}),
+                     **{k: torch.stack(trace[k]) for k in ("dt", "alpha", "n_pos")})
     return pos, c, e
+
+
+def _fire_params(name, fmax, dt, dt_max, max_step, max_steps) -> int:
+    """``max_steps`` as an int, after the checks of FIRE's parameters (``ValueError``)."""
+    if not fmax > 0.0:
+        raise ValueError(f"{name}: fmax must be > 0 (got {fmax})")
+    if not dt > 0.0:
+        raise ValueError(f"{name}: dt must be > 0 (got {dt})")
+    if not dt_max >= dt:
+        raise ValueError(f"{name}: dt_max must be >= dt (got {dt_max} < {dt})")
+    if not max_step > 0.0:
+        raise ValueError(f"{name}: max_step must be > 0 (got {max_step})")
+    if not int(max_steps) >= 0:
+        raise ValueError(f"{name}: max_steps must be >= 0 (got {max_steps})")
+    return int(max_steps)
+
+
+class _Fire:
+    """ASE's FIRE over ``G`` contiguous replicas of the rows ``rp [n,3]`` (updated in place), on the device: the per-replica
+    state (``dt``, ``alpha``, ``n_pos``, ``steps``, sticky ``converged``, the step's ``coef``, ``fmax``, ``n_active``), the
+    row velocities and the per-iteration sequence ``ops.opt_fire_reduce`` -> ``ops.opt_fire_step`` -> ``ops.opt_fire_update``.
+    ``trace`` keeps ``fmax`` and the state after each step (``dt``, ``alpha``, ``n_pos``).  The cell rows of
+    ``fire_relax_device`` are passed in by the caller, which owns that state."""
+
+    def __init__(self, rp, replica, replica_ptr, G, fmax, dt, dt_max, max_step):
+        dev = rp.device
+        f64 = dict(dtype=torch.float64, device=dev)
+        self.rp, self.replica, self.replica_ptr = rp, replica, replica_ptr
+        self.fmax_limit, self.dt_max, self.max_step = fmax, dt_max, max_step
+        self.dt, self.alpha = torch.full((G,), float(dt), **f64), torch.full((G,), 0.1, **f64)
+        self.n_pos, self.steps, self.converged = (torch.zeros(G, dtype=torch.int32, device=dev) for _ in range(3))
+        self.coef, self.fmax = torch.zeros((G, 3), **f64), torch.zeros(G, **f64)
+        self.n_active = torch.zeros(1, dtype=torch.int32, device=dev)
+        self.vel = torch.zeros_like(rp)
+        self.trace = {k: [] for k in ("fmax", "dt", "alpha", "n_pos")}
+
+    def step(self, f, move, A=None, virial=None, cell=None, h0=None, A_prev=None, vcell=None, P0=None, cell_factor=None) -> bool:
+        """Convergence test and, with ``move``, FIRE's step logic at forces ``f`` (cell rows with ``A``).  True when the run
+        ends here: ``move`` is False or no replica moves any more (one int read back)."""
+        sums = ops.opt_fire_reduce(f, self.vel, A, self.replica, self.replica_ptr)
+        ops.opt_fire_step(sums, virial, cell, h0, A, A_prev, vcell, P0, cell_factor, self.dt, self.alpha, self.n_pos, self.steps,
+                          self.converged, self.fmax_limit, self.dt_max, self.max_step, move, self.coef, self.fmax, self.n_active)
+        for k in self.trace:
+            self.trace[k].append(getattr(self, k).clone())
+        return not move or int(self.n_active.item()) == 0
+
+    def update(self, f, x=None, A_prev=None, A=None):
+        """The rows of the replicas still moving (and ``x = rp A`` with ``A``)."""
+        ops.opt_fire_update(x, self.rp, self.vel, f, A_prev, A, self.replica, self.converged, self.coef)

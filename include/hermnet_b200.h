@@ -532,6 +532,39 @@ int hn_opt_fire_update(float *x /*[N,3]*/, float *rp /*[N,3]*/, float *vel /*[N,
                        const double *A_prev /*[G,9]*/, const double *A /*[G,9] or NULL*/, const int32_t *replica /*[N]*/,
                        const int32_t *converged /*[G]*/, const double *coef /*[G,3]*/, int64_t n_atoms, void *stream);
 
+/* ---------------------------------------------------------------------------------------------
+ * Nudged elastic band forces (csrc/hn_neb.cu): ASE's NEB(method="improvedtangent", climb=...) over B bands of K interior
+ * images each.  Band-major layout of the N_img = B K images: image g = b K + k of band b is the contiguous atom range
+ * [image_ptr[g], image_ptr[g+1]) of n_b atoms (image[i] = g), images 0..K-1 of a band one after the other; the endpoints are
+ * `initial` / `final` [sum n_b, 3] with band b at rows band_ptr[b] .. band_ptr[b+1] in the same atom order.  For atom i of
+ * image k: R_{k-1} is pos[i - n_b] (k > 0) or initial[band_ptr[b] + local] (k == 0), R_{k+1} is pos[i + n_b] (k < K-1) or
+ * final[band_ptr[b] + local] (k == K-1);  D+ = R_{k+1} - R_k,  D- = R_k - R_{k-1}.
+ *   hn_neb_reduce    sums[g] = (|D+|^2, |D-|^2, D+.D-, F.D+, F.D-) over the atoms of image g, float64 from fp32 positions and
+ *                    forces; the fixed-order chunk / slot scheme of hn_opt_fire_reduce (bitwise reproducible for a given
+ *                    layout), workspace of hn_neb_reduce_workspace_bytes.
+ *   hn_neb_step      one thread per band, float64 (energies promoted from fp32; end_energy[b] = (E_initial, E_final)):
+ *                    imax[b] = 1 + the first k of maximal energy (1..K, the numbering with the endpoints at 0 and K+1);
+ *                    tangent tau = a D+ + w D-:  E_{k+1} > E_k > E_{k-1}: (1, 0);  E_{k+1} < E_k < E_{k-1}: (0, 1);  else
+ *                    with V_max / V_min the larger / smaller of |E_{k+1} - E_k|, |E_{k-1} - E_k|:  (V_max, V_min) if
+ *                    E_{k+1} > E_{k-1} else (V_min, V_max), and (1, 1) when V_max == 0.  T = a^2 S++ + 2 a w S+- + w^2 S--,
+ *                    Ft = a F+ + w F-;  q = -2 Ft / T for the climbing image (climb != 0 and k == imax - 1), else
+ *                    q = -Ft / T + spring[b] (sqrt S++ - sqrt S--) / sqrt T;  q = 0 when T == 0.  coef[g] = (q a, q w).
+ *   hn_neb_project   per atom: F <- F + coef[g][0] D+ + coef[g][1] D-  (float64 arithmetic, fp32 in place).
+ * Checks: 0 <= n_atoms < 2^31, n_bands >= 0, n_images >= 1, non-null pointers when there is work (no atoms / no bands:
+ * no-op).  No host synchronisation.
+ * ------------------------------------------------------------------------------------------- */
+int64_t hn_neb_reduce_workspace_bytes(int64_t n_atoms, int32_t n_img);
+int hn_neb_reduce(const float *pos /*[M,3]*/, const float *force /*[M,3]*/, const float *initial /*[N,3]*/, const float *final_ /*[N,3]*/,
+                  const int32_t *image /*[M]*/, const int32_t *image_ptr /*[B*K+1]*/, const int32_t *band_ptr /*[B+1]*/,
+                  int32_t n_bands, int32_t n_images, int64_t n_atoms /*M = K N*/, double *sums /*[B*K,5]*/, void *workspace,
+                  int64_t workspace_bytes, void *stream);
+int hn_neb_step(const double *sums /*[B*K,5]*/, const float *energy /*[B*K]*/, const float *end_energy /*[B,2]*/,
+                const double *spring /*[B]*/, int32_t climb, int32_t n_bands, int32_t n_images, double *coef /*[B*K,2]*/,
+                int32_t *imax /*[B]*/, void *stream);
+int hn_neb_project(float *force /*[M,3]*/, const float *pos /*[M,3]*/, const float *initial /*[N,3]*/, const float *final_ /*[N,3]*/,
+                   const int32_t *image /*[M]*/, const int32_t *image_ptr /*[B*K+1]*/, const int32_t *band_ptr /*[B+1]*/,
+                   int32_t n_bands, int32_t n_images, const double *coef /*[B*K,2]*/, int64_t n_atoms, void *stream);
+
 #ifdef __cplusplus
 }
 #endif
